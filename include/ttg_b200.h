@@ -50,45 +50,31 @@ int ttg_conv2d_wgrad_direct_det(const void* x, const void* gy, float* gw, int N,
                                 int ksize, int up, int dtype_x, int dtype_gy, void* workspace, void* stream);
 
 /* ---- tensor-core convolution (bf16 operands, fp32 accumulate in TMEM, tcgen05.mma)
- * same reference call sites as above; Cin, Cout multiples of 16.
+ * same reference call sites as above; Cin, Cout multiples of 16, stride 1, no fused upsample: the
+ * generator's nearest x2 upsample (generator.py:58) is materialised by ttg_upsample2 first, so that the
+ * activation tiles of fprop, dgrad and wgrad are all fetched with tensor-map (TMA) loads.  The CUDA driver must
+ * provide cuTensorMapEncodeTiled; otherwise these entry points return an error.
  * ttg_pack_weight_tc: OIHW fp32 -> bf16 UMMA B-operand image, mode 0 fprop / 1 dgrad.
- * ttg_conv2d_tc: y = conv(x) (+bias); optional fused input transform
- *   a = lrelu((x - mean[c]) * invstd[c] * gamma[c] + beta[c]) (pre_mean != NULL), i.e. the
- *   BatchNorm2d+LeakyReLU that precedes the conv in every residual block, and optional
- *   nearest x2 upsample folded into the addressing (up=1).
+ * ttg_conv2d_tc: y = conv(x) (+bias), y bf16 or fp32 (dtype_out).
  * ttg_conv2d_wgrad_tc: gw (fp32 OIHW) = sum_pixels gy x shifted(x). */
 size_t ttg_pack_weight_tc_bytes(int Cout, int Cin, int ksize);
 int ttg_pack_weight_tc(const float* w, void* wp, int Cout, int Cin, int ksize, int mode, void* stream);
 int ttg_conv2d_tc(const void* x, const void* wp, const float* bias, void* y, int N, int H, int W, int Cin, int Cout,
-                  int ksize, int up, int dtype_out, void* stream);
-/* tuning switch: 1 (default) = TMA-fed activation tiles where applicable, 0 = cp.async staging everywhere; any other
- * value is rejected (the layout timing experiments 2 / 3 exist in -DTTG_TRACE development builds only) */
-int ttg_set_use_tma(int on);
-int ttg_set_use_fold(int on);   /* development switch: kx-folded row-tile conv kernel on / off */
-/* A/B switch (default 0: measured slower than the tensor-map tiles, DESIGN.md 3.3; always used for the fused nearest
- * upsample `up == 1`): resident-filter layers (Cin in {16, 32, 64}) fetch their halo tiles as whole pixel rows with
- * cp.async.bulk and re-lay them out in shared memory (where the fused BatchNorm/LeakyReLU prologue, the fused nearest
- * upsample and the channel padding of 8-channel tensors are applied); 0 = tensor-map (TMA tile) loads. */
-int ttg_set_use_rows(int on);
-/* A/B switch (default 1): the TMA-fed resident-filter conv kernel fetches its halo tile pixel-major with a
- * SWIZZLE_32B/64B/128B tensor map (one L2 request per pixel) instead of 16-byte channel-group rows. */
-int ttg_set_use_swz(int on);
-int ttg_conv2d_tc_pre(const void* x, const void* wp, const float* bias, void* y, int N, int H, int W, int Cin,
-                      int Cout, int ksize, int up, int dtype_out, const float* pre_scale, const float* pre_shift,
-                      float slope, void* stream);
+                  int ksize, int dtype_out, void* stream);
 /* channel-padded variants: Cin/Cout are the padded GEMM sizes (16), cin_real/cout_real the channel counts in memory
- * (RGB layers: Cin == 3 first D conv discriminator.py:63, Cout == 3 image gradient / generator.py:124) */
+ * (RGB layers: Cin == 3 first D conv discriminator.py:63, Cout == 3 image gradient / generator.py:124).
+ * ttg_conv2d_tc_ex also accepts other narrow tensors (<= 8 input channels; <= 16 output channels when Cout == 16),
+ * read / written with scalar accesses; the wgrad entry points accept only the 8-channel staging tensors below. */
 int ttg_pack_weight_tc_pad(const float* w, void* wp, int Cout, int Cin, int CoutP, int CinP, int ksize, int mode,
                            void* stream);
 int ttg_conv2d_tc_ex(const void* x, const void* wp, const float* bias, void* y, int N, int H, int W, int Cin, int Cout,
-                     int cin_real, int cout_real, int ksize, int up, int dtype_out, const float* pre_scale,
-                     const float* pre_shift, float slope, void* stream);
+                     int cin_real, int cout_real, int ksize, int dtype_out, void* stream);
 int ttg_conv2d_wgrad_tc_ex(const void* x, const void* gy, float* gw, int N, int H, int W, int Cin, int Cout,
-                           int cin_real, int cout_real, int ksize, int up, void* workspace, void* stream);
+                           int cin_real, int cout_real, int ksize, void* workspace, void* stream);
 /* 8-channel staging copies of the <= 8-channel (RGB) bf16 tensors: y8[p][0..7] = x[p][0..c_real-1], 0...  With
  * cin_real / cout_real == 8 (Cin / Cout == 16) the _ex entry points above read / write such tensors through the
  * same TMA tiles and 16-byte stores as the wide layers (missing channel groups are zero-filled by the TMA engine). */
-/* conv (bf16 NHWC, channels multiples of 16, no upsample) that also returns the BatchNorm statistics of its output:
+/* conv (bf16 NHWC, channels multiples of 16) that also returns the BatchNorm statistics of its output:
  * sums[0..Cout) = sum over pixels, sums[Cout..2Cout) = sum of squares (fp64; of the bf16 values written).  Replaces the
  * first pass of native_batch_norm over the conv output (conv -> BatchNorm2d pairs: generator.py:41-43,
  * discriminator.py:63-65).  ttg_bn_finalize turns the sums into mean / invstd / running statistics. */
@@ -105,14 +91,10 @@ int ttg_unpad_channels8(const void* y8, void* y, long long npix, int c_real, voi
 /* wgrad + bias gradient gbias[co] = sum_pixels gy (fp32) in ONE pass over gy (both halves of convolution_backward's
  * parameter gradients, nn.Conv2d(bias=True): generator.py:41,44, discriminator.py:63,66) */
 int ttg_conv2d_wgrad_bias_tc_ex(const void* x, const void* gy, float* gw, float* gbias, int N, int H, int W, int Cin,
-                                int Cout, int cin_real, int cout_real, int ksize, int up, void* workspace, void* stream);
+                                int Cout, int cin_real, int cout_real, int ksize, void* workspace, void* stream);
 int ttg_conv2d_wgrad_tc(const void* x, const void* gy, float* gw, int N, int H, int W, int Cin, int Cout, int ksize,
-                        int up, void* workspace, void* stream);
+                        void* workspace, void* stream);
 size_t ttg_conv2d_wgrad_tc_workspace_bytes(int Cin, int Cout, int ksize);
-/* A/B switch (default 1): 3x3 wgrad of narrow layers (3 Cout <= 128, 3 Cin <= 256) with the filter column folded into
- * the MMA's M dimension (three column-shifted copies of the gy tile) and the filter row into N: 8 instead of 24 MMAs
- * per 128-pixel tile.  0 restores the per-column variant. */
-int ttg_set_wgrad_mfold(int on);
 
 /* ---- train-mode BatchNorm2d fused with LeakyReLU
  * (nn.BatchNorm2d + nn.LeakyReLU(0.2) pairs: generator.py:38-43,120-122;
@@ -162,7 +144,7 @@ int ttg_channel_sum(const void* x, long long M, int C, float* out, void* workspa
  * behaviour of the entry point without suffix; ttg_conv2d_wgrad_tc_acc always accumulates), bit 1 = the caller
  * guarantees that `workspace` is all zero already (one clear per training step instead of one memset per call). */
 int ttg_conv2d_wgrad_tc_acc(const void* x, const void* gy, float* gw, float* gbias, int N, int H, int W, int Cin, int Cout,
-                            int cin_real, int cout_real, int ksize, int up, int flags, void* workspace, void* stream);
+                            int cin_real, int cout_real, int ksize, int flags, void* workspace, void* stream);
 int ttg_bn_act_bwd_acc(const void* x, const void* ga, void* gx, long long M, int C, const float* mean,
                        const float* invstd, const float* gamma, const float* beta, float slope, float* ggamma,
                        float* gbeta, int accumulate, void* workspace, int dtype, void* stream);

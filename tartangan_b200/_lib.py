@@ -67,13 +67,6 @@ class _Lib:
                 fn = getattr(dll, name)       # AttributeError if the header and the library disagree
                 fn.restype, fn.argtypes = restype, argtypes
             self._dll = dll
-            # development A/B switches (kernel variants); unset = the library defaults
-            for env, fn in (('TTG_ROWS', 'ttg_set_use_rows'), ('TTG_SWZ', 'ttg_set_use_swz'), ('TTG_MFOLD', 'ttg_set_wgrad_mfold'), ('TTG_NBUF', 'ttg_set_nbuf_exp'), ('TTG_PERSM', 'ttg_set_persm_cap')):
-                if os.environ.get(env) is not None and hasattr(dll, fn):
-                    getattr(dll, fn)(int(os.environ[env]))
-            if os.environ.get('TTG_WG_TUNE') and hasattr(dll, 'ttg_set_wgrad_tuning'):
-                nb, ps = os.environ['TTG_WG_TUNE'].split(',')
-                dll.ttg_set_wgrad_tuning(int(nb), int(ps))
         return self._dll
 
     def __getattr__(self, name):

@@ -283,9 +283,8 @@ __global__ void __launch_bounds__(CB_THREADS) chan_reduce_bulk_kernel(Op op, lon
   for (int i = tid; i < Op::NACC * C; i += blockDim.x) atomicAdd(&out[i], s_acc[i]);
 }
 
-static int g_chan_bulk = 1;      // development switch (ttg_set_chan_bulk)
 template <typename T, class Op> static inline bool cb_ok(int C, const void* const* ptrs, int n, long long nelem) {
-  if (!g_chan_bulk || !std::is_same<T, bf16>::value) return false;
+  if (!std::is_same<T, bf16>::value) return false;
   const int groups = C >> 3;
   if (C % 8 || groups < 1 || groups > 32 || (groups & (groups - 1)) || nelem % 8) return false;
   for (int i = 0; i < n; ++i)
@@ -392,8 +391,7 @@ __global__ void __launch_bounds__(256) chan_reduce_c3_kernel(Op op, long long ng
   if (threadIdx.x < Op::NACC * 3) atomicAdd(&out[threadIdx.x], s_acc[threadIdx.x]);
 }
 template <typename T> static inline bool c3_ok(int C, const void* const* ptrs, int nptr, long long n) {
-  static const bool off = getenv("TTG_NO_C3") != nullptr;       // development A/B switch
-  if (off || C != 3 || n % (3 * Vec<T>::N)) return false;
+  if (C != 3 || n % (3 * Vec<T>::N)) return false;
   for (int i = 0; i < nptr; ++i)
     if (reinterpret_cast<uintptr_t>(ptrs[i]) & 15) return false;
   return true;

@@ -9,12 +9,10 @@
 // 9 filter taps is just a shifted descriptor start address (no im2col copies, no re-reads):
 //   fprop/dgrad: A = pixels x channels (K-major),  B = packed weights (K-major),  N = Cout
 //   wgrad      : A = gy^T   (MN-major, K = pixels), B = shifted x (MN-major),     N = Cin
-// Zero padding = zero-filled halo; nearest x2 upsample (generator.py:58) = (y>>1, x>>1) addressing;
-// the BatchNorm+LeakyReLU that precedes each conv can be applied while staging (pre_scale/shift).
+// Zero padding = zero-filled halo.
 // The epilogue reads the fp32 accumulator from TMEM (tcgen05.ld 32x32b), adds the bias and
 // writes NHWC rows (one thread = one pixel = Cout contiguous channels).
 #include "tc_common.cuh"
-#include <string.h>
 
 #define TC_TH 16
 #define TC_TW 8
@@ -26,7 +24,6 @@ template <int... Is, typename F>
 __device__ __forceinline__ void static_for_impl(std::integer_sequence<int, Is...>, F&& f) { (f(std::integral_constant<int, Is>{}), ...); }
 template <int N, typename F>
 __device__ __forceinline__ void static_for(F&& f) { static_for_impl(std::make_integer_sequence<int, N>{}, f); }
-#define TC_STAGE_BYTES (32 * 1024)
 
 // ------------------------------------------------------------------ weight packing
 // mode 0 (fprop): wp[tap][ci/8][co][ci%8]            = w[co][ci][ky][kx]        (B: N=co, K=ci)
@@ -65,37 +62,36 @@ __device__ __forceinline__ void cp_async16(uint32_t dst, const void* src, uint32
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
 template <int HALO>
-__device__ __forceinline__ bool tile_src(int u, int c8n, int n, int y0, int x0, int H, int W, int C, int up,
+__device__ __forceinline__ bool tile_src(int u, int c8n, int n, int y0, int x0, int H, int W, int C,
                                          long long& src_elem, uint32_t& dst_unit) {
-  constexpr int WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO, HP = WH * HH;
+  constexpr int WH = TC_TW + 2 * HALO;
   const int c8 = u % c8n, pix = u / c8n;
   const int hy = pix / WH, hx = pix - hy * WH;
   const int gy = y0 + hy - HALO, gx = x0 + hx - HALO;
   dst_unit = (uint32_t)((hy * c8n + c8) * WH + hx);
   const bool ok = gy >= 0 && gy < H && gx >= 0 && gx < W;
-  src_elem = ok ? ((((long long)n * (H >> up) + (gy >> up)) * (W >> up) + (gx >> up)) * C + c8 * 8) : 0;
+  src_elem = ok ? ((((long long)n * H + gy) * W + gx) * C + c8 * 8) : 0;
   return ok;
 }
 
 // asynchronous version (LDGSTS, zero-fill outside the image); caller waits with cp_async_wait_all()
 template <int HALO>
 __device__ __forceinline__ void stage_tile_async(uint8_t* sA, const bf16* __restrict__ x, int n, int y0, int x0, int H,
-                                                 int W, int C, int up, int nthr) {
+                                                 int W, int C, int nthr) {
   constexpr int HP = (TC_TW + 2 * HALO) * (TC_TH + 2 * HALO);
   const int c8n = C >> 3;
   const uint32_t base = smem_u32(sA);
   for (int u = threadIdx.x; u < HP * c8n; u += nthr) {
     long long se; uint32_t du;
-    const bool ok = tile_src<HALO>(u, c8n, n, y0, x0, H, W, C, up, se, du);
+    const bool ok = tile_src<HALO>(u, c8n, n, y0, x0, H, W, C, se, du);
     cp_async16(base + du * 16, x + se, ok ? 16u : 0u);
   }
 }
 
-// register version, 4 loads in flight per thread, optional fused BatchNorm+LeakyReLU transform
+// register version, 4 loads in flight per thread
 template <int HALO>
 __device__ __forceinline__ void stage_tile(uint8_t* sA, const bf16* __restrict__ x, int n, int y0, int x0, int H, int W,
-                                           int C, int up, const float* __restrict__ pre_scale,
-                                           const float* __restrict__ pre_shift, float slope, int nthr) {
+                                           int C, int nthr) {
   constexpr int HP = (TC_TW + 2 * HALO) * (TC_TH + 2 * HALO);
   const int c8n = C >> 3;
   const int total = HP * c8n;
@@ -109,29 +105,12 @@ __device__ __forceinline__ void stage_tile(uint8_t* sA, const bf16* __restrict__
       du[j] = 0;
       if (live[j]) {
         long long se;
-        if (tile_src<HALO>(u, c8n, n, y0, x0, H, W, C, up, se, du[j])) v[j] = __ldg(reinterpret_cast<const uint4*>(x + se));
-        else du[j] |= 0x80000000u;       // mark padding: stays exactly zero (padding applies after the activation)
+        if (tile_src<HALO>(u, c8n, n, y0, x0, H, W, C, se, du[j])) v[j] = __ldg(reinterpret_cast<const uint4*>(x + se));
       }
     }
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      if (!live[j]) continue;
-      const bool pad = du[j] & 0x80000000u;
-      const uint32_t unit = du[j] & 0x7fffffffu;
-      if (pre_scale && !pad) {
-        const int c8 = (int)(unit / (TC_TW + 2 * HALO)) % c8n;
-        __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&v[j]);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          float2 f = __bfloat1622float2(h[q]);
-          const int c = c8 * 8 + 2 * q;
-          f.x = lrelu(f.x * pre_scale[c] + pre_shift[c], slope);
-          f.y = lrelu(f.y * pre_scale[c + 1] + pre_shift[c + 1], slope);
-          h[q] = __floats2bfloat162_rn(f.x, f.y);
-        }
-      }
-      *reinterpret_cast<uint4*>(sA + (size_t)unit * 16) = v[j];
-    }
+    for (int j = 0; j < 4; ++j)
+      if (live[j]) *reinterpret_cast<uint4*>(sA + (size_t)du[j] * 16) = v[j];
   }
 }
 
@@ -167,16 +146,15 @@ extern "C" int ttg_pack_weight_tc_pad(const float* w, void* wp, int Cout, int Ci
 // stage a tile of a tensor with c_real (<= 8) channels into the C-channel (padded) shared-memory image
 template <int HALO>
 __device__ __forceinline__ void stage_tile_pad(uint8_t* sA, const bf16* __restrict__ x, int n, int y0, int x0, int H, int W,
-                                               int C, int c_real, int up, int nthr) {
+                                               int C, int c_real, int nthr) {
   constexpr int WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO, HP = WH * HH;
-  const int c8n = C >> 3, Hi = H >> up, Wi = W >> up;
+  const int c8n = C >> 3;
   for (int pix = threadIdx.x; pix < HP; pix += nthr) {
     const int hy = pix / WH, hx = pix - hy * WH;
     const int gy = y0 + hy - HALO, gx = x0 + hx - HALO;
     uint32_t w[4] = {0u, 0u, 0u, 0u};
     if (gy >= 0 && gy < H && gx >= 0 && gx < W) {
-      const unsigned short* src = reinterpret_cast<const unsigned short*>(x) +
-                                  (((long long)n * Hi + (gy >> up)) * Wi + (gx >> up)) * c_real;
+      const unsigned short* src = reinterpret_cast<const unsigned short*>(x) + (((long long)n * H + gy) * W + gx) * c_real;
       for (int c = 0; c < c_real; ++c) w[c >> 1] |= (uint32_t)src[c] << (16 * (c & 1));
     }
     uint8_t* d = sA + (size_t)((hy * c8n) * WH + hx) * 16;
@@ -204,149 +182,22 @@ __device__ __forceinline__ RowStager make_row_stager(int C, int tid) {
   rs.q_c8 = q - rs.q_hx * c8n;
   return rs;
 }
-template <int HALO, bool ASYNC>
+template <int HALO>
 __device__ __forceinline__ void stage_rows(const RowStager& rs, uint8_t* sA, const bf16* __restrict__ x, int n, int y0,
-                                           int x0, int H, int W, int C, int up, const float* __restrict__ pre_scale,
-                                           const float* __restrict__ pre_shift, float slope) {
-  constexpr int WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO, HP = WH * HH;
+                                           int x0, int H, int W, int C) {
+  constexpr int WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO;
   if (!rs.active) return;
   const int gx = x0 + rs.q_hx - HALO;
   const bool xok = gx >= 0 && gx < W;
-  const int Wi = W >> up, Hi = H >> up;
-  const bf16* col = x + ((long long)n * Hi * Wi + (gx >> up)) * C + rs.q_c8 * 8;
+  const bf16* col = x + ((long long)n * H * W + gx) * C + rs.q_c8 * 8;
   const int c8n = C >> 3;
   uint32_t dst = smem_u32(sA) + (uint32_t)((rs.r0 * c8n + rs.q_c8) * WH + rs.q_hx) * 16;
   const uint32_t dstep = (uint32_t)(rs.rpp * c8n * WH) * 16;
-  float sc[8], sh[8];
-  if constexpr (!ASYNC) {
-#pragma unroll
-    for (int j = 0; j < 8; ++j) { sc[j] = pre_scale[rs.q_c8 * 8 + j]; sh[j] = pre_shift[rs.q_c8 * 8 + j]; }
-  }
   for (int r = rs.r0; r < HH; r += rs.rpp, dst += dstep) {
     const int gy = y0 + r - HALO;
     const bool ok = xok && gy >= 0 && gy < H;
-    const bf16* src = ok ? col + (long long)(gy >> up) * Wi * C : x;
-    if constexpr (ASYNC) {
-      cp_async16(dst, src, ok ? 16u : 0u);
-    } else {
-      uint4 v = make_uint4(0u, 0u, 0u, 0u);
-      if (ok) {
-        v = __ldg(reinterpret_cast<const uint4*>(src));
-        __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&v);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          float2 f = __bfloat1622float2(h[q]);
-          f.x = lrelu(f.x * sc[2 * q] + sh[2 * q], slope);
-          f.y = lrelu(f.y * sc[2 * q + 1] + sh[2 * q + 1], slope);
-          h[q] = __floats2bfloat162_rn(f.x, f.y);
-        }
-      }
-      asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(dst), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-    }
+    cp_async16(dst, ok ? col + (long long)gy * W * C : x, ok ? 16u : 0u);
   }
-}
-
-// ------------------------------------------------------------------ fprop / dgrad
-template <int K>
-__global__ void __launch_bounds__(128) conv_tc_kernel(const bf16* __restrict__ x, const bf16* __restrict__ wp,
-                                                      const float* __restrict__ bias, void* __restrict__ y, int out_f32,
-                                                      int H, int W, int Cin, int Cout, int up,
-                                                      const float* __restrict__ pre_scale,
-                                                      const float* __restrict__ pre_shift, float slope, int stage_slices,
-                                                      int nstages, int tmem_cols) {
-  constexpr int HALO = K / 2, WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO, HP = WH * HH;
-  extern __shared__ __align__(128) uint8_t smem[];
-  const int tid = threadIdx.x, warp = tid >> 5;
-  const uint32_t a_bytes = (uint32_t)(Cin >> 3) * HP * 16;
-  const uint32_t slice_bytes = (uint32_t)Cout * 32;                 // one K=16 slice of one tap: [2][Cout][8] bf16
-  const uint32_t stage_bytes = (uint32_t)stage_slices * slice_bytes;
-  uint8_t* sA = smem;
-  uint8_t* sW = smem + a_bytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sW + (size_t)nstages * stage_bytes);   // [0..1] stage free, [2] done
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 4);
-
-  const int tiles_x = (W + TC_TW - 1) / TC_TW, tiles_y = (H + TC_TH - 1) / TC_TH;
-  const int tile = blockIdx.x;
-  const int n = tile / (tiles_x * tiles_y), t2 = tile - n * tiles_x * tiles_y;
-  const int y0 = (t2 / tiles_x) * TC_TH, x0 = (t2 % tiles_x) * TC_TW;
-
-  if (warp == 0) tmem_alloc(tmem_slot, (uint32_t)tmem_cols);
-  if (tid == 32) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); mbar_init(&bars[2], 1); mbar_fence_init(); }
-  stage_tile<HALO>(sA, x, n, y0, x0, H, W, Cin, up, pre_scale, pre_shift, slope, 128);
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  const uint32_t tmem_base = *tmem_slot;
-
-  const int k16n = Cin >> 4;
-  const int total_slices = K * K * k16n;
-  const int nchunks = (total_slices + stage_slices - 1) / stage_slices;
-  const uint32_t idesc = umma_idesc_bf16(128, Cout, 0, 0);
-  const uint32_t sA_addr = smem_u32(sA);
-
-  for (int c = 0; c < nchunks; ++c) {
-    const int s = c % nstages;
-    if (c >= nstages) mbar_wait(&bars[s], (uint32_t)((c / nstages) - 1) & 1u);     // MMAs that read this stage are done
-    const int first = c * stage_slices;
-    const int cnt = min(stage_slices, total_slices - first);
-    {
-      const uint4* src = reinterpret_cast<const uint4*>(reinterpret_cast<const uint8_t*>(wp) + (size_t)first * slice_bytes);
-      uint4* dst = reinterpret_cast<uint4*>(sW + (size_t)s * stage_bytes);
-      const int nvec = (int)((size_t)cnt * slice_bytes / 16);
-      for (int i = tid; i < nvec; i += blockDim.x) dst[i] = __ldg(src + i);
-    }
-    fence_proxy_async_smem();          // generic-proxy smem writes -> visible to the tensor-core (async) proxy
-    __syncthreads();
-    if (tid == 0) {
-      tc_fence_after_sync();
-      const uint32_t sW_addr = smem_u32(sW + (size_t)s * stage_bytes);
-      for (int i = 0; i < cnt; ++i) {
-        const int slice = first + i;
-        const int tap = slice / k16n, j = slice - tap * k16n;
-        const int ky = tap / K, kx = tap - ky * K;
-        // A: rows = 16 groups of 8 pixels (SBO = one halo row = C/8*WH units), K chunks of 8 channels (LBO = WH units)
-        const int c8n = Cin >> 3;
-        const uint64_t adesc = umma_desc(sA_addr + (uint32_t)((ky * c8n * WH + kx) + 2 * j * WH) * 16, WH * 16, c8n * WH * 16);
-        // B: rows = Cout (SBO = 8 rows x 16 B), K chunks (LBO = Cout units)
-        const uint64_t bdesc = umma_desc(sW_addr + (uint32_t)i * slice_bytes, (uint32_t)Cout * 16, 128);
-        umma_bf16(tmem_base, adesc, bdesc, idesc, slice > 0 ? 1u : 0u);
-      }
-      umma_commit(&bars[s]);
-      if (c == nchunks - 1) umma_commit(&bars[2]);
-    }
-  }
-
-  // ---- epilogue: thread = pixel (TMEM lane), columns = output channels
-  mbar_wait(&bars[2], 0);
-  tc_fence_after_sync();
-  const int m = tid, gy = y0 + (m >> 3), gx = x0 + (m & 7);
-  const bool valid = gy < H && gx < W;
-  const long long opix = ((long long)n * H + gy) * W + gx;
-  for (int c0 = 0; c0 < Cout; c0 += 16) {
-    uint32_t r[16];
-    tmem_ld16(tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)c0, r);
-    tmem_ld_wait();
-    if (valid) {
-      float f[16];
-#pragma unroll
-      for (int j = 0; j < 16; ++j) f[j] = __uint_as_float(r[j]) + (bias ? bias[c0 + j] : 0.f);
-      if (out_f32) {
-        float4* dst = reinterpret_cast<float4*>(reinterpret_cast<float*>(y) + opix * Cout + c0);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) dst[j] = make_float4(f[4 * j], f[4 * j + 1], f[4 * j + 2], f[4 * j + 3]);
-      } else {
-        uint4 o[2];
-        __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(o);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) h[j] = __floats2bfloat162_rn(f[2 * j], f[2 * j + 1]);
-        uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<bf16*>(y) + opix * Cout + c0);
-        dst[0] = o[0]; dst[1] = o[1];
-      }
-    }
-  }
-  tc_fence_before_sync();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem_base, (uint32_t)tmem_cols);
 }
 
 // ------------------------------------------------------------------ fprop / dgrad, persistent (weights resident)
@@ -625,12 +476,12 @@ template <int N> __device__ __forceinline__ void cp_async_wait_group() { asm vol
 // epilogue; warp 4 only issues tcgen05.mma.  Hand-offs are mbarriers (full/empty per activation slot,
 // full/empty per TMEM accumulator), so loads of tile i+NBUF-1, MMAs of tile i and the epilogue of
 // tile i-1 are in flight together and nobody waits for the single MMA-issuing thread.
-template <int K, int NBUF, bool LEAN>
+// Serves the channel-padded layers that the TMA kernels do not cover: <= 8 real input channels read with scalar
+// loads, or a 16-channel accumulator of which only cout_real channels are stored (the fp32 RGB output conv).
+template <int K, int NBUF>
 __global__ void __launch_bounds__(160) conv_tc_persist_kernel(const bf16* __restrict__ x, const bf16* __restrict__ wp,
                                                               const float* __restrict__ bias, void* __restrict__ y,
-                                                              int out_f32, int H, int W, int Cin, int Cout, int up,
-                                                              const float* __restrict__ pre_scale,
-                                                              const float* __restrict__ pre_shift, float slope,
+                                                              int out_f32, int H, int W, int Cin, int Cout,
                                                               int total_tiles, int tmem_cols, int cin_real, int cout_real) {
   constexpr int HALO = K / 2, WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO, HP = WH * HH;
   // DIST tiles are prefetched ahead; NBUF - DIST >= 2 leaves a slot of slack so that re-using a slot never
@@ -687,17 +538,9 @@ __global__ void __launch_bounds__(160) conv_tc_persist_kernel(const bf16* __rest
         int n, y0, x0;
         tile_coords(j, n, y0, x0);
         uint8_t* dst = sA + (size_t)s * a_bytes;
-        if constexpr (LEAN) {         // common case only: keeps the instruction footprint small
-          stage_rows<HALO, true>(rs, dst, x, n, y0, x0, H, W, Cin, up, nullptr, nullptr, 1.f);
-        } else if (cin_real != Cin) {
-          stage_tile_pad<HALO>(dst, x, n, y0, x0, H, W, Cin, cin_real, up, 128);
-        } else if (fast_stage) {
-          if (pre_scale) stage_rows<HALO, false>(rs, dst, x, n, y0, x0, H, W, Cin, up, pre_scale, pre_shift, slope);
-          else stage_rows<HALO, true>(rs, dst, x, n, y0, x0, H, W, Cin, up, nullptr, nullptr, 1.f);
-        } else {
-          if (pre_scale) stage_tile<HALO>(dst, x, n, y0, x0, H, W, Cin, up, pre_scale, pre_shift, slope, 128);
-          else stage_tile_async<HALO>(dst, x, n, y0, x0, H, W, Cin, up, 128);
-        }
+        if (cin_real != Cin) stage_tile_pad<HALO>(dst, x, n, y0, x0, H, W, Cin, cin_real, 128);
+        else if (fast_stage) stage_rows<HALO>(rs, dst, x, n, y0, x0, H, W, Cin);
+        else stage_tile_async<HALO>(dst, x, n, y0, x0, H, W, Cin, 128);
       }
       cp_async_commit();
     };
@@ -707,11 +550,11 @@ __global__ void __launch_bounds__(160) conv_tc_persist_kernel(const bf16* __rest
       tile_coords(j, n, y0, x0);
       mbar_wait(&acc_full[acc], (uint32_t)(j / NACC) & 1u);
       tc_fence_after_sync();
-      if (!out_f32 && (LEAN || cout_real == Cout))
+      if (!out_f32 && cout_real == Cout)
         conv_tc_epilogue_coalesced(tmem_base + (uint32_t)(acc * Cout), reinterpret_cast<uint8_t*>(full) + 256, warp, lane, n, y0, x0, H, W,
                                    Cout, bias, reinterpret_cast<bf16*>(y));
       else
-      conv_tc_epilogue<HALO>(tmem_base + (uint32_t)(acc * Cout), warp, tid, n, y0, x0, H, W, Cout, bias, y, out_f32, LEAN ? 0 : cout_real);
+      conv_tc_epilogue<HALO>(tmem_base + (uint32_t)(acc * Cout), warp, tid, n, y0, x0, H, W, Cout, bias, y, out_f32, cout_real);
       tc_fence_before_sync();
       mbar_arrive(&acc_empty[acc]);
     };
@@ -758,20 +601,20 @@ __global__ void __launch_bounds__(160) conv_tc_persist_kernel(const bf16* __rest
   if (warp == 4) tmem_dealloc(tmem_base, (uint32_t)tmem_cols);
 }
 
-template <int K, int NBUF, bool LEAN>
+template <int K, int NBUF>
 static int launch_conv_tc_persist(const void* x, const void* wp, const float* bias, void* y, int out_f32, int H, int W,
-                                  int Cin, int Cout, int up, const float* pre_scale, const float* pre_shift, float slope,
-                                  long long tiles, int psmem, int pcols, int per_sm, int cin_real, int cout_real, cudaStream_t st) {
+                                  int Cin, int Cout, long long tiles, int psmem, int pcols, int per_sm, int cin_real,
+                                  int cout_real, cudaStream_t st) {
   static int smem_set = 0;
   if (psmem > smem_set) {
-    cudaError_t e = cudaFuncSetAttribute(conv_tc_persist_kernel<K, NBUF, LEAN>, cudaFuncAttributeMaxDynamicSharedMemorySize, psmem);
+    cudaError_t e = cudaFuncSetAttribute(conv_tc_persist_kernel<K, NBUF>, cudaFuncAttributeMaxDynamicSharedMemorySize, psmem);
     if (e != cudaSuccess) return ttg_set_error(TTG_ERR_CUDA, "conv2d_tc: smem attribute: %s", cudaGetErrorString(e));
     smem_set = psmem;
   }
   long long grid = (long long)ttg_num_sms() * per_sm;
   if (grid > tiles) grid = tiles;
-  conv_tc_persist_kernel<K, NBUF, LEAN><<<(unsigned)grid, 160, psmem, st>>>((const bf16*)x, (const bf16*)wp, bias, y, out_f32, H, W, Cin,
-                                                                     Cout, up, pre_scale, pre_shift, slope, (int)tiles, pcols, cin_real, cout_real);
+  conv_tc_persist_kernel<K, NBUF><<<(unsigned)grid, 160, psmem, st>>>((const bf16*)x, (const bf16*)wp, bias, y, out_f32, H, W, Cin,
+                                                               Cout, (int)tiles, pcols, cin_real, cout_real);
   TTG_CHECK_LAUNCH("conv2d_tc_persist");
   return TTG_OK;
 }
@@ -783,8 +626,9 @@ static int launch_conv_tc_persist(const void* x, const void* wp, const float* bi
 // cp.async.bulk.tensor (TMA) instruction per tile: a rank-5 tensor map over the NHWC tensor viewed as
 // (8 channels, W, C/8, H, N) with box (8, WH, C/8, HH, 1) lands in shared memory exactly as the
 // [halo row][channel group][halo col] x 16 B image the UMMA descriptors expect, zero-filled outside the
-// image (the conv padding), completion counted in bytes on the slot's mbarrier.  warp 5 = TMA producer,
-// warp 4 = MMA issuer, warps 0-3 = epilogue only.
+// image (the conv padding), completion counted in bytes on the slot's mbarrier.  Layers with a compile-time
+// input channel count (CIN in {16, 32, 64}) use the pixel-major swizzled tile instead (see umma_desc_swz).
+// warp 5 = TMA producer, warp 4 = MMA issuer, warps 0-3 = epilogue only.
 #include <cuda.h>
 typedef CUresult (*ttg_encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                         const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
@@ -799,6 +643,10 @@ static ttg_encode_tiled_fn ttg_get_encode_tiled() {
   }
   return fn;
 }
+// Every driver that runs sm_100a exports cuTensorMapEncodeTiled; all tensor-core convolutions fetch their tiles with it.
+static int ttg_no_encode_tiled(const char* who) {
+  return ttg_set_error(TTG_ERR_UNSUPPORTED, "%s: the CUDA driver does not provide cuTensorMapEncodeTiled", who);
+}
 
 // accumulate flag as an immediate: with a compile-time input channel count every A descriptor of a tile is base + constant
 template <bool ACC>
@@ -809,16 +657,6 @@ __device__ __forceinline__ void umma_bf16_imm(uint32_t d_tmem, uint64_t adesc, u
   else
     asm volatile("{\n\t.reg .pred p;\n\tsetp.eq.u32 p, 1, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
                  ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc) : "memory");
-}
-// all K*K*CIN/16 MMAs of one tile, statically unrolled (weights resident: B advances by b_step per slice)
-template <int K, int CIN, int SL = 0>
-__device__ __forceinline__ void resident_issue_tile(uint32_t dacc, uint64_t a0, uint64_t b, uint32_t b_step, uint32_t idesc) {
-  constexpr int K16N = CIN / 16, C8N = CIN / 8, WH = TC_TW + 2 * (K / 2);
-  if constexpr (SL < K * K * K16N) {
-    constexpr int tap = SL / K16N, j = SL % K16N, ky = tap / K, kx = tap % K;
-    umma_bf16_imm<(SL > 0)>(dacc, a0 + (uint64_t)(ky * C8N * WH + kx + 2 * j * WH), b, idesc);
-    resident_issue_tile<K, CIN, SL + 1>(dacc, a0, b + b_step, b_step, idesc);
-  }
 }
 
 // Pixel-major ("NHWC as it lies in memory") activation tile for the A operand: halo pixel (hy, hx) at
@@ -837,6 +675,7 @@ __device__ __forceinline__ uint64_t umma_desc_sw(uint32_t smem_addr, uint32_t lb
          ((uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32) | (1ull << 46) | ((uint64_t)layout_type << 61);
 }
 __host__ __device__ __forceinline__ uint32_t umma_swz_layout_for(int channels) { return channels == 16 ? 6u : channels == 32 ? 4u : 2u; }
+// all K*K*CIN/16 MMAs of one tile, statically unrolled (weights resident: B advances by b_step per slice)
 template <int K, int CIN, int SL = 0>
 __device__ __forceinline__ void resident_issue_tile_swz(uint32_t dacc, uint64_t a0, uint64_t b, uint32_t b_step, uint32_t idesc) {
   constexpr int K16N = CIN / 16, WH = TC_TW + 2 * (K / 2);
@@ -847,17 +686,11 @@ __device__ __forceinline__ void resident_issue_tile_swz(uint32_t dacc, uint64_t 
   }
 }
 
-// PRE (needs the pixel-major swizzled tile, compile-time CIN): four extra warps apply the BatchNorm + LeakyReLU that
-// precedes the conv (a = lrelu(x * scale[c] + shift[c]); generator.py:38-47, discriminator.py:60-66) IN PLACE on the
-// tile the TMA engine has just delivered, before the MMAs read it; pixels outside the image keep the TMA's zero fill
-// (the reference pads the activation, not x).  The separate BatchNorm-apply pass over the tensor disappears.
-template <int K, int NBUF, int CIN, bool STATS, bool PRE = false>
-__global__ void __launch_bounds__(PRE ? 320 : 192) conv_tc_tma_kernel(const __grid_constant__ CUtensorMap tmap, const bf16* __restrict__ wp,
+template <int K, int NBUF, int CIN, bool STATS>
+__global__ void __launch_bounds__(192) conv_tc_tma_kernel(const __grid_constant__ CUtensorMap tmap, const bf16* __restrict__ wp,
                                                           const float* __restrict__ bias, void* __restrict__ y, int out_f32,
                                                           int H, int W, int Cin_rt, int Cout, int total_tiles, int tmem_cols,
-                                                          int mode, int cstore, double* __restrict__ stats, int swz,
-                                                          const float* __restrict__ pre_scale = nullptr,
-                                                          const float* __restrict__ pre_shift = nullptr, float slope = 1.f) {
+                                                          int cstore, double* __restrict__ stats) {
   constexpr int HALO = K / 2, WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO, HP = WH * HH;
   constexpr int NACC = 4;
   extern __shared__ __align__(128) uint8_t smem[];
@@ -873,8 +706,7 @@ __global__ void __launch_bounds__(PRE ? 320 : 192) conv_tc_tma_kernel(const __gr
   uint64_t* empty = full + NBUF;
   uint64_t* acc_full = empty + NBUF;
   uint64_t* acc_empty = acc_full + NACC;
-  uint64_t* ready = acc_empty + NACC;                                         // PRE: tile transformed in place (128 arrivals)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(ready + NBUF);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + NACC);
 
   const int tiles_x = (W + TC_TW - 1) / TC_TW, tiles_y = (H + TC_TH - 1) / TC_TH, tiles_img = tiles_x * tiles_y;
   const int T = (total_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
@@ -891,7 +723,7 @@ __global__ void __launch_bounds__(PRE ? 320 : 192) conv_tc_tma_kernel(const __gr
     for (int i = tid; i < 2 * Cout; i += blockDim.x) s_stats[i] = 0.f;
   if (warp == 4) tmem_alloc(tmem_slot, (uint32_t)tmem_cols);
   if (tid == 0) {
-    for (int i = 0; i < NBUF; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); mbar_init(&ready[i], 128); }
+    for (int i = 0; i < NBUF; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
     for (int i = 0; i < NACC; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 128); }
     mbar_fence_init();
   }
@@ -920,23 +752,7 @@ __global__ void __launch_bounds__(PRE ? 320 : 192) conv_tc_tma_kernel(const __gr
       if (warp == 0) mbar_wait(&acc_full[acc], (uint32_t)(j / NACC) & 1u);
       asm volatile("bar.sync 1, 128;" ::: "memory");
       tc_fence_after_sync();
-      if (mode == 1) {       // TIMING EXPERIMENT: stores as a [N][H][C/8][W][8] layout would issue them
-        const uint32_t tacc = tmem_base + (uint32_t)(acc * Cout);
-        const int gy = y0 + (tid >> 3), gx = x0 + (tid & 7);
-        for (int c0 = 0; c0 < Cout; c0 += 16) {
-          uint32_t r[16];
-          tmem_ld16(tacc + ((uint32_t)(warp * 32) << 16) + (uint32_t)c0, r);
-          tmem_ld_wait();
-          if (gy < H && gx < W) {
-            uint4 o[2];
-            __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(o);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) h[j] = __floats2bfloat162_rn(__uint_as_float(r[2 * j]), __uint_as_float(r[2 * j + 1]));
-            uint4* dst = reinterpret_cast<uint4*>(y) + (((long long)n * H + gy) * (Cout >> 3) + (c0 >> 3)) * W + gx;
-            dst[0] = o[0]; dst[W] = o[1];
-          }
-        }
-      } else if (!out_f32)
+      if (!out_f32)
         conv_tc_epilogue_coalesced(tmem_base + (uint32_t)(acc * Cout), reinterpret_cast<uint8_t*>(full) + 512, warp, lane, n, y0, x0, H, W,
                                    cstore, bias, reinterpret_cast<bf16*>(y), STATS ? s_stats : nullptr,
                                    (STATS && reg_stats) ? &est : nullptr);
@@ -953,19 +769,16 @@ __global__ void __launch_bounds__(PRE ? 320 : 192) conv_tc_tma_kernel(const __gr
     const uint32_t b_step = slice_bytes >> 4;
     for (int it = 0; it < T; ++it) {
       const int s = it % NBUF, acc = it & (NACC - 1);
-      mbar_wait(PRE ? &ready[s] : &full[s], (uint32_t)(it / NBUF) & 1u);
+      mbar_wait(&full[s], (uint32_t)(it / NBUF) & 1u);
       if (it >= NACC) mbar_wait(&acc_empty[acc], (uint32_t)((it / NACC) - 1) & 1u);
       tc_fence_after_sync();
       if (elect_one()) {
-        const uint64_t a0 = umma_desc(smem_u32(sA + (size_t)s * a_bytes), WH * 16, c8n * WH * 16);
         const uint32_t dacc = tmem_base + (uint32_t)(acc * Cout);
         if constexpr (CIN > 0) {
-          if (swz) {
-            const uint64_t a0s = umma_desc_swz(smem_u32(sA + (size_t)s * a_bytes), (uint32_t)(WH * CIN * 2), (uint32_t)swz);
-            resident_issue_tile_swz<K, CIN>(dacc, a0s, b0, b_step, idesc);
-          } else
-          resident_issue_tile<K, CIN>(dacc, a0, b0, b_step, idesc);
+          const uint64_t a0 = umma_desc_swz(smem_u32(sA + (size_t)s * a_bytes), (uint32_t)(WH * CIN * 2), umma_swz_layout_for(CIN));
+          resident_issue_tile_swz<K, CIN>(dacc, a0, b0, b_step, idesc);
         } else {
+          const uint64_t a0 = umma_desc(smem_u32(sA + (size_t)s * a_bytes), WH * 16, c8n * WH * 16);
           uint32_t sl = 0;
 #pragma unroll
           for (int tap = 0; tap < K * K; ++tap) {
@@ -979,43 +792,6 @@ __global__ void __launch_bounds__(PRE ? 320 : 192) conv_tc_tma_kernel(const __gr
       }
       __syncwarp();
     }
-  } else if (PRE && warp >= 6) {
-    // ------------------------------------------------------------ in-place BatchNorm + LeakyReLU on the delivered tile
-    if constexpr (PRE && CIN > 0) {
-      constexpr int C8N = CIN / 8, PSTEP = 128 / C8N;
-      const int tt = tid - 192, lc = tt % C8N, p0 = tt / C8N;       // this thread's (logical) channel group: fixed
-      float sc[8], sh[8];
-#pragma unroll
-      for (int k = 0; k < 8; ++k) { sc[k] = __ldg(pre_scale + lc * 8 + k); sh[k] = __ldg(pre_shift + lc * 8 + k); }
-      for (int j = 0; j < T; ++j) {
-        const int s = j % NBUF;
-        if (warp == 6) mbar_wait(&full[s], (uint32_t)(j / NBUF) & 1u);
-        asm volatile("bar.sync 2, 128;" ::: "memory");
-        int n, y0, x0;
-        tile_coords(j, n, y0, x0);
-        const uint32_t sa = smem_u32(sA + (size_t)s * a_bytes);
-        for (int p = p0; p < HP; p += PSTEP) {
-          const int hy = p / WH, hx = p - hy * WH;
-          const int gy = y0 + hy - HALO, gx = x0 + hx - HALO;
-          if (gy < 0 || gy >= H || gx < 0 || gx >= W) continue;      // zero fill = the conv's padding of the ACTIVATION
-          const uint32_t pa = sa + (uint32_t)p * (CIN * 2);
-          const uint32_t ua = pa + (uint32_t)((lc ^ (int)((pa >> 7) & (C8N - 1))) << 4);   // swizzled home of chunk lc
-          uint4 v;
-          asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(ua));
-          __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&v);
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            float2 f = __bfloat1622float2(h[q]);
-            f.x = lrelu(f.x * sc[2 * q] + sh[2 * q], slope);
-            f.y = lrelu(f.y * sc[2 * q + 1] + sh[2 * q + 1], slope);
-            h[q] = __floats2bfloat162_rn(f.x, f.y);
-          }
-          asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(ua), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-        }
-        fence_proxy_async_smem();
-        mbar_arrive(&ready[s]);
-      }
-    }
   } else if (warp == 5 && elect_one()) {
     // ------------------------------------------------------------ TMA producer (warp 5, one lane)
     for (int j = 0; j < T; ++j) {
@@ -1025,20 +801,15 @@ __global__ void __launch_bounds__(PRE ? 320 : 192) conv_tc_tma_kernel(const __gr
       tile_coords(j, n, y0, x0);
       const uint32_t bar = smem_u32(&full[s]);
       asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(a_bytes) : "memory");
-      if (swz)
+      if constexpr (CIN > 0)
       asm volatile(
           "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
           ::"r"(smem_u32(sA + (size_t)s * a_bytes)), "l"(&tmap), "r"(0), "r"(x0 - HALO), "r"(y0 - HALO), "r"(n), "r"(bar)
           : "memory");
-      else if (mode == 0)
+      else
       asm volatile(
           "cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5, %6}], [%7];"
           ::"r"(smem_u32(sA + (size_t)s * a_bytes)), "l"(&tmap), "r"(0), "r"(x0 - HALO), "r"(0), "r"(y0 - HALO), "r"(n), "r"(bar)
-          : "memory");
-      else
-      asm volatile(
-          "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
-          ::"r"(smem_u32(sA + (size_t)s * a_bytes)), "l"(&tmap), "r"(mode == 1 ? (x0 - HALO) * 8 : 0), "r"(mode == 1 ? 0 : x0 - HALO), "r"(y0 - HALO), "r"(n), "r"(bar)
           : "memory");
     }
   }
@@ -1049,56 +820,34 @@ __global__ void __launch_bounds__(PRE ? 320 : 192) conv_tc_tma_kernel(const __gr
     for (int i = tid; i < 2 * Cout; i += blockDim.x) atomicAdd(&stats[i], (double)s_stats[i]);
 }
 
-static int g_persm_cap = 0;     // experiment: cap on resident CTAs per SM of the TMA conv kernel (0 = none)
-extern "C" int ttg_set_persm_cap(int n) { g_persm_cap = n; return TTG_OK; }
-static int g_nbuf_exp = 0;      // experiment: deeper activation rings (8 / 6 slots) for the 16 / 32-channel layers
-extern "C" int ttg_set_nbuf_exp(int on) { g_nbuf_exp = on; return TTG_OK; }
-static int g_use_swz = 1;       // A/B switch: pixel-major swizzled activation tiles in the TMA-fed conv kernel
-extern "C" int ttg_set_use_swz(int on) { g_use_swz = on ? 1 : 0; return TTG_OK; }
-static int g_use_tma = 1;       // 1: NHWC rank-5 map; 2/3: TIMING EXPERIMENTS (blocked layout / pixel-major rows; results are not a convolution)
 template <int K, int NBUF, int CIN>
 static int launch_conv_tc_tma(const void* x, const void* wp, const float* bias, void* y, int out_f32, int N, int H, int W,
                               int Cin, int Cout, int cin_mem, int cstore, long long tiles, int w_bytes, int a_bytes, int pcols,
-                              double* stats, cudaStream_t st, bool* used, const float* pre_scale = nullptr,
-                              const float* pre_shift = nullptr, float slope = 1.f) {
-  *used = false;
-  ttg_encode_tiled_fn enc = ttg_get_encode_tiled();
-  if (!enc) return TTG_OK;
+                              double* stats, cudaStream_t st) {
+  const ttg_encode_tiled_fn enc = ttg_get_encode_tiled();
+  if (!enc) return ttg_no_encode_tiled("conv2d_tc");
   constexpr int HALO = K / 2;
   CUtensorMap tmap;
-  // cin_mem = channels per pixel in memory (Cin, or 8 for the RGB staging tensors: the box still asks for Cin / 8
-  // channel groups and the groups that do not exist are zero-filled by the TMA engine, like the spatial halo)
-  const cuuint64_t gdim[5] = {8, (cuuint64_t)W, (cuuint64_t)(cin_mem / 8), (cuuint64_t)H, (cuuint64_t)N};
-  const cuuint64_t gstr[4] = {(cuuint64_t)cin_mem * 2, 16, (cuuint64_t)W * cin_mem * 2, (cuuint64_t)H * W * cin_mem * 2};
-  const cuuint32_t box[5] = {8, (cuuint32_t)(TC_TW + 2 * HALO), (cuuint32_t)(Cin / 8), (cuuint32_t)(TC_TH + 2 * HALO), 1};
   const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
   CUresult r;
-  int mode = g_use_tma - 1;
-  // pixel-major swizzled tile (see umma_desc_swz): compile-time channel counts 16 / 32 / 64 only
-  const int swz = (g_use_swz && CIN > 0 && mode == 0) ? (CIN == 16 ? 6 : CIN == 32 ? 4 : 2) : 0;
-  if (swz) {
+  if constexpr (CIN > 0) {
+    // pixel-major swizzled tile (see umma_desc_swz).  cin_mem = channels per pixel in memory (Cin, or 8 for the RGB
+    // staging tensors: the box still asks for Cin channels and those that do not exist are zero-filled by the TMA
+    // engine, like the spatial halo)
     const cuuint64_t d4[4] = {(cuuint64_t)cin_mem, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
     const cuuint64_t s4[3] = {(cuuint64_t)cin_mem * 2, (cuuint64_t)W * cin_mem * 2, (cuuint64_t)H * W * cin_mem * 2};
     const cuuint32_t b4[4] = {(cuuint32_t)Cin, (cuuint32_t)(TC_TW + 2 * HALO), (cuuint32_t)(TC_TH + 2 * HALO), 1};
     r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), d4, s4, b4, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
             CIN == 16 ? CU_TENSOR_MAP_SWIZZLE_32B : CIN == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
             CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  } else if (mode == 1) {
-    const cuuint64_t d4[4] = {(cuuint64_t)W * 8, (cuuint64_t)(Cin / 8), (cuuint64_t)H, (cuuint64_t)N};
-    const cuuint64_t s4[3] = {(cuuint64_t)W * 16, (cuuint64_t)(Cin / 8) * W * 16, (cuuint64_t)H * (Cin / 8) * W * 16};
-    const cuuint32_t b4[4] = {(cuuint32_t)(TC_TW + 2 * HALO) * 8, (cuuint32_t)(Cin / 8), (cuuint32_t)(TC_TH + 2 * HALO), 1};
-    r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), d4, s4, b4, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  } else if (mode == 2) {
-    const cuuint64_t d4[4] = {(cuuint64_t)Cin, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-    const cuuint64_t s4[3] = {(cuuint64_t)Cin * 2, (cuuint64_t)W * Cin * 2, (cuuint64_t)H * W * Cin * 2};
-    const cuuint32_t b4[4] = {(cuuint32_t)Cin, (cuuint32_t)(TC_TW + 2 * HALO), (cuuint32_t)(TC_TH + 2 * HALO), 1};
-    r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), d4, s4, b4, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  } else
-  r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  } else {
+    const cuuint64_t gdim[5] = {8, (cuuint64_t)W, (cuuint64_t)(cin_mem / 8), (cuuint64_t)H, (cuuint64_t)N};
+    const cuuint64_t gstr[4] = {(cuuint64_t)cin_mem * 2, 16, (cuuint64_t)W * cin_mem * 2, (cuuint64_t)H * W * cin_mem * 2};
+    const cuuint32_t box[5] = {8, (cuuint32_t)(TC_TW + 2 * HALO), (cuuint32_t)(Cin / 8), (cuuint32_t)(TC_TH + 2 * HALO), 1};
+    r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), gdim, gstr, box, estr,
+            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  }
   if (r != CUDA_SUCCESS) return ttg_set_error(TTG_ERR_CUDA, "conv2d_tc: cuTensorMapEncodeTiled failed (%d)", (int)r);
   const int smem = ((w_bytes + 127) & ~127) + NBUF * a_bytes + 512 + tc_epi_bytes(Cout);     // 512: mbarriers (up to 8 slots) + TMEM slot
   static int smem_set = 0;
@@ -1111,49 +860,23 @@ static int launch_conv_tc_tma(const void* x, const void* wp, const float* bias, 
   int per_sm = (200 * 1024) / smem;
   if (per_sm > 512 / pcols) per_sm = 512 / pcols;
   if (per_sm > 8) per_sm = 8;
-  if (g_persm_cap > 0 && per_sm > g_persm_cap) per_sm = g_persm_cap;
   if (per_sm < 1) per_sm = 1;
-  if (pre_scale) {
-    if constexpr (CIN > 0) {
-      if (!swz) return TTG_OK;                 // (*used stays false: the caller takes another path)
-      static int smem_set_pre = 0;
-      if (smem > smem_set_pre) {
-        cudaError_t e = cudaFuncSetAttribute(conv_tc_tma_kernel<K, NBUF, CIN, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_tma_kernel<K, NBUF, CIN, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return ttg_set_error(TTG_ERR_CUDA, "conv2d_tc: smem attribute: %s", cudaGetErrorString(e));
-        smem_set_pre = smem;
-      }
-      if (per_sm > 6) per_sm = 6;              // 320 threads per CTA
-      long long gridp = (long long)ttg_num_sms() * per_sm;
-      if (gridp > tiles) gridp = tiles;
-      if (stats)
-        conv_tc_tma_kernel<K, NBUF, CIN, true, true><<<(unsigned)gridp, 320, smem, st>>>(tmap, (const bf16*)wp, bias, y, out_f32, H, W, Cin, Cout,
-                                                                             (int)tiles, pcols, mode, cstore, stats, swz, pre_scale, pre_shift, slope);
-      else
-        conv_tc_tma_kernel<K, NBUF, CIN, false, true><<<(unsigned)gridp, 320, smem, st>>>(tmap, (const bf16*)wp, bias, y, out_f32, H, W, Cin, Cout,
-                                                                              (int)tiles, pcols, mode, cstore, stats, swz, pre_scale, pre_shift, slope);
-      TTG_CHECK_LAUNCH("conv2d_tc_tma_pre");
-      *used = true;
-    }
-    return TTG_OK;
-  }
   long long grid = (long long)ttg_num_sms() * per_sm;
   if (grid > tiles) grid = tiles;
   if (stats)
     conv_tc_tma_kernel<K, NBUF, CIN, true><<<(unsigned)grid, 192, smem, st>>>(tmap, (const bf16*)wp, bias, y, out_f32, H, W, Cin, Cout,
-                                                                        (int)tiles, pcols, mode, cstore, stats, swz);
+                                                                        (int)tiles, pcols, cstore, stats);
   else
     conv_tc_tma_kernel<K, NBUF, CIN, false><<<(unsigned)grid, 192, smem, st>>>(tmap, (const bf16*)wp, bias, y, out_f32, H, W, Cin, Cout,
-                                                                         (int)tiles, pcols, mode, cstore, stats, swz);
+                                                                         (int)tiles, pcols, cstore, stats);
   TTG_CHECK_LAUNCH("conv2d_tc_tma");
-  *used = true;
   return TTG_OK;
 }
 
 // ------------------------------------------------------------------ fprop / dgrad, filters too large for shared memory
-// (128->128, 256->256 ...): persistent, warp-specialised, weights STREAMED.  warps 0-3 stage activation tiles
-// (cp.async, NA slots) and run the epilogue; warp 4 issues tcgen05.mma; warp 5 streams the packed filter from L2
-// through a ring of NW 16 KB stages (cp.async) for every tile.  These layers are tensor/L2 bound, not HBM bound.
+// (128->128, 256->256 ...): persistent, warp-specialised, weights STREAMED.  warps 0-3 run the epilogue; warp 4 issues
+// tcgen05.mma; warp 5 fetches the activation tiles (tensor-map loads, NA slots) and streams the packed filter from L2
+// through a ring of NW 16 KB stages for every tile.  These layers are tensor/L2 bound, not HBM bound.
 #define TC_WSTAGE_BYTES (16 * 1024)
 #ifdef TTG_TRACE
 // development build only: per-event clock64() stamps of CTA 0 (role, index, t0, t1)
@@ -1190,10 +913,10 @@ __device__ __forceinline__ void stream_issue_chunk(uint32_t dacc, uint64_t a0, u
 
 // CIN / COUT > 0: 3x3 layer with compile-time channel counts (lean, fully unrolled issue sequence);
 // CIN == 0: any supported layer, runtime walk.
-template <int K, int NA, bool TMA_A, int CIN, int COUT>
-__global__ void __launch_bounds__(192) conv_tc_stream_ws_kernel(const bf16* __restrict__ x, const bf16* __restrict__ wp,
+template <int K, int NA, int CIN, int COUT>
+__global__ void __launch_bounds__(192) conv_tc_stream_ws_kernel(const bf16* __restrict__ wp,
                                                                 const float* __restrict__ bias, void* __restrict__ y,
-                                                                int out_f32, int H, int W, int Cin_rt, int Cout_rt, int up,
+                                                                int out_f32, int H, int W, int Cin_rt, int Cout_rt,
                                                                 int total_tiles, int tmem_cols, int chunk_slices_rt,
                                                                 const __grid_constant__ CUtensorMap tmap,
                                                                 double* __restrict__ stats) {
@@ -1237,7 +960,7 @@ __global__ void __launch_bounds__(192) conv_tc_stream_ws_kernel(const bf16* __re
     for (int i = tid; i < 2 * Cout; i += blockDim.x) s_stats[i] = 0.f;
   if (warp == 4) tmem_alloc(tmem_slot, (uint32_t)tmem_cols);
   if (tid == 0) {
-    for (int i = 0; i < NA; ++i) { mbar_init(&afull[i], TMA_A ? 1 : 128); mbar_init(&aempty[i], 1); }
+    for (int i = 0; i < NA; ++i) { mbar_init(&afull[i], 1); mbar_init(&aempty[i], 1); }
     for (int i = 0; i < NW; ++i) { mbar_init(&wfull[i], 1); mbar_init(&wempty[i], 1); }
     for (int i = 0; i < NACC; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 128); }
     mbar_fence_init();
@@ -1248,18 +971,8 @@ __global__ void __launch_bounds__(192) conv_tc_stream_ws_kernel(const bf16* __re
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp < 4) {
-    // ------------------------------------------------------------ activation tiles + epilogue
-    auto stage = [&](int j) {
-      if (j < T) {
-        const int s = j % NA;
-        if (j >= NA) mbar_wait(&aempty[s], (uint32_t)((j / NA) - 1) & 1u);
-        int n, y0, x0;
-        tile_coords(j, n, y0, x0);
-        stage_tile_async<HALO>(sA + (size_t)s * a_bytes, x, n, y0, x0, H, W, Cin, up, 128);
-      }
-      cp_async_commit();
-    };
-    auto epilogue = [&](int j) {
+    // ------------------------------------------------------------ epilogue (tiles arrive by TMA, warp 5)
+    for (int j = 0; j < T; ++j) {
       const int acc = j % NACC;
       int n, y0, x0;
       tile_coords(j, n, y0, x0);
@@ -1274,23 +987,6 @@ __global__ void __launch_bounds__(192) conv_tc_stream_ws_kernel(const bf16* __re
       tc_fence_before_sync();
       mbar_arrive(&acc_empty[acc]);
       if (tid == 0) { TTG_T1(6, j); }
-    };
-    if constexpr (TMA_A) {
-      for (int j = 0; j < T; ++j) epilogue(j);          // tiles arrive by TMA (warp 5)
-    } else {
-      // tile `it` is published BEFORE the loads of tile it+1 are issued, so the MMAs of a tile never wait for
-      // the (instruction-heavy) staging of its successor
-      stage(0);
-      for (int it = 0; it < T; ++it) {
-        cp_async_wait_group<0>();
-        fence_proxy_async_smem();
-        mbar_arrive(&afull[it % NA]);
-        if (NA > 1) stage(it + 1);
-        if (it > 0) epilogue(it - 1);
-        if (NA == 1) stage(it + 1);
-      }
-      if (T > 0) epilogue(T - 1);
-      cp_async_wait_all();
     }
   } else if (warp == 4) {
     // ------------------------------------------------------------ MMA issuer
@@ -1362,7 +1058,7 @@ __global__ void __launch_bounds__(192) conv_tc_stream_ws_kernel(const bf16* __re
   } else {
     // ------------------------------------------------------------ producer (warp 5, one lane)
     // weights: cp.async.bulk (TMA 1-D bulk copy), one instruction per 16 KB stage, completion counted in bytes on
-    // the stage's mbarrier, NW stages in flight; activation halo tiles (TMA_A): one tensor-map load per tile.
+    // the stage's mbarrier, NW stages in flight; activation halo tiles: one tensor-map load per tile.
     if (elect_one()) {
       const uint32_t G = (uint32_t)T * (uint32_t)nchunks;
       const uint32_t chunk_bytes = (uint32_t)chunk_slices * slice_bytes;
@@ -1389,7 +1085,7 @@ __global__ void __launch_bounds__(192) conv_tc_stream_ws_kernel(const bf16* __re
       // pieces of the next tile start once the ring has turned over (its slot is then known to be free: NA == 2),
       // or after the last stage when there is a single activation slot
       const int c_first = NA > 1 ? min(NW, nchunks - 1) : nchunks - 1;
-      if (TMA_A && T > 0)
+      if (T > 0)
         for (int pc = 0; pc < APIECES; ++pc) issue_a_piece(0, pc);
       int c = 0, tile = 0, piece = 0;
       for (uint32_t g = 0; g < G; ++g) {
@@ -1401,7 +1097,7 @@ __global__ void __launch_bounds__(192) conv_tc_stream_ws_kernel(const bf16* __re
         asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
         asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                      ::"r"(sW_addr + ws * WSB), "l"(src), "r"(bytes), "r"(bar) : "memory");
-        if (TMA_A && tile + 1 < T && c >= c_first) {
+        if (tile + 1 < T && c >= c_first) {
           if (piece < APIECES) issue_a_piece(tile + 1, piece++);
           if (c == nchunks - 1)
             while (piece < APIECES) issue_a_piece(tile + 1, piece++);
@@ -1419,555 +1115,38 @@ __global__ void __launch_bounds__(192) conv_tc_stream_ws_kernel(const bf16* __re
 
 template <int K, int NA, int CIN, int COUT>
 static int launch_conv_tc_stream_ws(const void* x, const void* wp, const float* bias, void* y, int out_f32, int N, int H, int W,
-                                    int Cin, int Cout, int up, long long tiles, double* stats, cudaStream_t st) {
+                                    int Cin, int Cout, long long tiles, double* stats, cudaStream_t st) {
+  const ttg_encode_tiled_fn enc = ttg_get_encode_tiled();
+  if (!enc) return ttg_no_encode_tiled("conv2d_tc");
   constexpr int HALO = K / 2;
   const int HP = (TC_TW + 2 * HALO) * (TC_TH + 2 * HALO);
   constexpr int NW = CIN > 0 ? 3 : 4, WSB = CIN > 0 ? 2 * TC_WSTAGE_BYTES : TC_WSTAGE_BYTES;
   constexpr int APIECES = K == 3 ? 6 : 4;
   const int smem = NA * (Cin / 8) * HP * 16 + NW * WSB + 256 + tc_epi_bytes(Cout);
   CUtensorMap tmap;
-  memset(&tmap, 0, sizeof(tmap));
-  ttg_encode_tiled_fn enc = (g_use_tma && up == 0) ? ttg_get_encode_tiled() : nullptr;
-  if (enc) {
-    const cuuint64_t gdim[5] = {8, (cuuint64_t)W, (cuuint64_t)(Cin / 8), (cuuint64_t)H, (cuuint64_t)N};
-    const cuuint64_t gstr[4] = {(cuuint64_t)Cin * 2, 16, (cuuint64_t)W * Cin * 2, (cuuint64_t)H * W * Cin * 2};
-    const cuuint32_t box[5] = {8, (cuuint32_t)(TC_TW + 2 * HALO), (cuuint32_t)(Cin / 8), (cuuint32_t)((TC_TH + 2 * HALO) / APIECES), 1};
-    const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    CUresult r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), gdim, gstr, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return ttg_set_error(TTG_ERR_CUDA, "conv2d_tc: cuTensorMapEncodeTiled failed (%d)", (int)r);
-  }
-  static int smem_set[2] = {0, 0};
-  if (smem > smem_set[enc ? 1 : 0]) {
-    cudaError_t e = enc ? cudaFuncSetAttribute(conv_tc_stream_ws_kernel<K, NA, true, CIN, COUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)
-                        : cudaFuncSetAttribute(conv_tc_stream_ws_kernel<K, NA, false, CIN, COUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  const cuuint64_t gdim[5] = {8, (cuuint64_t)W, (cuuint64_t)(Cin / 8), (cuuint64_t)H, (cuuint64_t)N};
+  const cuuint64_t gstr[4] = {(cuuint64_t)Cin * 2, 16, (cuuint64_t)W * Cin * 2, (cuuint64_t)H * W * Cin * 2};
+  const cuuint32_t box[5] = {8, (cuuint32_t)(TC_TW + 2 * HALO), (cuuint32_t)(Cin / 8), (cuuint32_t)((TC_TH + 2 * HALO) / APIECES), 1};
+  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+  CUresult r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), gdim, gstr, box, estr,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) return ttg_set_error(TTG_ERR_CUDA, "conv2d_tc: cuTensorMapEncodeTiled failed (%d)", (int)r);
+  static int smem_set = 0;
+  if (smem > smem_set) {
+    cudaError_t e = cudaFuncSetAttribute(conv_tc_stream_ws_kernel<K, NA, CIN, COUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return ttg_set_error(TTG_ERR_CUDA, "conv2d_tc: smem attribute: %s", cudaGetErrorString(e));
-    smem_set[enc ? 1 : 0] = smem;
+    smem_set = smem;
   }
   int chunk_slices = WSB / (Cout * 32);
   if (chunk_slices < 1) chunk_slices = 1;
   const int cols = (int)tmem_cols_for(2 * Cout);
   long long grid = ttg_num_sms();
   if (grid > tiles) grid = tiles;
-  if (enc)
-    conv_tc_stream_ws_kernel<K, NA, true, CIN, COUT><<<(unsigned)grid, 192, smem, st>>>(
-        (const bf16*)x, (const bf16*)wp, bias, y, out_f32, H, W, Cin, Cout, up, (int)tiles, cols, chunk_slices, tmap, stats);
-  else
-    conv_tc_stream_ws_kernel<K, NA, false, CIN, COUT><<<(unsigned)grid, 192, smem, st>>>(
-        (const bf16*)x, (const bf16*)wp, bias, y, out_f32, H, W, Cin, Cout, up, (int)tiles, cols, chunk_slices, tmap, stats);
+  conv_tc_stream_ws_kernel<K, NA, CIN, COUT><<<(unsigned)grid, 192, smem, st>>>(
+      (const bf16*)wp, bias, y, out_f32, H, W, Cin, Cout, (int)tiles, cols, chunk_slices, tmap, stats);
   TTG_CHECK_LAUNCH("conv2d_tc_stream_ws");
   return TTG_OK;
-}
-
-static int g_conv_tc_smem[2] = {0, 0};
-extern "C" int ttg_set_use_tma(int on) {
-#ifdef TTG_TRACE      // development builds only: 2 / 3 are the layout TIMING experiments (results are not a convolution)
-  g_use_tma = on;
-#else
-  if (on != 0 && on != 1) return ttg_set_error(TTG_ERR_ARG, "set_use_tma: %d is a development-build experiment (0 or 1 here)", on);
-  g_use_tma = on;
-#endif
-  return TTG_OK;
-}
-
-
-// ------------------------------------------------------------------ fprop / dgrad, horizontal taps folded into N
-// Small-channel 3x3 layers are bound by the tensor pipe's operand fetch, not by HBM: an SS-mode 128 x 16 x 16 MMA
-// occupies the pipe ~57 cycles (4 KB A fragment from shared memory) and the tap-shift scheme needs 9 of them per
-// 128 pixels.  Here the three horizontal taps are folded into the N dimension:
-//     D[p, (kx, co)] = sum_{ky, ci} X[p + (ky-1) rows, ci] * Wf[(ky, ci), (kx, co)]          3 MMAs (N = 3 Cout) per k16
-//     out[x, co]     = D[x-1, (0, co)] + D[x, (1, co)] + D[x+1, (2, co)]                      shift-and-add in the epilogue
-// A tile is 4 full image rows (M groups of 128 consecutive pixels = 128 / W rows, W <= 128), so the x-neighbours of a
-// pixel are the neighbouring TMEM lanes (warp shuffles; warp-boundary values through shared memory) and image borders
-// are the conv's zero padding.  The activation tile [channel/8][6 rows][W] needs no horizontal halo: the vertical
-// taps are descriptor start addresses one row apart.  The packed filter [tap][ci/8][co][8] is re-ordered to
-// [ky][ci/8][(kx, co)][8] while it is copied into shared memory, so callers pass the usual packed weights.
-template <int CIN, int COUT, int W>
-__global__ void __launch_bounds__((4 * (4 / (128 / W)) + 2) * 32) conv_tc_fold_kernel(const __grid_constant__ CUtensorMap tmap, const bf16* __restrict__ wp,
-                                                           const float* __restrict__ bias, bf16* __restrict__ y, int H,
-                                                           int total_tiles, int cstore) {
-  constexpr int C8N = CIN / 8, K16N = CIN / 16, NF = 3 * COUT;
-  constexpr int R = 128 / W, G = 4 / R, HY = 6;                  // rows per M group, M groups per tile, tile rows incl. halo
-  constexpr int NBUF = 3, NACC = 2;
-  constexpr uint32_t A_BYTES = (uint32_t)C8N * HY * W * 16;
-  constexpr uint32_t W_BYTES = 9u * K16N * COUT * 32;
-  static_assert(128 % W == 0 && W >= 32 && 4 % R == 0, "row tiles: W in {32, 64, 128}");
-  static_assert(NACC * G * NF <= 512, "TMEM columns");
-  extern __shared__ __align__(128) uint8_t smem[];
-  uint8_t* sW = smem;
-  uint8_t* sA = smem + ((W_BYTES + 127) & ~127u);
-  uint64_t* full = reinterpret_cast<uint64_t*>(sA + NBUF * (size_t)A_BYTES);
-  uint64_t* empty = full + NBUF;
-  uint64_t* acc_full = empty + NBUF;
-  uint64_t* acc_empty = acc_full + NACC;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + NACC);
-  float* xch = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(full) + 256);       // [G sets][2 parity][4 warps][2][16]
-  constexpr int EPI_WARPS = 4 * G;          // one set of 4 epilogue warps per M group: a lone warp per scheduler cannot
-                                            // hide its own instruction latencies (measured 3100 cycles per group)
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int tiles_img = (H + 3) / 4;
-  const int T = (total_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-
-  if (warp == EPI_WARPS) tmem_alloc(tmem_slot, 512u);
-  if (tid == 0) {
-    for (int i = 0; i < NBUF; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-    for (int i = 0; i < NACC; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 128 * G); }
-    mbar_fence_init();
-  }
-  if (warp < EPI_WARPS) {
-    // packed filter unit (tap, c8, co) -> folded unit ((ky * C8N + c8) * 3 + kx) * COUT + co
-    for (int u = tid; u < 9 * C8N * COUT; u += 32 * EPI_WARPS) {
-      const int co = u % COUT, c8 = (u / COUT) % C8N, tap = u / (COUT * C8N);
-      const int ky = tap / 3, kx = tap - ky * 3;
-      reinterpret_cast<uint4*>(sW)[((ky * C8N + c8) * 3 + kx) * COUT + co] = __ldg(reinterpret_cast<const uint4*>(wp) + u);
-    }
-  }
-  fence_proxy_async_smem();
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp < EPI_WARPS) {
-    // ------------------------------------------------------------ epilogue: shift-and-add of the three kx blocks
-    const int g = warp >> 2, q = warp & 3;                        // M group of this warp set, TMEM lane quadrant
-    const int m = q * 32 + lane;                                  // pixel of the M group = TMEM lane
-    const int r = m / W, xx = m - r * W;
-    const bool has_left = xx > 0, has_right = xx < W - 1;
-    float* xs = xch + g * (2 * 4 * 2 * 16);
-    // W is a multiple of 32: a row starts at lane 0 and ends at lane 31, so only those lanes can sit on an image
-    // border, and they are also the only lanes that take their neighbour from the exchange buffer
-    const bool edge_l = lane == 0, edge_r = lane == 31;
-    float bv[COUT];
-#pragma unroll
-    for (int k = 0; k < COUT; ++k) bv[k] = bias ? __ldg(bias + k) : 0.f;
-    int par = 0;
-    for (int j = 0; j < T; ++j) {
-      const int acc = j & (NACC - 1);
-      const int tile = blockIdx.x + j * gridDim.x;
-      const int n = tile / tiles_img, y0 = (tile - n * tiles_img) * 4;
-      { TTG_T0(); mbar_wait(&acc_full[acc], (uint32_t)(j / NACC) & 1u); if (tid == 0) { TTG_T1(5, j); } }
-      tc_fence_after_sync();
-      TTG_T0();
-      const int row = y0 + g * R + r;
-      const uint32_t tcol = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)((acc * G + g) * NF);
-      bf16* yrow = y + (((long long)n * H + row) * W + xx) * (cstore == 8 ? 8 : COUT);
-#pragma unroll
-      for (int c0 = 0; c0 < COUT; c0 += 16, par ^= 1) {
-        uint32_t d0[16], d1[16], d2[16];
-        tmem_ld16(tcol + (uint32_t)c0, d0);
-        tmem_ld16(tcol + (uint32_t)(COUT + c0), d1);
-        tmem_ld16(tcol + (uint32_t)(2 * COUT + c0), d2);
-        tmem_ld_wait();
-        float4* mine = reinterpret_cast<float4*>(xs + ((par * 4 + q) * 2) * 16);
-        if (edge_r) {
-#pragma unroll
-          for (int k = 0; k < 4; ++k)          // for lane 0 of the next warp
-            mine[k] = make_float4(__uint_as_float(d0[4 * k]), __uint_as_float(d0[4 * k + 1]), __uint_as_float(d0[4 * k + 2]), __uint_as_float(d0[4 * k + 3]));
-        }
-        if (edge_l) {
-#pragma unroll
-          for (int k = 0; k < 4; ++k)          // for lane 31 of the previous warp
-            mine[4 + k] = make_float4(__uint_as_float(d2[4 * k]), __uint_as_float(d2[4 * k + 1]), __uint_as_float(d2[4 * k + 2]), __uint_as_float(d2[4 * k + 3]));
-        }
-        asm volatile("bar.sync %0, 128;" ::"r"(1 + g) : "memory");
-        // the one value a border lane cannot get from a shuffle: its neighbour in the adjacent warp (0 on an image border)
-        float ex[16];
-#pragma unroll
-        for (int k = 0; k < 16; ++k) ex[k] = 0.f;
-        if ((edge_l && has_left) || (edge_r && has_right)) {
-          const float4* src = edge_l ? reinterpret_cast<const float4*>(xs + ((par * 4 + ((q + 3) & 3)) * 2) * 16)
-                                     : reinterpret_cast<const float4*>(xs + ((par * 4 + ((q + 1) & 3)) * 2) * 16 + 16);
-#pragma unroll
-          for (int k = 0; k < 4; ++k) { const float4 a4 = src[k]; ex[4 * k] = a4.x; ex[4 * k + 1] = a4.y; ex[4 * k + 2] = a4.z; ex[4 * k + 3] = a4.w; }
-        }
-        uint32_t o[8];
-#pragma unroll
-        for (int k = 0; k < 16; k += 2) {
-          float v[2];
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-            const float left = __shfl_up_sync(0xffffffffu, __uint_as_float(d0[k + h]), 1);
-            const float right = __shfl_down_sync(0xffffffffu, __uint_as_float(d2[k + h]), 1);
-            v[h] = (__uint_as_float(d1[k + h]) + bv[c0 + k + h]) + (edge_l ? ex[k + h] : left) + (edge_r ? ex[k + h] : right);
-          }
-          __nv_bfloat162 hh = __floats2bfloat162_rn(v[0], v[1]);
-          o[k >> 1] = *reinterpret_cast<uint32_t*>(&hh);
-        }
-        if (row < H) {
-          if (cstore == 8) {                  // 8-channel staging tensor of an RGB layer: channels 8..15 are padding
-            *reinterpret_cast<uint4*>(yrow) = make_uint4(o[0], o[1], o[2], o[3]);
-          } else {
-            uint4* dst = reinterpret_cast<uint4*>(yrow + c0);
-            dst[0] = make_uint4(o[0], o[1], o[2], o[3]);
-            dst[1] = make_uint4(o[4], o[5], o[6], o[7]);
-          }
-        }
-      }
-      tc_fence_before_sync();
-      mbar_arrive(&acc_empty[acc]);
-      if (tid == 0) { TTG_T1(6, j); }
-    }
-  } else if (warp == EPI_WARPS) {
-    // ------------------------------------------------------------ MMA issuer: G groups x 3 vertical taps x K16N slices
-    const uint32_t idesc = umma_idesc_bf16(128, NF, 0, 0);
-    const uint64_t b0 = umma_desc(smem_u32(sW), (uint32_t)NF * 16, 128);
-    for (int it = 0; it < T; ++it) {
-      const int s = it % NBUF, acc = it & (NACC - 1);
-      { TTG_T0(); mbar_wait(&full[s], (uint32_t)(it / NBUF) & 1u); if (lane == 0) { TTG_T1(2, it); } }
-      { TTG_T0(); if (it >= NACC) mbar_wait(&acc_empty[acc], (uint32_t)((it / NACC) - 1) & 1u); if (lane == 0) { TTG_T1(3, it); } }
-      tc_fence_after_sync();
-      if (elect_one()) {
-        TTG_T0();
-        // A: 8-pixel groups 128 B apart (rows are contiguous: no horizontal halo), channel groups HY*W units apart
-        const uint64_t a0 = umma_desc(smem_u32(sA + (size_t)s * A_BYTES), (uint32_t)HY * W * 16, 128);
-        static_for<G>([&](auto gg) {
-          constexpr int g = decltype(gg)::value;
-          const uint32_t dacc = tmem_base + (uint32_t)((acc * G + g) * NF);
-          static_for<3 * K16N>([&](auto ss) {
-            constexpr int sl = decltype(ss)::value, ky = sl / K16N, jj = sl % K16N;
-            constexpr uint32_t aoff = (uint32_t)((2 * jj) * HY * W + (g * R + ky) * W);
-            constexpr uint32_t boff = (uint32_t)((ky * C8N + 2 * jj) * NF);
-            umma_bf16_imm<(sl > 0)>(dacc, a0 + (uint64_t)aoff, b0 + (uint64_t)boff, idesc);
-          });
-        });
-        umma_commit(&empty[s]);
-        umma_commit(&acc_full[acc]);
-        TTG_T1(7, it);
-      }
-      __syncwarp();
-    }
-  } else if (elect_one()) {
-    // ------------------------------------------------------------ TMA producer: rows y0-1 .. y0+4 of the image, all channels
-    for (int j = 0; j < T; ++j) {
-      const int s = j % NBUF;
-      { TTG_T0(); if (j >= NBUF) mbar_wait(&empty[s], (uint32_t)((j / NBUF) - 1) & 1u); TTG_T1(4, j); }
-      const int tile = blockIdx.x + j * gridDim.x;
-      const int n = tile / tiles_img, y0 = (tile - n * tiles_img) * 4;
-      const uint32_t bar = smem_u32(&full[s]);
-      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(A_BYTES) : "memory");
-      asm volatile(
-          "cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5, %6}], [%7];"
-          ::"r"(smem_u32(sA + (size_t)s * A_BYTES)), "l"(&tmap), "r"(0), "r"(0), "r"(y0 - 1), "r"(0), "r"(n), "r"(bar)
-          : "memory");
-    }
-  }
-  tc_fence_before_sync();
-  __syncthreads();
-  if (warp == EPI_WARPS) tmem_dealloc(tmem_base, 512u);
-}
-
-// Off by default: correct (tests/test_gpu_paths.py) but not faster on B200 -- 16->16 @128^2: 90-93 us against 80-90 us for
-// the 9-MMA tap-shift kernel; the MMA count drops 3x but the shift-and-add epilogue (3 TMEM loads, 32 shuffles, a
-// cross-warp exchange per 16 channels) is issue-bound at ~1700-1900 cycles per 512-pixel tile even with one warp set
-// per M group (clock64 trace: epi.run).  Kept as the starting point for a version whose epilogue adds in TMEM.
-static int g_use_fold = 0;
-extern "C" int ttg_set_use_fold(int on) { g_use_fold = on; return TTG_OK; }
-
-template <int CIN, int COUT, int W>
-static int launch_conv_tc_fold(const void* x, const void* wp, const float* bias, void* y, int N, int H, int cin_mem, int cstore,
-                               cudaStream_t st) {
-  ttg_encode_tiled_fn enc = ttg_get_encode_tiled();
-  if (!enc) return ttg_set_error(TTG_ERR_CUDA, "conv2d_tc: cuTensorMapEncodeTiled unavailable");
-  constexpr int C8N = CIN / 8, HY = 6;
-  CUtensorMap tmap;
-  // (8 channels, x, y, channel group, image): the box lands as [channel group][row][x] x 16 B
-  const cuuint64_t gdim[5] = {8, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)(cin_mem / 8), (cuuint64_t)N};
-  const cuuint64_t gstr[4] = {(cuuint64_t)cin_mem * 2, (cuuint64_t)W * cin_mem * 2, 16, (cuuint64_t)H * W * cin_mem * 2};
-  const cuuint32_t box[5] = {8, (cuuint32_t)W, (cuuint32_t)HY, (cuuint32_t)C8N, 1};
-  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  CUresult r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return ttg_set_error(TTG_ERR_CUDA, "conv2d_tc: cuTensorMapEncodeTiled failed (%d)", (int)r);
-  constexpr int W_BYTES = 9 * (CIN / 16) * COUT * 32, A_BYTES = C8N * HY * W * 16;
-  constexpr int G = 4 / (128 / W), THREADS = (4 * G + 2) * 32;
-  constexpr int smem = ((W_BYTES + 127) & ~127) + 3 * A_BYTES + 256 + G * 2 * 4 * 2 * 16 * 4;
-  static bool attr = false;
-  if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(conv_tc_fold_kernel<CIN, COUT, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) return ttg_set_error(TTG_ERR_CUDA, "conv2d_tc: smem attribute: %s", cudaGetErrorString(e));
-    attr = true;
-  }
-  const long long tiles = (long long)N * ((H + 3) / 4);
-  long long grid = ttg_num_sms();
-  if (grid > tiles) grid = tiles;
-  conv_tc_fold_kernel<CIN, COUT, W><<<(unsigned)grid, THREADS, smem, st>>>(tmap, (const bf16*)wp, bias, (bf16*)y, H, (int)tiles, cstore);
-  TTG_CHECK_LAUNCH("conv2d_tc_fold");
-  return TTG_OK;
-}
-
-// ------------------------------------------------------------------ fprop / dgrad, bulk-row loads + transform stage
-// The tensor-map loads above fetch an NHWC halo tile as 16-byte "rows" (8 channels of one pixel), and the TMA engine
-// delivers about ONE such row per clock per SM (measured, round 2: clock64 traces of the wgrad kernel: a tile of 1056
-// rows takes 3170 cycles at three CTAs per SM), i.e. <= 16 B / clk / SM = 4.6 TB/s over the chip before any other
-// cost -- below the HBM roofline of the small-channel layers.  Here the producer warp copies whole pixel ROWS of the
-// halo tile with cp.async.bulk (contiguous (TW+2) * Cin * 2 bytes each, no tensor map) into a raw staging slot, and
-// four transform warps re-lay it out into the [halo row][channel group][halo col] x 16 B UMMA operand image.  The
-// transform stage is where everything that used to be a separate pass over the tensor happens for free:
-//   * the BatchNorm + LeakyReLU that precedes the conv (generator.py:38-47, discriminator.py:60-66):
-//     a = lrelu(x * scale[c] + shift[c]), zero padding applied AFTER the activation like the reference;
-//   * the nearest x2 upsample of the generator blocks (generator.py:58): the raw slot holds the LOW resolution
-//     tile (10 x 6 pixels) and is replicated while it is re-laid out;
-//   * the zero fill of the conv padding and of the missing channel group of 8-channel (RGB staging) tensors.
-// warps 0-3 epilogue, warp 4 MMA issuer, warp 5 row producer, warps 6-9 transform.
-template <int K, int CIN, bool UP, bool PRE, bool STATS>
-__global__ void __launch_bounds__(320) conv_tc_rows_kernel(const bf16* __restrict__ x, const bf16* __restrict__ wp,
-                                                          const float* __restrict__ bias, void* __restrict__ y, int out_f32,
-                                                          int H, int W, int Cout, int total_tiles, int tmem_cols, int cin_mem,
-                                                          int cstore, int nraw, int nbuf, const float* __restrict__ pre_scale,
-                                                          const float* __restrict__ pre_shift, float slope,
-                                                          double* __restrict__ stats) {
-  constexpr int HALO = K / 2, WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO, HP = WH * HH;
-  constexpr int RH = UP ? TC_TH / 2 + 2 * HALO : HH, RW = UP ? TC_TW / 2 + 2 * HALO : WH;   // raw tile (low resolution when UP)
-  constexpr int NACC = 4, C8N = CIN / 8, K16N = CIN / 16;
-  extern __shared__ __align__(128) uint8_t smem[];
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const uint32_t slice_bytes = (uint32_t)Cout * 32;
-  const uint32_t w_bytes = (uint32_t)(K * K * K16N) * slice_bytes;
-  constexpr uint32_t a_bytes = (uint32_t)C8N * HP * 16;
-  const int c8n_mem = cin_mem >> 3;                                          // channel groups present in memory
-  const uint32_t pix_bytes = (uint32_t)cin_mem * 2;
-  const uint32_t raw_bytes = ((uint32_t)(RH * RW) * pix_bytes + 127) & ~127u;
-  uint8_t* sW = smem;
-  uint8_t* sA = smem + ((w_bytes + 127) & ~127u);
-  uint8_t* sR = sA + (size_t)nbuf * a_bytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sR + (size_t)nraw * raw_bytes);
-  uint64_t* raw_full = bars;              // [nraw]  bytes of the tile's rows have landed (tx count)
-  uint64_t* raw_empty = raw_full + 4;     // [nraw]  transform warps are done reading the slot (128 arrivals)
-  uint64_t* ready = raw_empty + 4;        // [nbuf]  operand image written and fenced (128 arrivals)
-  uint64_t* empty = ready + 4;            // [nbuf]  MMAs have consumed the operand image (commit)
-  uint64_t* acc_full = empty + 4;
-  uint64_t* acc_empty = acc_full + NACC;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + NACC);
-  uint8_t* sE = reinterpret_cast<uint8_t*>(bars) + 256;
-  float* s_stats = reinterpret_cast<float*>(sE + tc_epi_strip_bytes_dev(Cout));
-
-  const int tiles_x = (W + TC_TW - 1) / TC_TW, tiles_y = (H + TC_TH - 1) / TC_TH, tiles_img = tiles_x * tiles_y;
-  const int T = (total_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-  auto tile_coords = [&](int j, int& n, int& y0, int& x0) {
-    const int tile = blockIdx.x + j * gridDim.x;
-    n = tile / tiles_img;
-    const int t2 = tile - n * tiles_img;
-    y0 = (t2 / tiles_x) * TC_TH;
-    x0 = (t2 % tiles_x) * TC_TW;
-  };
-
-  if constexpr (STATS)
-    for (int i = tid; i < 2 * Cout; i += blockDim.x) s_stats[i] = 0.f;
-  if (warp == 4) tmem_alloc(tmem_slot, (uint32_t)tmem_cols);
-  if (tid == 0) {
-    for (int i = 0; i < nraw; ++i) { mbar_init(&raw_full[i], 1); mbar_init(&raw_empty[i], 128); }
-    for (int i = 0; i < nbuf; ++i) { mbar_init(&ready[i], 128); mbar_init(&empty[i], 1); }
-    for (int i = 0; i < NACC; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 128); }
-    mbar_fence_init();
-  }
-  if (warp < 4)
-    for (int i = tid; i < (int)(w_bytes / 16); i += 128)
-      reinterpret_cast<uint4*>(sW)[i] = __ldg(reinterpret_cast<const uint4*>(wp) + i);
-  fence_proxy_async_smem();
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp < 4) {
-    // ------------------------------------------------------------ epilogue
-    EpiStats est;
-    if constexpr (STATS) {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) est.s[k] = est.q[k] = 0.f;
-    }
-    const bool reg_stats = STATS && epi_stats_in_regs(Cout) && cstore == Cout;
-    for (int j = 0; j < T; ++j) {
-      const int acc = j & (NACC - 1);
-      int n, y0, x0;
-      tile_coords(j, n, y0, x0);
-      { TTG_T0(); if (warp == 0) mbar_wait(&acc_full[acc], (uint32_t)(j / NACC) & 1u);
-        asm volatile("bar.sync 1, 128;" ::: "memory"); if (tid == 0) { TTG_T1(5, j); } }
-      tc_fence_after_sync();
-      TTG_T0();
-      if (!out_f32)
-        conv_tc_epilogue_coalesced(tmem_base + (uint32_t)(acc * Cout), sE, warp, lane, n, y0, x0, H, W, cstore, bias,
-                                   reinterpret_cast<bf16*>(y), STATS ? s_stats : nullptr, (STATS && reg_stats) ? &est : nullptr);
-      else
-        conv_tc_epilogue<HALO>(tmem_base + (uint32_t)(acc * Cout), warp, tid, n, y0, x0, H, W, Cout, bias, y, out_f32,
-                               cstore == Cout ? 0 : cstore);
-      tc_fence_before_sync();
-      mbar_arrive(&acc_empty[acc]);
-      if (tid == 0) { TTG_T1(6, j); }
-    }
-    if constexpr (STATS) { if (reg_stats) epi_stats_flush(est, lane, Cout, s_stats); }
-  } else if (warp == 4) {
-    // ------------------------------------------------------------ MMA issuer
-    const uint32_t idesc = umma_idesc_bf16(128, Cout, 0, 0);
-    const uint64_t b0 = umma_desc(smem_u32(sW), (uint32_t)Cout * 16, 128);
-    const uint32_t b_step = slice_bytes >> 4;
-    int s = 0;
-    uint32_t sph = 0;
-    for (int it = 0; it < T; ++it) {
-      const int acc = it & (NACC - 1);
-      { TTG_T0(); mbar_wait(&ready[s], sph); if (lane == 0) { TTG_T1(2, it); } }
-      { TTG_T0(); if (it >= NACC) mbar_wait(&acc_empty[acc], (uint32_t)((it / NACC) - 1) & 1u); if (lane == 0) { TTG_T1(3, it); } }
-      tc_fence_after_sync();
-      if (elect_one()) {
-        const uint64_t a0 = umma_desc(smem_u32(sA + (size_t)s * a_bytes), WH * 16, C8N * WH * 16);
-        resident_issue_tile<K, CIN>(tmem_base + (uint32_t)(acc * Cout), a0, b0, b_step, idesc);
-        umma_commit(&empty[s]);
-        umma_commit(&acc_full[acc]);
-      }
-      __syncwarp();
-      if (++s == nbuf) { s = 0; sph ^= 1u; }
-    }
-  } else if (warp == 5) {
-    // ------------------------------------------------------------ row producer: one bulk copy per pixel row of the raw tile
-    const int Hs = H >> (UP ? 1 : 0), Ws = W >> (UP ? 1 : 0);
-    int r = 0;
-    uint32_t rph = 0;
-    for (int j = 0; j < T; ++j) {
-      { TTG_T0(); if (j >= nraw) mbar_wait(&raw_empty[r], rph ^ 1u); if (lane == 0) { TTG_T1(1, j); } }
-      TTG_T0();
-      int n, y0, x0;
-      tile_coords(j, n, y0, x0);
-      const int ylo = (y0 - HALO) >> (UP ? 1 : 0), xlo = (x0 - HALO) >> (UP ? 1 : 0);    // arithmetic shifts: -1 >> 1 == -1
-      const int c0 = max(xlo, 0), c1 = min(xlo + RW, Ws);
-      const int r0 = max(ylo, 0), r1 = min(ylo + RH, Hs);
-      const uint32_t row_bytes = (uint32_t)(c1 - c0) * pix_bytes;
-      const uint32_t bar = smem_u32(&raw_full[r]);
-      // (one elected lane walks the rows: UBLKCP is a uniform-datapath instruction, and 18 lanes with different
-      //  addresses made ptxas serialise them in a ~100-cycle-per-copy waterfall loop: 1900 cycles per tile, measured)
-      if (elect_one()) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t)(r1 - r0) * row_bytes) : "memory");
-        const uint8_t* src = reinterpret_cast<const uint8_t*>(x) + (((long long)n * Hs + r0) * Ws + c0) * (long long)pix_bytes;
-        uint32_t dst = smem_u32(sR + (size_t)r * raw_bytes) + (uint32_t)((r0 - ylo) * RW + (c0 - xlo)) * pix_bytes;
-        const long long src_step = (long long)Ws * pix_bytes;
-        const uint32_t dst_step = (uint32_t)RW * pix_bytes;
-        for (int ry = r0; ry < r1; ++ry, src += src_step, dst += dst_step)
-          asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                       ::"r"(dst), "l"(src), "r"(row_bytes), "r"(bar) : "memory");
-      }
-      __syncwarp();
-      if (lane == 0) { TTG_T1(9, j); }
-      if (++r == nraw) { r = 0; rph ^= 1u; }
-    }
-  } else {
-    // ------------------------------------------------------------ transform: raw rows -> UMMA operand image
-    const int tt = tid - 192;                       // 0..127
-    const int c8 = tt % C8N, p0 = tt / C8N;         // this thread's channel group (fixed) and first halo pixel
-    constexpr int PSTEP = 128 / C8N;
-    float sc[8], sh[8];
-    if constexpr (PRE) {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) {        // (arrays of cin_mem entries; padded channels must carry scale = shift = 0)
-        sc[k] = c8 < c8n_mem ? __ldg(pre_scale + c8 * 8 + k) : 0.f;
-        sh[k] = c8 < c8n_mem ? __ldg(pre_shift + c8 * 8 + k) : 0.f;
-      }
-    }
-    const bool have_c8 = c8 < c8n_mem;
-    int r = 0, s = 0;
-    uint32_t rph = 0, sph = 0;
-    for (int j = 0; j < T; ++j) {
-      int n, y0, x0;
-      tile_coords(j, n, y0, x0);
-      const int ylo = (y0 - HALO) >> (UP ? 1 : 0), xlo = (x0 - HALO) >> (UP ? 1 : 0);
-      { TTG_T0();
-        if (warp == 6) { mbar_wait(&raw_full[r], rph); if (j >= nbuf) mbar_wait(&empty[s], sph ^ 1u); }
-        asm volatile("bar.sync 2, 128;" ::: "memory");
-        if (tt == 0) { TTG_T1(4, j); } }
-      TTG_T0();
-      const uint8_t* raw = sR + (size_t)r * raw_bytes;
-      const uint32_t dst0 = smem_u32(sA + (size_t)s * a_bytes);
-      for (int p = p0; p < HP; p += PSTEP) {
-        const int hy = p / WH, hx = p - hy * WH;
-        const int gy = y0 + hy - HALO, gx = x0 + hx - HALO;
-        uint4 v = make_uint4(0u, 0u, 0u, 0u);
-        if (have_c8 && gy >= 0 && gy < H && gx >= 0 && gx < W) {
-          const int ry = (gy >> (UP ? 1 : 0)) - ylo, rx = (gx >> (UP ? 1 : 0)) - xlo;
-          v = *reinterpret_cast<const uint4*>(raw + (size_t)(ry * RW + rx) * pix_bytes + c8 * 16);
-          if constexpr (PRE) {
-            __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&v);
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              float2 f = __bfloat1622float2(h[q]);
-              f.x = lrelu(f.x * sc[2 * q] + sh[2 * q], slope);
-              f.y = lrelu(f.y * sc[2 * q + 1] + sh[2 * q + 1], slope);
-              h[q] = __floats2bfloat162_rn(f.x, f.y);
-            }
-          }
-        }
-        asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(dst0 + (uint32_t)((hy * C8N + c8) * WH + hx) * 16), "r"(v.x), "r"(v.y),
-                     "r"(v.z), "r"(v.w) : "memory");
-      }
-      fence_proxy_async_smem();
-      mbar_arrive(&ready[s]);
-      mbar_arrive(&raw_empty[r]);
-      if (tt == 0) { TTG_T1(7, j); }
-      if (++r == nraw) { r = 0; rph ^= 1u; }
-      if (++s == nbuf) { s = 0; sph ^= 1u; }
-    }
-  }
-  tc_fence_before_sync();
-  __syncthreads();
-  if (warp == 4) tmem_dealloc(tmem_base, (uint32_t)tmem_cols);
-  if constexpr (STATS)
-    for (int i = tid; i < 2 * Cout; i += blockDim.x) atomicAdd(&stats[i], (double)s_stats[i]);
-}
-
-static int g_use_rows = 0;       // A/B switch: bulk-row + transform kernel for resident-filter layers (0: tensor-map tiles)
-extern "C" int ttg_set_use_rows(int on) { g_use_rows = on ? 1 : 0; return TTG_OK; }
-
-template <int K, int CIN, bool UP, bool PRE>
-static int launch_conv_tc_rows(const void* x, const void* wp, const float* bias, void* y, int out_f32, int N, int H, int W,
-                               int Cout, int cin_mem, int cstore, long long tiles, const float* pre_scale,
-                               const float* pre_shift, float slope, double* stats, cudaStream_t st) {
-  constexpr int HALO = K / 2, WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO, HP = WH * HH;
-  constexpr int RH = UP ? TC_TH / 2 + 2 * HALO : HH, RW = UP ? TC_TW / 2 + 2 * HALO : WH;
-  const int w_bytes = K * K * (CIN / 16) * Cout * 32;
-  const int a_bytes = (CIN / 8) * HP * 16;
-  const int raw_bytes = (RH * RW * cin_mem * 2 + 127) & ~127;
-  const int fixed = ((w_bytes + 127) & ~127) + 256 + tc_epi_bytes(Cout) + 64;
-  // slots: as deep as fits, at most 3 operand + 3 raw slots
-  int nbuf = 3, nraw = 3;
-  while (nbuf > 2 && fixed + nbuf * a_bytes + nraw * raw_bytes > 200 * 1024) --nbuf;
-  while (nraw > 2 && fixed + nbuf * a_bytes + nraw * raw_bytes > 200 * 1024) --nraw;
-  const int smem = fixed + nbuf * a_bytes + nraw * raw_bytes;
-  if (smem > 227 * 1024) return ttg_set_error(TTG_ERR_UNSUPPORTED, "conv2d_tc_rows: layer does not fit shared memory");
-  const int pcols = (int)tmem_cols_for(4 * Cout);
-  auto kern_s = conv_tc_rows_kernel<K, CIN, UP, PRE, true>;
-  auto kern_n = conv_tc_rows_kernel<K, CIN, UP, PRE, false>;
-  static int smem_set = 0;
-  if (smem > smem_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern_n, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(kern_s, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) return ttg_set_error(TTG_ERR_CUDA, "conv2d_tc_rows: smem attribute: %s", cudaGetErrorString(e));
-    smem_set = smem;
-  }
-  int per_sm = (220 * 1024) / smem;
-  if (per_sm > 512 / pcols) per_sm = 512 / pcols;
-  if (per_sm > 2048 / 320) per_sm = 2048 / 320;
-  if (per_sm < 1) per_sm = 1;
-  long long grid = (long long)ttg_num_sms() * per_sm;
-  if (grid > tiles) grid = tiles;
-  if (stats)
-    kern_s<<<(unsigned)grid, 320, smem, st>>>((const bf16*)x, (const bf16*)wp, bias, y, out_f32, H, W, Cout, (int)tiles, pcols, cin_mem,
-                                              cstore, nraw, nbuf, pre_scale, pre_shift, slope, stats);
-  else
-    kern_n<<<(unsigned)grid, 320, smem, st>>>((const bf16*)x, (const bf16*)wp, bias, y, out_f32, H, W, Cout, (int)tiles, pcols, cin_mem,
-                                              cstore, nraw, nbuf, pre_scale, pre_shift, slope, stats);
-  TTG_CHECK_LAUNCH("conv2d_tc_rows");
-  return TTG_OK;
-}
-
-template <int K, int CIN>
-static int dispatch_conv_tc_rows(int up, bool pre, const void* x, const void* wp, const float* bias, void* y, int out_f32, int N,
-                                 int H, int W, int Cout, int cin_mem, int cstore, long long tiles, const float* pre_scale,
-                                 const float* pre_shift, float slope, double* stats, cudaStream_t st) {
-#define TTG_ROWS(UPF, PREF) launch_conv_tc_rows<K, CIN, UPF, PREF>(x, wp, bias, y, out_f32, N, H, W, Cout, cin_mem, cstore, tiles, \
-                                                                  pre_scale, pre_shift, slope, stats, st)
-  if (up) return pre ? TTG_ROWS(true, true) : TTG_ROWS(true, false);
-  return pre ? TTG_ROWS(false, true) : TTG_ROWS(false, false);
-#undef TTG_ROWS
 }
 
 // Cin / Cout are the (padded, multiple-of-16) GEMM channel counts; cin_real / cout_real the channel counts of the
@@ -1975,69 +1154,49 @@ static int dispatch_conv_tc_rows(int up, bool pre, const void* x, const void* wp
 // stats (optional): double[2 * Cout], zeroed by the caller; receives sum / sum of squares per output channel of the
 // tensor written (BatchNorm statistics of the next layer, see ttg_conv2d_tc_stats).
 static int conv2d_tc_core(const void* x, const void* wp, const float* bias, void* y, int N, int H, int W, int Cin,
-                          int Cout, int cin_real, int cout_real, int ksize, int up, int dtype_out,
-                          const float* pre_scale, const float* pre_shift, float slope, double* stats, void* stream) {
+                          int Cout, int cin_real, int cout_real, int ksize, int dtype_out, double* stats, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
-  // (taken for the cases the tensor-map kernel has no variant for: fused upsample, prologue on an 8-channel tensor;
-  //  for plain layers the pixel-major swizzled TMA kernel below is faster: 83 vs 116 us on 16->16 @128^2)
-  if ((g_use_rows || up == 1 || (pre_scale != nullptr && cin_real != Cin)) && (ksize == 1 || ksize == 3) &&
-      (Cin == 16 || Cin == 32 || Cin == 64) && Cout % 16 == 0 && Cout >= 16 &&
-      Cout <= 256 && ksize * ksize * (Cin / 16) * Cout * 32 <= TC_RESIDENT_W_BYTES && (up == 0 || (H % 2 == 0 && W % 2 == 0)) &&
-      (dtype_out == TTG_BF16 || dtype_out == TTG_F32)) {
-    // bulk-row loads + transform stage (fused BatchNorm/LeakyReLU prologue, fused nearest upsample, 8-channel inputs)
-    const bool in8r = cin_real == 8 && Cin == 16, out8r = cout_real == 8 && Cout == 16 && dtype_out == TTG_BF16;
-    const bool okc = (cin_real == Cin || in8r) && (cout_real == Cout || out8r);
-    const bool ok_stats = stats == nullptr || (dtype_out == TTG_BF16 && cout_real == Cout);
-    const long long tiles_r = (long long)N * ((H + TC_TH - 1) / TC_TH) * ((W + TC_TW - 1) / TC_TW);
-    if (okc && ok_stats && tiles_r > 0 && tiles_r < (1ll << 31) && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
-        (reinterpret_cast<uintptr_t>(y) & 15) == 0 && (reinterpret_cast<uintptr_t>(wp) & 15) == 0) {
-      const int of32 = dtype_out == TTG_F32;
-#define TTG_ROWS_K(KK, CI) dispatch_conv_tc_rows<KK, CI>(up, pre_scale != nullptr, x, wp, bias, y, of32, N, H, W, Cout, cin_real, cout_real, \
-                                                      tiles_r, pre_scale, pre_shift, slope, stats, st)
-      if (ksize == 3) return Cin == 16 ? TTG_ROWS_K(3, 16) : Cin == 32 ? TTG_ROWS_K(3, 32) : TTG_ROWS_K(3, 64);
-      return Cin == 16 ? TTG_ROWS_K(1, 16) : Cin == 32 ? TTG_ROWS_K(1, 32) : TTG_ROWS_K(1, 64);
-#undef TTG_ROWS_K
-    }
-  }
   // 8-channel staging tensors (ttg_pad_channels8) ride the TMA path: not "padded" in the scalar-access sense
-  // (genuine 8-channel layers of the '512thin' config look the same; with an upsample, a prologue or an fp32 output
-  // they take the scalar-access padded path below instead)
-  const bool tma8 = !pre_scale && up == 0 && g_use_tma && dtype_out == TTG_BF16 && ttg_get_encode_tiled() != nullptr;
+  // (genuine 8-channel layers of the '512thin' config look the same; with an fp32 output they take the scalar-access
+  // padded path below instead)
+  const bool tma8 = dtype_out == TTG_BF16;
   const bool in8 = tma8 && cin_real == 8 && Cin == 16, out8 = tma8 && cout_real == 8 && Cout == 16;
   const bool padded = (cin_real != Cin && !in8) || (cout_real != Cout && !out8);
   TTG_REQUIRE(cin_real >= 1 && cin_real <= Cin && cout_real >= 1 && cout_real <= Cout, "conv2d_tc: bad real channel counts");
-  TTG_REQUIRE(!padded || ((cin_real == Cin || cin_real <= 8) && (cout_real == Cout || (cout_real <= 16 && Cout == 16)) && !pre_scale),
-              "conv2d_tc: channel padding supports <= 8 real input channels / Cout padded to 16, without prologue");
+  TTG_REQUIRE(!padded || ((cin_real == Cin || cin_real <= 8) && (cout_real == Cout || (cout_real <= 16 && Cout == 16))),
+              "conv2d_tc: channel padding supports <= 8 real input channels / Cout padded to 16");
   TTG_REQUIRE(ksize == 1 || ksize == 3, "conv2d_tc: ksize %d unsupported", ksize);
   TTG_REQUIRE(Cin % 16 == 0 && Cout % 16 == 0 && Cin >= 16 && Cout >= 16 && Cin <= 256 && Cout <= 256,
               "conv2d_tc: channels must be multiples of 16 in [16,256] (got %d -> %d)", Cin, Cout);
-  TTG_REQUIRE(up == 0 || (H % 2 == 0 && W % 2 == 0), "conv2d_tc: upsample needs even output size");
   TTG_REQUIRE(dtype_out == TTG_BF16 || dtype_out == TTG_F32, "conv2d_tc: bad output dtype");
   TTG_REQUIRE(padded || ((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(y) & 15) == 0),
               "conv2d_tc: activation pointers must be 16-byte aligned");
   TTG_REQUIRE((reinterpret_cast<uintptr_t>(wp) & 15) == 0, "conv2d_tc: weight pointer must be 16-byte aligned");
   const int halo = ksize / 2;
   const int HP = (TC_TW + 2 * halo) * (TC_TH + 2 * halo);
-  const int total_slices = ksize * ksize * (Cin / 16);
-  const int slice_bytes = Cout * 32;
-  int stage_slices = TC_STAGE_BYTES / slice_bytes;
-  if (stage_slices < 1) stage_slices = 1;
-  if (stage_slices > total_slices) stage_slices = total_slices;
-  const int nstages = total_slices > stage_slices ? 2 : 1;
-  const int smem = (Cin / 8) * HP * 16 + nstages * stage_slices * slice_bytes + 64;
+  const int a_bytes = (Cin / 8) * HP * 16;
   const long long tiles = (long long)N * ((H + TC_TH - 1) / TC_TH) * ((W + TC_TW - 1) / TC_TW);
   TTG_REQUIRE(tiles > 0 && tiles < (1ll << 31), "conv2d_tc: bad problem size");
-  const int w_bytes = total_slices * slice_bytes;
+  const int w_bytes = ksize * ksize * (Cin / 16) * Cout * 32;
   TTG_REQUIRE(!padded || w_bytes <= TC_RESIDENT_W_BYTES, "conv2d_tc: padded layers must fit the resident-filter kernel");
-  if (g_use_fold && g_use_tma && ksize == 3 && up == 0 && !padded && !pre_scale && stats == nullptr && dtype_out == TTG_BF16) {
-    // small-channel 3x3 layers on full-row tiles: horizontal taps folded into N (see conv_tc_fold_kernel)
-#define TTG_FOLD(CI, CO, WW) if (Cin == CI && Cout == CO && W == WW) return launch_conv_tc_fold<CI, CO, WW>(x, wp, bias, y, N, H, cin_real, cout_real, st)
-    TTG_FOLD(16, 16, 128);
-    TTG_FOLD(32, 32, 64);
-#undef TTG_FOLD
+  const int of32 = dtype_out == TTG_F32;
+  if (w_bytes <= TC_RESIDENT_W_BYTES && !padded) {
+    const int tcols = (int)tmem_cols_for(4 * Cout);
+    const bool deep = a_bytes <= 12 * 1024;       // small tiles: 4 slots, else 3
+#define TTG_TMA(KK, NB, CI) launch_conv_tc_tma<KK, NB, CI>(x, wp, bias, y, of32, N, H, W, Cin, Cout, cin_real, cout_real, tiles, w_bytes, a_bytes, tcols, stats, st)
+    // activation slots that fit next to the resident filter (256 -> 128 1x1: 64 KB filter + 64 KB tiles -> 2 slots)
+    const bool three = ((w_bytes + 127) & ~127) + 3 * a_bytes + 256 + tc_epi_bytes(Cout) <= 227 * 1024;
+    // ring depth: the pipeline of one CTA is latency bound (one CTA per SM reaches half the throughput of three), so the
+    // small tiles get 8 / 6 slots: 16->16 @128^2 80 -> 66 us, 32->32 @64^2 39 -> 37 us (round 2 sweep)
+    const bool four64 = ((w_bytes + 127) & ~127) + 4 * a_bytes + 256 + tc_epi_bytes(Cout) <= 200 * 1024;
+    if (ksize == 3) return Cin == 16 ? TTG_TMA(3, 8, 16) : Cin == 32 ? TTG_TMA(3, 6, 32) : Cin == 64 ? (four64 ? TTG_TMA(3, 4, 64) : TTG_TMA(3, 3, 64))
+                                   : (deep ? TTG_TMA(3, 4, 0) : three ? TTG_TMA(3, 3, 0) : TTG_TMA(3, 2, 0));
+    return Cin == 16 ? TTG_TMA(1, 8, 16) : Cin == 32 ? TTG_TMA(1, 8, 32) : Cin == 64 ? (four64 ? TTG_TMA(1, 4, 64) : TTG_TMA(1, 3, 64))
+                     : (deep ? TTG_TMA(1, 4, 0) : three ? TTG_TMA(1, 3, 0) : TTG_TMA(1, 2, 0));
+#undef TTG_TMA
   }
-  if (w_bytes <= TC_RESIDENT_W_BYTES) {
-    const int a_bytes = (Cin / 8) * HP * 16;
+  if (padded) {
+    TTG_REQUIRE(stats == nullptr, "conv2d_tc: output statistics need the TMA kernels (bf16 output, no padding)");
     const int nbuf = a_bytes <= 12 * 1024 ? 4 : (a_bytes <= 24 * 1024 ? 3 : 2);
     const int psmem = w_bytes + nbuf * a_bytes + 256 + tc_epi_bytes(Cout);
     const int pcols = (int)tmem_cols_for(4 * Cout);
@@ -2045,107 +1204,53 @@ static int conv2d_tc_core(const void* x, const void* wp, const float* bias, void
     if (per_sm > 512 / pcols) per_sm = 512 / pcols;
     if (per_sm > 8) per_sm = 8;
     if (per_sm < 1) per_sm = 1;
-    const int of32 = dtype_out == TTG_F32;
-    if (!padded && up == 0 && g_use_tma && (!pre_scale || (g_use_swz && cin_real == Cin && (Cin == 16 || Cin == 32 || Cin == 64)))) {
-      bool used = false;
-      const int tcols = (int)tmem_cols_for(4 * Cout);
-      const bool deep = a_bytes <= 12 * 1024;       // small tiles: 4 slots, else 3
-#define TTG_TMA(KK, NB, CI) launch_conv_tc_tma<KK, NB, CI>(x, wp, bias, y, dtype_out == TTG_F32, N, H, W, Cin, Cout, cin_real, cout_real, tiles, w_bytes, a_bytes, tcols, stats, st, &used, pre_scale, pre_shift, slope)
-      int rc;
-      // activation slots that fit next to the resident filter (256 -> 128 1x1: 64 KB filter + 64 KB tiles -> 2 slots)
-      const bool three = ((w_bytes + 127) & ~127) + 3 * a_bytes + 256 + tc_epi_bytes(Cout) <= 227 * 1024;
-      // ring depth: the pipeline of one CTA is latency bound (one CTA per SM reaches half the throughput of three), so the
-      // small tiles get 8 / 6 slots: 16->16 @128^2 80 -> 66 us, 32->32 @64^2 39 -> 37 us (round 2 sweep, tools/kb2.sh)
-      const bool four64 = ((w_bytes + 127) & ~127) + 4 * a_bytes + 256 + tc_epi_bytes(Cout) <= 200 * 1024;
-      if (ksize == 3) rc = Cin == 16 ? TTG_TMA(3, 8, 16) : Cin == 32 ? TTG_TMA(3, 6, 32) : Cin == 64 ? (four64 ? TTG_TMA(3, 4, 64) : TTG_TMA(3, 3, 64))
-                                     : (deep ? TTG_TMA(3, 4, 0) : three ? TTG_TMA(3, 3, 0) : TTG_TMA(3, 2, 0));
-      else rc = Cin == 16 ? TTG_TMA(1, 8, 16) : Cin == 32 ? TTG_TMA(1, 8, 32) : Cin == 64 ? (four64 ? TTG_TMA(1, 4, 64) : TTG_TMA(1, 3, 64))
-                          : (deep ? TTG_TMA(1, 4, 0) : three ? TTG_TMA(1, 3, 0) : TTG_TMA(1, 2, 0));
-#undef TTG_TMA
-      if (rc != TTG_OK || used) return rc;
-    }
-    TTG_REQUIRE(stats == nullptr, "conv2d_tc: output statistics need the TMA kernels (bf16 output, no upsample / prologue / padding)");
-    const bool lean = !padded && !pre_scale && (TC_TW + 2 * halo) * (Cin / 8) <= 128;
-#define TTG_PERSIST(KK, NB) (lean ? launch_conv_tc_persist<KK, NB, true>(x, wp, bias, y, of32, H, W, Cin, Cout, up, pre_scale, \
-                                        pre_shift, slope, tiles, psmem, pcols, per_sm, cin_real, cout_real, st)              \
-                                  : launch_conv_tc_persist<KK, NB, false>(x, wp, bias, y, of32, H, W, Cin, Cout, up, pre_scale, \
-                                        pre_shift, slope, tiles, psmem, pcols, per_sm, cin_real, cout_real, st))
+#define TTG_PERSIST(KK, NB) launch_conv_tc_persist<KK, NB>(x, wp, bias, y, of32, H, W, Cin, Cout, tiles, psmem, pcols, per_sm, \
+                                                           cin_real, cout_real, st)
     if (ksize == 3) return nbuf == 4 ? TTG_PERSIST(3, 4) : nbuf == 3 ? TTG_PERSIST(3, 3) : TTG_PERSIST(3, 2);
     return nbuf == 4 ? TTG_PERSIST(1, 4) : nbuf == 3 ? TTG_PERSIST(1, 3) : TTG_PERSIST(1, 2);
 #undef TTG_PERSIST
   }
-  if (!pre_scale && Cout * 32 <= TC_WSTAGE_BYTES) {
-    const int a_bytes = (Cin / 8) * HP * 16;
-    const bool two = 2 * a_bytes + 4 * TC_WSTAGE_BYTES + 256 + tc_epi_bytes(Cout) <= 200 * 1024;
-    const int of32 = dtype_out == TTG_F32;
-#define TTG_STREAM(KK, NAA, CI, CO) launch_conv_tc_stream_ws<KK, NAA, CI, CO>(x, wp, bias, y, of32, N, H, W, Cin, Cout, up, tiles, stats, st)
-    const bool two32 = 2 * a_bytes + 6 * TC_WSTAGE_BYTES + 256 + tc_epi_bytes(Cout) <= 224 * 1024;
-    const bool one32 = a_bytes + 6 * TC_WSTAGE_BYTES + 256 + tc_epi_bytes(Cout) <= 224 * 1024;
-    if (ksize == 3 && two32) {
-      if (Cin == 128 && Cout == 128) return TTG_STREAM(3, 2, 128, 128);
-      if (Cin == 128 && Cout == 64) return TTG_STREAM(3, 2, 128, 64);
-      if (Cin == 64 && Cout == 128) return TTG_STREAM(3, 2, 64, 128);
-      if (Cin == 128 && Cout == 256) return TTG_STREAM(3, 2, 128, 256);
-    }
-    if (ksize == 3 && !two32 && one32) {
-      if (Cin == 256 && Cout == 256) return TTG_STREAM(3, 1, 256, 256);
-      if (Cin == 256 && Cout == 128) return TTG_STREAM(3, 1, 256, 128);
-    }
-    if (ksize == 3) return two ? TTG_STREAM(3, 2, 0, 0) : TTG_STREAM(3, 1, 0, 0);
-    return two ? TTG_STREAM(1, 2, 0, 0) : TTG_STREAM(1, 1, 0, 0);
+  // filter streamed through shared memory: one K slice of it (Cout * 32 bytes) always fits a weight stage
+  static_assert(256 * 32 <= TC_WSTAGE_BYTES, "weight stage smaller than one K slice");
+  const bool two = 2 * a_bytes + 4 * TC_WSTAGE_BYTES + 256 + tc_epi_bytes(Cout) <= 200 * 1024;
+#define TTG_STREAM(KK, NAA, CI, CO) launch_conv_tc_stream_ws<KK, NAA, CI, CO>(x, wp, bias, y, of32, N, H, W, Cin, Cout, tiles, stats, st)
+  const bool two32 = 2 * a_bytes + 6 * TC_WSTAGE_BYTES + 256 + tc_epi_bytes(Cout) <= 224 * 1024;
+  const bool one32 = a_bytes + 6 * TC_WSTAGE_BYTES + 256 + tc_epi_bytes(Cout) <= 224 * 1024;
+  if (ksize == 3 && two32) {
+    if (Cin == 128 && Cout == 128) return TTG_STREAM(3, 2, 128, 128);
+    if (Cin == 128 && Cout == 64) return TTG_STREAM(3, 2, 128, 64);
+    if (Cin == 64 && Cout == 128) return TTG_STREAM(3, 2, 64, 128);
+    if (Cin == 128 && Cout == 256) return TTG_STREAM(3, 2, 128, 256);
+  }
+  if (ksize == 3 && !two32 && one32) {
+    if (Cin == 256 && Cout == 256) return TTG_STREAM(3, 1, 256, 256);
+    if (Cin == 256 && Cout == 128) return TTG_STREAM(3, 1, 256, 128);
+  }
+  if (ksize == 3) return two ? TTG_STREAM(3, 2, 0, 0) : TTG_STREAM(3, 1, 0, 0);
+  return two ? TTG_STREAM(1, 2, 0, 0) : TTG_STREAM(1, 1, 0, 0);
 #undef TTG_STREAM
-  }
-  TTG_REQUIRE(stats == nullptr, "conv2d_tc: output statistics are not available on the generic streaming kernel");
-  const int ki = ksize == 3 ? 1 : 0;
-  if (smem > g_conv_tc_smem[ki]) {
-    cudaError_t e = ksize == 3
-        ? cudaFuncSetAttribute(conv_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)
-        : cudaFuncSetAttribute(conv_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) return ttg_set_error(TTG_ERR_CUDA, "conv2d_tc: smem attribute: %s", cudaGetErrorString(e));
-    g_conv_tc_smem[ki] = smem;
-  }
-  const int cols = (int)tmem_cols_for(Cout);
-  if (ksize == 3)
-    conv_tc_kernel<3><<<(unsigned)tiles, 128, smem, st>>>((const bf16*)x, (const bf16*)wp, bias, y, dtype_out == TTG_F32, H, W,
-                                                         Cin, Cout, up, pre_scale, pre_shift, slope, stage_slices, nstages, cols);
-  else
-    conv_tc_kernel<1><<<(unsigned)tiles, 128, smem, st>>>((const bf16*)x, (const bf16*)wp, bias, y, dtype_out == TTG_F32, H, W,
-                                                         Cin, Cout, up, pre_scale, pre_shift, slope, stage_slices, nstages, cols);
-  TTG_CHECK_LAUNCH("conv2d_tc");
-  return TTG_OK;
 }
 
 extern "C" int ttg_conv2d_tc_ex(const void* x, const void* wp, const float* bias, void* y, int N, int H, int W, int Cin,
-                                int Cout, int cin_real, int cout_real, int ksize, int up, int dtype_out,
-                                const float* pre_scale, const float* pre_shift, float slope, void* stream) {
-  return conv2d_tc_core(x, wp, bias, y, N, H, W, Cin, Cout, cin_real, cout_real, ksize, up, dtype_out, pre_scale, pre_shift, slope,
-                        nullptr, stream);
+                                int Cout, int cin_real, int cout_real, int ksize, int dtype_out, void* stream) {
+  return conv2d_tc_core(x, wp, bias, y, N, H, W, Cin, Cout, cin_real, cout_real, ksize, dtype_out, nullptr, stream);
 }
 // conv + BatchNorm statistics of its output in one pass: sums[0..Cout) = sum_pixels y, sums[Cout..2Cout) = sum y^2
 // (fp64, of the bf16 values written).  The epilogue reduces the tile it holds in registers, so the statistics pass of
 // the following nn.BatchNorm2d (native_batch_norm's first read of the tensor) disappears.
 extern "C" int ttg_conv2d_tc_stats_supported(int Cin, int Cout, int ksize) {
-  if (!g_use_tma || ttg_get_encode_tiled() == nullptr) return 0;
-  if (Cin % 16 || Cout % 16 || Cin < 16 || Cout < 16 || Cin > 256 || Cout > 256 || (ksize != 1 && ksize != 3)) return 0;
-  const int w_bytes = ksize * ksize * (Cin / 16) * Cout * 32;
-  return w_bytes <= TC_RESIDENT_W_BYTES || Cout * 32 <= TC_WSTAGE_BYTES;
+  return Cin % 16 == 0 && Cout % 16 == 0 && Cin >= 16 && Cout >= 16 && Cin <= 256 && Cout <= 256 && (ksize == 1 || ksize == 3);
 }
 extern "C" int ttg_conv2d_tc_stats(const void* x, const void* wp, const float* bias, void* y, int N, int H, int W, int Cin,
                                    int Cout, int ksize, double* sums, void* stream) {
   TTG_REQUIRE(sums != nullptr, "conv2d_tc_stats: sums is required");
   TTG_REQUIRE(ttg_conv2d_tc_stats_supported(Cin, Cout, ksize), "conv2d_tc_stats: unsupported layer %d -> %d k%d", Cin, Cout, ksize);
   cudaMemsetAsync(sums, 0, sizeof(double) * 2 * (size_t)Cout, (cudaStream_t)stream);
-  return conv2d_tc_core(x, wp, bias, y, N, H, W, Cin, Cout, Cin, Cout, ksize, 0, TTG_BF16, nullptr, nullptr, 1.f, sums, stream);
-}
-
-extern "C" int ttg_conv2d_tc_pre(const void* x, const void* wp, const float* bias, void* y, int N, int H, int W, int Cin,
-                                 int Cout, int ksize, int up, int dtype_out, const float* pre_scale,
-                                 const float* pre_shift, float slope, void* stream) {
-  return ttg_conv2d_tc_ex(x, wp, bias, y, N, H, W, Cin, Cout, Cin, Cout, ksize, up, dtype_out, pre_scale, pre_shift, slope, stream);
+  return conv2d_tc_core(x, wp, bias, y, N, H, W, Cin, Cout, Cin, Cout, ksize, TTG_BF16, sums, stream);
 }
 extern "C" int ttg_conv2d_tc(const void* x, const void* wp, const float* bias, void* y, int N, int H, int W, int Cin,
-                             int Cout, int ksize, int up, int dtype_out, void* stream) {
-  return ttg_conv2d_tc_ex(x, wp, bias, y, N, H, W, Cin, Cout, Cin, Cout, ksize, up, dtype_out, nullptr, nullptr, 1.f, stream);
+                             int Cout, int ksize, int dtype_out, void* stream) {
+  return ttg_conv2d_tc_ex(x, wp, bias, y, N, H, W, Cin, Cout, Cin, Cout, ksize, dtype_out, stream);
 }
 
 // ------------------------------------------------------------------ wgrad
@@ -2155,7 +1260,7 @@ extern "C" int ttg_conv2d_tc(const void* x, const void* wp, const float* bias, v
 template <int K>
 __global__ void __launch_bounds__(128) conv_wgrad_tc_kernel(const bf16* __restrict__ x, const bf16* __restrict__ gy,
                                                             float* __restrict__ gw, int N, int H, int W, int Cin, int Cout,
-                                                            int up, int taps_per_group, int tmem_cols) {
+                                                            int taps_per_group, int tmem_cols) {
   constexpr int HALO = K / 2, WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO, HP = WH * HH, NPIX = TC_TH * TC_TW;
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, warp = tid >> 5;
@@ -2190,7 +1295,7 @@ __global__ void __launch_bounds__(128) conv_wgrad_tc_kernel(const bf16* __restri
     const int n = (int)(tile / (tiles_x * tiles_y)), t2 = (int)(tile - (long long)n * tiles_x * tiles_y);
     const int y0 = (t2 / tiles_x) * TC_TH, x0 = (t2 % tiles_x) * TC_TW;
     if (!first) { mbar_wait(&bars[0], phase); phase ^= 1u; }       // previous tile's MMAs have consumed the smem
-    stage_tile<HALO>(sX, x, n, y0, x0, H, W, Cin, up, nullptr, nullptr, 1.f, 128);
+    stage_tile<HALO>(sX, x, n, y0, x0, H, W, Cin, 128);
     for (int u = tid; u < NPIX * g8n; u += blockDim.x) {
       const int g8 = u % g8n, pix = u / g8n;
       const int py = y0 + (pix >> 3), px = x0 + (pix & 7);
@@ -2241,26 +1346,24 @@ __global__ void __launch_bounds__(128) conv_wgrad_tc_kernel(const bf16* __restri
 }
 
 // ------------------------------------------------------------------ wgrad, persistent + warp-specialised
-// warps 0-3 stage (x halo tile, gy tile) pairs with cp.async into an NBUF ring; warps 4-6 each issue the
+// warp 7 loads (x halo tile, gy tile) pairs with tensor-map loads into an NBUF ring; warps 4-6 each issue the
 // MMAs of a share of the accumulator "units" (disjoint TMEM columns, so the issuing threads never touch
-// the same accumulator); accumulators stay in TMEM over all tiles of the CTA; one atomic epilogue.
+// the same accumulator); accumulators stay in TMEM over all tiles of the CTA; warps 0-3 run one atomic epilogue.
 // For Cin <= 80 a unit is a filter column kx with N = 3*Cin: the [row][c8][col] tile layout makes the
 // three vertical taps one uniform-stride B operand, so gy^T (the A operand, mostly padding rows for
 // small Cout) is read 3 instead of 9 times per K step; with Cout <= 64 the MMA uses M = 64.
-template <int K, int NBUF, bool TMA>
-__global__ void __launch_bounds__(256) conv_wgrad_tc_ws_kernel(const bf16* __restrict__ x, const bf16* __restrict__ gy,
-                                                               float* __restrict__ gw, int N, int H, int W, int Cin,
-                                                               int Cout, int up, int units_per_group, int fuse,
-                                                               int tmem_cols, int g_bytes, int cin_real, int cout_real,
+template <int K, int NBUF>
+__global__ void __launch_bounds__(256) conv_wgrad_tc_ws_kernel(float* __restrict__ gw, int N, int H, int W, int Cin,
+                                                               int Cout, int units_per_group, int fuse,
+                                                               int tmem_cols, int g_bytes, int cout_real,
                                                                const __grid_constant__ CUtensorMap tmap_x,
                                                                const __grid_constant__ CUtensorMap tmap_g,
                                                                float* __restrict__ gbias) {
-  constexpr int HALO = K / 2, WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO, HP = WH * HH, NPIX = TC_TH * TC_TW;
-  constexpr int DIST = NBUF > 2 ? NBUF - 2 : 1;
+  constexpr int HALO = K / 2, WH = TC_TW + 2 * HALO, HH = TC_TH + 2 * HALO, NPIX = TC_TH * TC_TW;
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int c8n = Cin >> 3;
-  // fuse == 3 ("mfold", TMA only): the filter column kx is folded into M and the filter row ky into N, so a tile
+  // fuse == 3 ("mfold"): the filter column kx is folded into M and the filter row ky into N, so a tile
   // costs 8 MMAs instead of 24:  D[(j, co), (ky, ci)] = sum_q gy[q + j - 1][co] * x[q + (ky-1) rows][ci],  kx = 2 - j.
   // Both tiles are PIXEL-MAJOR (NHWC as in memory: one TMA request per pixel, SWIZZLE_32B/64B/128B by channel count),
   // which is the MN-major canonical layout with one swizzle row per pixel:
@@ -2303,15 +1406,15 @@ __global__ void __launch_bounds__(256) conv_wgrad_tc_ws_kernel(const bf16* __res
     x0 = (t2 % tiles_x) * TC_TW;
   };
 
-  // Bias gradient (sum over pixels of gy) for free: with TMA-fed tiles warps 0-3 are idle during the main loop, so
-  // they add up the gy tile that sits in shared memory anyway (CTAs of the first tap group only).  Replaces the
-  // separate ttg_channel_sum pass over gy.
-  const bool do_bias = TMA && gbias != nullptr && blockIdx.y == 0;
+  // Bias gradient (sum over pixels of gy) for free: warps 0-3 are idle during the main loop, so they add up the gy
+  // tile that sits in shared memory anyway (CTAs of the first tap group only).  Replaces the separate ttg_channel_sum
+  // pass over gy.
+  const bool do_bias = gbias != nullptr && blockIdx.y == 0;
   float* s_bias = reinterpret_cast<float*>(tmem_slot + 4);        // [128] floats after the barriers
   if (do_bias && tid < 128) s_bias[tid] = 0.f;
   if (warp == 4) tmem_alloc(tmem_slot, (uint32_t)tmem_cols);
   if (tid == 0) {
-    for (int i = 0; i < NBUF; ++i) { mbar_init(&full[i], TMA ? 1 : 128); mbar_init(&empty[i], (uint32_t)n_issuers + (do_bias ? 4u : 0u)); }
+    for (int i = 0; i < NBUF; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], (uint32_t)n_issuers + (do_bias ? 4u : 0u)); }
     mbar_init(done, (uint32_t)n_issuers);
     mbar_fence_init();
   }
@@ -2321,53 +1424,6 @@ __global__ void __launch_bounds__(256) conv_wgrad_tc_ws_kernel(const bf16* __res
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp < 4) {
-    const bool fast_stage = WH * c8n <= 128;
-    const RowStager rs = make_row_stager<HALO>(fast_stage ? Cin : 16, tid);
-    auto stage = [&](int j) {
-      if (j < T) {
-        const int s = j % NBUF;
-        if (j >= NBUF) mbar_wait(&empty[s], (uint32_t)((j / NBUF) - 1) & 1u);
-        int n, y0, x0;
-        tile_coords(j, n, y0, x0);
-        uint8_t* dx = sX + (size_t)s * x_bytes;
-        if (cin_real != Cin) stage_tile_pad<HALO>(dx, x, n, y0, x0, H, W, Cin, cin_real, up, 128);
-        else if (fast_stage) stage_rows<HALO, true>(rs, dx, x, n, y0, x0, H, W, Cin, up, nullptr, nullptr, 1.f);
-        else stage_tile_async<HALO>(dx, x, n, y0, x0, H, W, Cin, up, 128);
-        const uint32_t dg = smem_u32(sG + (size_t)s * g_bytes);
-        if (cout_real != Cout) {                      // padded gy (<= 8 real channels): scalar loads
-          for (int pix = tid; pix < NPIX; pix += 128) {
-            const int py = y0 + (pix >> 3), px = x0 + (pix & 7);
-            uint32_t w4[4] = {0u, 0u, 0u, 0u};
-            if (py < H && px < W) {
-              const unsigned short* src = reinterpret_cast<const unsigned short*>(gy) + (((long long)n * H + py) * W + px) * cout_real;
-              for (int c = 0; c < cout_real; ++c) w4[c >> 1] |= (uint32_t)src[c] << (16 * (c & 1));
-            }
-            uint8_t* d = sG + (size_t)s * g_bytes + (size_t)pix * 16;
-            *reinterpret_cast<uint4*>(d) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
-            for (int g8 = 1; g8 < g8n; ++g8) *reinterpret_cast<uint4*>(d + (size_t)g8 * NPIX * 16) = make_uint4(0u, 0u, 0u, 0u);
-          }
-        } else
-        for (int u = tid; u < NPIX * g8n; u += 128) {
-          const int g8 = u % g8n, pix = u / g8n;
-          const int py = y0 + (pix >> 3), px = x0 + (pix & 7);
-          const bool ok = py < H && px < W;
-          const bf16* src = ok ? gy + (((long long)n * H + py) * W + px) * Cout + co_base + g8 * 8 : gy;
-          cp_async16(dg + (uint32_t)(g8 * NPIX + pix) * 16, src, ok ? 16u : 0u);
-        }
-      }
-      cp_async_commit();
-    };
-    if constexpr (!TMA) {
-#pragma unroll
-      for (int d = 0; d < DIST; ++d) stage(d);
-      for (int it = 0; it < T; ++it) {
-        stage(it + DIST);
-        cp_async_wait_group<DIST>();
-        fence_proxy_async_smem();
-        mbar_arrive(&full[it % NBUF]);
-      }
-      cp_async_wait_all();
-    }
     if (do_bias) {
       // thread -> one 8-channel group and every ppg-th pixel of the tile: consecutive lanes read consecutive pixels
       const int ppg = 128 / g8n, g8 = tid / ppg, p0 = tid - g8 * ppg;
@@ -2507,7 +1563,7 @@ __global__ void __launch_bounds__(256) conv_wgrad_tc_ws_kernel(const bf16* __res
       }
       __syncwarp();
     }
-  } else if (TMA && warp == 7 && elect_one()) {
+  } else if (warp == 7 && elect_one()) {
     // ---- TMA producer: one tensor-map load for the x halo tile, one for the gy tile, per slot
     for (int j = 0; j < T; ++j) {
       const int s = j % NBUF;
@@ -2545,18 +1601,14 @@ __global__ void __launch_bounds__(256) conv_wgrad_tc_ws_kernel(const bf16* __res
 }
 
 template <int K, int NBUF>
-static int launch_wgrad_ws(const void* x, const void* gy, float* gw, int N, int H, int W, int Cin, int Cout, int up,
-                           int upg, int fuse, int cols, int g_bytes, int smem, dim3 grid, int cin_real, int cout_real,
-                           float* gbias, bool* bias_done, cudaStream_t st) {
+static int launch_wgrad_ws(const void* x, const void* gy, float* gw, int N, int H, int W, int Cin, int Cout, int upg, int fuse,
+                           int cols, int g_bytes, int smem, dim3 grid, int cin_real, int cout_real, float* gbias, cudaStream_t st) {
+  const ttg_encode_tiled_fn enc = ttg_get_encode_tiled();
+  if (!enc) return ttg_no_encode_tiled("conv2d_wgrad_tc");
   constexpr int HALO = K / 2;
   CUtensorMap tx, tg;
-  memset(&tx, 0, sizeof(tx)); memset(&tg, 0, sizeof(tg));
-  const bool in8 = cin_real == 8 && Cin == 16, out8 = cout_real == 8 && Cout == 16;
-  bool tma = g_use_tma && up == 0 && (cin_real == Cin || in8) && (cout_real == Cout || out8);
-  ttg_encode_tiled_fn enc = tma ? ttg_get_encode_tiled() : nullptr;
-  if (!enc) tma = false;
-  if (fuse == 3 && !tma) return ttg_set_error(TTG_ERR_UNSUPPORTED, "conv2d_wgrad_tc: the kx-folded variant needs the TMA path");
-  if (tma && fuse == 3) {
+  CUresult r1, r2;
+  if (fuse == 3) {
     const cuuint32_t estr[4] = {1, 1, 1, 1};
     const cuuint64_t xd[4] = {(cuuint64_t)cin_real, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
     const cuuint64_t xs[3] = {(cuuint64_t)cin_real * 2, (cuuint64_t)W * cin_real * 2, (cuuint64_t)H * W * cin_real * 2};
@@ -2565,51 +1617,38 @@ static int launch_wgrad_ws(const void* x, const void* gy, float* gw, int N, int 
     const cuuint64_t gs[3] = {(cuuint64_t)cout_real * 2, (cuuint64_t)W * cout_real * 2, (cuuint64_t)H * W * cout_real * 2};
     const cuuint32_t gb[4] = {(cuuint32_t)Cout, TC_TW + 2, TC_TH, 1};
     auto swz_of = [](int c) { return c == 16 ? CU_TENSOR_MAP_SWIZZLE_32B : c == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B; };
-    CUresult r1 = enc(&tx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), xd, xs, xb, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                      swz_of(Cin), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    CUresult r2 = enc(&tg, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(gy), gd, gs, gb, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                      swz_of(Cout), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r1 != CUDA_SUCCESS || r2 != CUDA_SUCCESS)
-      return ttg_set_error(TTG_ERR_CUDA, "conv2d_wgrad_tc: cuTensorMapEncodeTiled failed (%d, %d)", (int)r1, (int)r2);
-  } else if (tma) {
+    r1 = enc(&tx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), xd, xs, xb, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+             swz_of(Cin), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    r2 = enc(&tg, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(gy), gd, gs, gb, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+             swz_of(Cout), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  } else {
     const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
     const cuuint64_t xd[5] = {8, (cuuint64_t)W, (cuuint64_t)(cin_real / 8), (cuuint64_t)H, (cuuint64_t)N};
     const cuuint64_t xs[4] = {(cuuint64_t)cin_real * 2, 16, (cuuint64_t)W * cin_real * 2, (cuuint64_t)H * W * cin_real * 2};
-    const cuuint32_t xb[5] = {8, (cuuint32_t)(fuse == 3 ? TC_TW : TC_TW + 2 * HALO), (cuuint32_t)(Cin / 8), (cuuint32_t)(TC_TH + 2 * HALO), 1};
+    const cuuint32_t xb[5] = {8, (cuuint32_t)(TC_TW + 2 * HALO), (cuuint32_t)(Cin / 8), (cuuint32_t)(TC_TH + 2 * HALO), 1};
     const int g8n = (Cout < 128 ? Cout : 128) / 8;
     const cuuint64_t gd[5] = {8, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)(cout_real / 8), (cuuint64_t)N};
     const cuuint64_t gs[4] = {(cuuint64_t)cout_real * 2, (cuuint64_t)W * cout_real * 2, 16, (cuuint64_t)H * W * cout_real * 2};
     const cuuint32_t gb[5] = {8, TC_TW, TC_TH, (cuuint32_t)g8n, 1};
-    CUresult r1 = enc(&tx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), xd, xs, xb, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                      CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    CUresult r2 = enc(&tg, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(gy), gd, gs, gb, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                      CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r1 != CUDA_SUCCESS || r2 != CUDA_SUCCESS)
-      return ttg_set_error(TTG_ERR_CUDA, "conv2d_wgrad_tc: cuTensorMapEncodeTiled failed (%d, %d)", (int)r1, (int)r2);
+    r1 = enc(&tx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), xd, xs, xb, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    r2 = enc(&tg, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(gy), gd, gs, gb, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   }
-  static int smem_set[2] = {0, 0};
-  if (smem > smem_set[tma ? 1 : 0]) {
-    cudaError_t e = tma ? cudaFuncSetAttribute(conv_wgrad_tc_ws_kernel<K, NBUF, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)
-                        : cudaFuncSetAttribute(conv_wgrad_tc_ws_kernel<K, NBUF, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  if (r1 != CUDA_SUCCESS || r2 != CUDA_SUCCESS)
+    return ttg_set_error(TTG_ERR_CUDA, "conv2d_wgrad_tc: cuTensorMapEncodeTiled failed (%d, %d)", (int)r1, (int)r2);
+  static int smem_set = 0;
+  if (smem > smem_set) {
+    cudaError_t e = cudaFuncSetAttribute(conv_wgrad_tc_ws_kernel<K, NBUF>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return ttg_set_error(TTG_ERR_CUDA, "conv2d_wgrad_tc: smem attribute: %s", cudaGetErrorString(e));
-    smem_set[tma ? 1 : 0] = smem;
+    smem_set = smem;
   }
-  if (tma)
-    conv_wgrad_tc_ws_kernel<K, NBUF, true><<<grid, 256, smem, st>>>((const bf16*)x, (const bf16*)gy, gw, N, H, W, Cin, Cout, up, upg,
-                                                                   fuse, cols, g_bytes, cin_real, cout_real, tx, tg, gbias);
-  else
-    conv_wgrad_tc_ws_kernel<K, NBUF, false><<<grid, 256, smem, st>>>((const bf16*)x, (const bf16*)gy, gw, N, H, W, Cin, Cout, up, upg,
-                                                                    fuse, cols, g_bytes, cin_real, cout_real, tx, tg, nullptr);
-  *bias_done = tma && gbias != nullptr;
+  conv_wgrad_tc_ws_kernel<K, NBUF><<<grid, 256, smem, st>>>(gw, N, H, W, Cin, Cout, upg, fuse, cols, g_bytes, cout_real, tx, tg, gbias);
   TTG_CHECK_LAUNCH("conv2d_wgrad_tc_ws");
   return TTG_OK;
 }
 
 static int g_wgrad_tc_smem[2] = {0, 0};
-static int g_wg_nbuf = 0, g_wg_persm = 0;     // experiments: ring depth / resident CTAs of the folded wgrad variant
-extern "C" int ttg_set_wgrad_tuning(int nbuf, int persm) { g_wg_nbuf = nbuf; g_wg_persm = persm; return TTG_OK; }
-static int g_use_mfold = 1;
-extern "C" int ttg_set_wgrad_mfold(int on) { g_use_mfold = on ? 1 : 0; return TTG_OK; }   // A/B switch (tools/kbench.py)
 
 // packed partial-sum image -> OIHW fp32 (layout 0: gwp[tap][co][ci], 1: gwp[tap][ci][co]; padded sizes CoutP x CinP)
 // acc != 0: added to gw (a view of the flat .grad buffer) instead of overwriting it
@@ -2627,50 +1666,44 @@ extern "C" size_t ttg_conv2d_wgrad_tc_workspace_bytes(int Cin, int Cout, int ksi
   return sizeof(float) * (size_t)ttg_pad16(Cin) * ttg_pad16(Cout) * ksize * ksize + 16 + 8 * 256 + 16;   // + channel-sum scratch (fp64 [C])
 }
 
-extern "C" int ttg_conv2d_wgrad_tc_ex(const void* x, const void* gy, float* gw, int N, int H, int W, int Cin, int Cout,
-                                      int cin_real, int cout_real, int ksize, int up, void* workspace, void* stream);
-extern "C" int ttg_conv2d_wgrad_tc(const void* x, const void* gy, float* gw, int N, int H, int W, int Cin, int Cout,
-                                   int ksize, int up, void* workspace, void* stream) {
-  return ttg_conv2d_wgrad_tc_ex(x, gy, gw, N, H, W, Cin, Cout, Cin, Cout, ksize, up, workspace, stream);
-}
 extern "C" int ttg_channel_sum_acc(const void* x, long long M, int C, float* out, int accumulate, void* workspace, int dtype, void* stream);
 static int wgrad_tc_core(const void* x, const void* gy, float* gw, float* gbias, int N, int H, int W, int Cin, int Cout,
-                         int cin_real, int cout_real, int ksize, int up, void* workspace, void* stream, int accumulate = 0);
+                         int cin_real, int cout_real, int ksize, void* workspace, void* stream, int accumulate = 0);
 extern "C" int ttg_conv2d_wgrad_tc_ex(const void* x, const void* gy, float* gw, int N, int H, int W, int Cin, int Cout,
-                                      int cin_real, int cout_real, int ksize, int up, void* workspace, void* stream) {
-  return wgrad_tc_core(x, gy, gw, nullptr, N, H, W, Cin, Cout, cin_real, cout_real, ksize, up, workspace, stream);
+                                      int cin_real, int cout_real, int ksize, void* workspace, void* stream) {
+  return wgrad_tc_core(x, gy, gw, nullptr, N, H, W, Cin, Cout, cin_real, cout_real, ksize, workspace, stream);
+}
+extern "C" int ttg_conv2d_wgrad_tc(const void* x, const void* gy, float* gw, int N, int H, int W, int Cin, int Cout,
+                                   int ksize, void* workspace, void* stream) {
+  return ttg_conv2d_wgrad_tc_ex(x, gy, gw, N, H, W, Cin, Cout, Cin, Cout, ksize, workspace, stream);
 }
 // wgrad + bias gradient (gbias[co] = sum over pixels of gy[., co], fp32) in one pass over gy: the idle warps of the
 // TMA-fed wgrad kernel add up the gy tiles while the tensor cores consume them (Conv2d bias gradient of
-// convolution_backward).  Falls back to ttg_channel_sum internally where the fused path does not apply.
+// convolution_backward).  The Cin = 256 layers (conv_wgrad_tc_kernel) use ttg_channel_sum internally instead.
 extern "C" int ttg_conv2d_wgrad_bias_tc_ex(const void* x, const void* gy, float* gw, float* gbias, int N, int H, int W, int Cin,
-                                           int Cout, int cin_real, int cout_real, int ksize, int up, void* workspace,
-                                           void* stream) {
+                                           int Cout, int cin_real, int cout_real, int ksize, void* workspace, void* stream) {
   TTG_REQUIRE(gbias != nullptr, "conv2d_wgrad_bias_tc: gbias is required");
-  return wgrad_tc_core(x, gy, gw, gbias, N, H, W, Cin, Cout, cin_real, cout_real, ksize, up, workspace, stream);
+  return wgrad_tc_core(x, gy, gw, gbias, N, H, W, Cin, Cout, cin_real, cout_real, ksize, workspace, stream);
 }
 // gw += / gbias += variant: the weight (and optional bias) gradient is accumulated into the caller's buffers
 // (views of the flat .grad buffer of the model), which removes autograd's per-parameter add kernels.
 // flags: bit 0 = accumulate (always set by this entry point's callers), bit 1 = the workspace is already all zero
 extern "C" int ttg_conv2d_wgrad_tc_acc(const void* x, const void* gy, float* gw, float* gbias, int N, int H, int W, int Cin,
-                                       int Cout, int cin_real, int cout_real, int ksize, int up, int flags, void* workspace,
+                                       int Cout, int cin_real, int cout_real, int ksize, int flags, void* workspace,
                                        void* stream) {
-  return wgrad_tc_core(x, gy, gw, gbias, N, H, W, Cin, Cout, cin_real, cout_real, ksize, up, workspace, stream, flags | 1);
+  return wgrad_tc_core(x, gy, gw, gbias, N, H, W, Cin, Cout, cin_real, cout_real, ksize, workspace, stream, flags | 1);
 }
 static int wgrad_tc_core(const void* x, const void* gy, float* gw, float* gbias, int N, int H, int W, int Cin, int Cout,
-                         int cin_real, int cout_real, int ksize, int up, void* workspace, void* stream, int accumulate) {
+                         int cin_real, int cout_real, int ksize, void* workspace, void* stream, int accumulate) {
   cudaStream_t st = (cudaStream_t)stream;
   TTG_REQUIRE(workspace != nullptr && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0, "conv2d_wgrad_tc: workspace must be 16-byte aligned");
   float* gwp = reinterpret_cast<float*>(workspace);
   const bool padded = cin_real != Cin || cout_real != Cout;
-  TTG_REQUIRE(!(cin_real == 8 && Cin == 16) && !(cout_real == 8 && Cout == 16) || (up == 0 && g_use_tma && ttg_get_encode_tiled() != nullptr),
-              "conv2d_wgrad_tc: 8-channel staging tensors need the TMA path");
-  TTG_REQUIRE(!padded || ((cin_real == Cin || cin_real <= 8) && (cout_real == Cout || cout_real <= 8)),
-              "conv2d_wgrad_tc: channel padding supports <= 8 real channels");
+  TTG_REQUIRE((cin_real == Cin || (cin_real == 8 && Cin == 16)) && (cout_real == Cout || (cout_real == 8 && Cout == 16)),
+              "conv2d_wgrad_tc: channel padding supports 8-channel staging tensors (ttg_pad_channels8) only");
   TTG_REQUIRE(ksize == 1 || ksize == 3, "conv2d_wgrad_tc: ksize %d unsupported", ksize);
   TTG_REQUIRE(Cin % 16 == 0 && Cout % 16 == 0 && Cin >= 16 && Cout >= 16 && Cin <= 256 && Cout <= 256,
               "conv2d_wgrad_tc: channels must be multiples of 16 in [16,256] (got %d -> %d)", Cin, Cout);
-  TTG_REQUIRE(up == 0 || (H % 2 == 0 && W % 2 == 0), "conv2d_wgrad_tc: upsample needs even output size");
   const int taps = ksize * ksize;
   int tpg = 512 / Cin;                 // accumulator columns: taps_per_group * Cin <= 512
   if (tpg > taps) tpg = taps;
@@ -2688,12 +1721,9 @@ static int wgrad_tc_core(const void* x, const void* gy, float* gw, float* gbias,
     // persistent warp-specialised variant when at least two (x, gy) slots fit in shared memory
     // measured: the swapped orientation only pays when the input is wider than the output (32->16: 204 -> 175 us);
     // for Cin <= Cout the MMA count, not the MMA shape, is what bounds these narrow layers
-    // kx folded into M and ky into N (fuse 3, TMA-fed tiles only): 8 MMAs per tile instead of 24 for the narrow
-    // layers, which are bound by the MMA count (16->16 @128^2: 131 us with 24 small MMAs per 128 pixels)
-    const bool in8_ = cin_real == 8 && Cin == 16, out8_ = cout_real == 8 && Cout == 16;
-    const bool tma_ok = g_use_tma && up == 0 && (cin_real == Cin || in8_) && (cout_real == Cout || out8_) &&
-                        ttg_get_encode_tiled() != nullptr;
-    const bool mfold = g_use_mfold && tma_ok && ksize == 3 && (Cout == 16 || Cout == 32) && (Cin == 16 || Cin == 32 || Cin == 64);
+    // kx folded into M and ky into N (fuse 3): 8 MMAs per tile instead of 24 for the narrow layers, which are bound
+    // by the MMA count (16->16 @128^2: 131 us with 24 small MMAs per 128 pixels)
+    const bool mfold = ksize == 3 && (Cout == 16 || Cout == 32) && (Cin == 16 || Cin == 32 || Cin == 64);
     const bool swap_ok = !mfold && ksize == 3 && 3 * Cin <= 128 && Cout <= 128 && Cin > Cout;
     const int fuse = mfold ? 3 : swap_ok ? 2 : ((ksize == 3 && 3 * Cin <= 256) ? 1 : 0);
     const int units_total = mfold ? 1 : fuse ? 3 : taps;
@@ -2711,7 +1741,7 @@ static int wgrad_tc_core(const void* x, const void* gy, float* gw, float* gbias,
     // swapped orientation: the padding rows of the A operand (ky = 3) reach one halo row past the last x slot
     const int xpad = swap_ok ? 2 * (Cin / 8) * (TC_TW + 2 * halo) * 16 : 0;
     int nbuf = (200 * 1024 - reach) / (x_bytes + g_bytes);
-    const int nbuf_cap = mfold ? (g_wg_nbuf > 0 ? g_wg_nbuf : 8) : 4;     // the folded variant's pipeline is latency bound: deeper ring
+    const int nbuf_cap = mfold ? 8 : 4;     // the folded variant's pipeline is latency bound: deeper ring
     if (nbuf > nbuf_cap) nbuf = nbuf_cap;
     if (nbuf == 5) nbuf = 4;
     if (nbuf == 7) nbuf = 6;
@@ -2723,16 +1753,14 @@ static int wgrad_tc_core(const void* x, const void* gy, float* gw, float* gbias,
       const int wsmem = body + xpad + 1024;          // barriers + the bias partial sums
       if (wper_sm > (220 * 1024) / wsmem) wper_sm = (220 * 1024) / wsmem;
       if (wper_sm > 4) wper_sm = 4;
-      if (g_wg_persm > 0 && wper_sm > g_wg_persm) wper_sm = g_wg_persm;
       if (wper_sm < 1) wper_sm = 1;
       long long wsplits = (long long)ttg_num_sms() * wper_sm / (wgroups * halves);
       if (wsplits < 1) wsplits = 1;
       if (wsplits > tiles) wsplits = tiles;
       if (!(accumulate & 2)) cudaMemsetAsync(gwp, 0, sizeof(float) * (size_t)Cout * Cin * taps, st);
       if (gbias && !(accumulate & 1)) cudaMemsetAsync(gbias, 0, sizeof(float) * (size_t)cout_real, st);
-      bool bias_done = false;
       dim3 wgrid((unsigned)wsplits, wgroups, halves);
-#define TTG_WG(KK, NB) launch_wgrad_ws<KK, NB>(x, gy, gwp, N, H, W, Cin, Cout, up, upg, fuse, wcols, g_bytes, wsmem, wgrid, cin_real, cout_real, gbias, &bias_done, st)
+#define TTG_WG(KK, NB) launch_wgrad_ws<KK, NB>(x, gy, gwp, N, H, W, Cin, Cout, upg, fuse, wcols, g_bytes, wsmem, wgrid, cin_real, cout_real, gbias, st)
       int rc;
       if (ksize == 3) rc = nbuf == 8 ? TTG_WG(3, 8) : nbuf == 6 ? TTG_WG(3, 6) : nbuf == 4 ? TTG_WG(3, 4) : nbuf == 3 ? TTG_WG(3, 3) : TTG_WG(3, 2);
       else rc = nbuf == 4 ? TTG_WG(1, 4) : nbuf == 3 ? TTG_WG(1, 3) : TTG_WG(1, 2);
@@ -2741,10 +1769,6 @@ static int wgrad_tc_core(const void* x, const void* gy, float* gw, float* gbias,
       const int total = cout_real * cin_real * taps;
       ttg_wgrad_unpack_kernel<<<ttg_grid_for(total, 256), 256, 0, st>>>(gwp, gw, cout_real, cin_real, Cout, Cin, taps, swap_ok ? 1 : 0, accumulate & 1);
       TTG_CHECK_LAUNCH("conv2d_wgrad_unpack");
-      if (gbias && !bias_done) {
-        void* scratch = reinterpret_cast<uint8_t*>(workspace) + ((sizeof(float) * (size_t)Cout * Cin * taps + 15) & ~(size_t)15);
-        return ttg_channel_sum_acc(gy, (long long)N * H * W, cout_real, gbias, accumulate, scratch, TTG_BF16, stream);
-      }
       return TTG_OK;
     }
   }
@@ -2763,9 +1787,9 @@ static int wgrad_tc_core(const void* x, const void* gy, float* gw, float* gbias,
   if (!(accumulate & 1)) cudaMemsetAsync(gw, 0, sizeof(float) * (size_t)Cout * Cin * taps, st);
   dim3 grid((unsigned)splits, groups, halves);
   if (ksize == 3)
-    conv_wgrad_tc_kernel<3><<<grid, 128, smem, st>>>((const bf16*)x, (const bf16*)gy, gw, N, H, W, Cin, Cout, up, tpg, cols);
+    conv_wgrad_tc_kernel<3><<<grid, 128, smem, st>>>((const bf16*)x, (const bf16*)gy, gw, N, H, W, Cin, Cout, tpg, cols);
   else
-    conv_wgrad_tc_kernel<1><<<grid, 128, smem, st>>>((const bf16*)x, (const bf16*)gy, gw, N, H, W, Cin, Cout, up, tpg, cols);
+    conv_wgrad_tc_kernel<1><<<grid, 128, smem, st>>>((const bf16*)x, (const bf16*)gy, gw, N, H, W, Cin, Cout, tpg, cols);
   TTG_CHECK_LAUNCH("conv2d_wgrad_tc");
   if (gbias) {
     void* scratch = reinterpret_cast<uint8_t*>(workspace) + ((sizeof(float) * (size_t)Cout * Cin * taps + 15) & ~(size_t)15);

@@ -253,39 +253,11 @@ __global__ void bilinear_down_bwd_kernel(const T* __restrict__ gy, const T* __re
     }
   }
 }
-// channel counts without a vector path (RGB, C = 3): one thread per ELEMENT, so that consecutive threads touch
-// consecutive 2-byte elements (the thread-per-pixel loop above took 98 us for a 256 x 128 x 128 x 3 gradient)
-template <typename T>
-__global__ void bilinear_down_bwd_elem_kernel(const T* __restrict__ gy, const T* __restrict__ add, T* __restrict__ gx, int N, int Hi, int Wi, int C) {
-  const int Ho = Hi / 2, Wo = Wi / 2;
-  const long long total = (long long)N * Hi * Wi * C;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const int c = (int)(i % C); const long long p = i / C;
-    const int ix = (int)(p % Wi); const long long q = p / Wi; const int iy = (int)(q % Hi); const int n = (int)(q / Hi);
-    int oys[4], oxs[4]; float wys[4], wxs[4];
-    const int ny = bil_candidates(iy, Hi, Ho, oys, wys), nx = bil_candidates(ix, Wi, Wo, oxs, wxs);
-    const T* gbase = gy + (long long)n * Ho * Wo * C + c;
-    float acc = add ? to_f(add[i]) : 0.f;
-    for (int a = 0; a < ny; ++a)
-      for (int b = 0; b < nx; ++b) acc += wys[a] * wxs[b] * to_f(gbase[((long long)oys[a] * Wo + oxs[b]) * C]);
-    gx[i] = from_f<T>(acc);
-  }
-}
 extern "C" int ttg_bilinear_down_bwd_add(const void* gy, const void* add, void* gx, int N, int Hi, int Wi, int C, int dtype, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
   const long long pixels = (long long)N * Hi * Wi;
-  // (measured in the step profile: ~200 us per RGB launch against ~98 us for the thread-per-pixel kernel below, whose
-  // per-pixel candidate search is shared by the channels; kept for A/B only)
   const size_t bsm = (size_t)(Hi + Wi) * 9 * sizeof(int);           // candidate tables of the thread-per-pixel kernel
   TTG_REQUIRE(bsm <= 48 * 1024, "bilinear_down_bwd: image too large for the candidate tables (%d x %d)", Hi, Wi);
-  static const bool use_elem = getenv("TTG_BILELEM") != nullptr;
-  if (C < 8 && use_elem) {
-    TTG_DISPATCH(dtype, {
-      bilinear_down_bwd_elem_kernel<T><<<ttg_grid_occ(bilinear_down_bwd_elem_kernel<T>, pixels * C, 256 * 4), 256, 0, st>>>((const T*)gy, (const T*)add, (T*)gx, N, Hi, Wi, C);
-    });
-    TTG_CHECK_LAUNCH("bilinear_down_bwd_elem");
-    return TTG_OK;
-  }
   const int pv = C >= 32 ? 1 : 0;
   TTG_DISPATCH(dtype, {
     if (vec2_ok<T>(C, gy, gx) && (add == nullptr || vec2_ok<T>(C, add, gx))) { bilinear_down_bwd_kernel<T, Vec<T>::N><<<ttg_grid_occ(bilinear_down_bwd_kernel<T, Vec<T>::N>, pixels * (pv ? C / Vec<T>::N : 1), 128 * 4, 128, bsm), 128, bsm, st>>>((const T*)gy, (const T*)add, (T*)gx, N, Hi, Wi, C, pv); }

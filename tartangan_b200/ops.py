@@ -240,7 +240,7 @@ def _wgrad_direct(x, gy, w, bias, up, want_b):
         ws, z = _ws_zero(_lib.lib.ttg_conv2d_wgrad_tc_workspace_bytes(cin, cout, k), x.device)
         fused_bias = want_b and cout >= 16
         call('ttg_conv2d_wgrad_tc_acc', ptr(x), ptr(gy), ptr(dw), ptr(db) if fused_bias else None, n, h, wd_, _pad16(cin),
-             _pad16(cout), cin, cout, k, 0, 1 | z, ptr(ws))
+             _pad16(cout), cin, cout, k, 1 | z, ptr(ws))
         if want_b and not fused_bias:
             ws2, z2 = _ws_zero(_lib.lib.ttg_bn_workspace_bytes(cout), x.device)
             call('ttg_channel_sum_acc', ptr(gy), n * h * wd_, cout, ptr(db), 1 | z2, ptr(ws2), dtype_code(gy.dtype))
@@ -433,16 +433,17 @@ def _conv_raw(x, w, bias, mode, up, out_dtype=None, stats=None):
     out_dtype = out_dtype or x.dtype
     y = empty_nhwc(n, c_out_eff, h, wd_, out_dtype, x.device)
     if _tc_ok(x.dtype, cin, cout) and out_dtype in (torch.bfloat16, torch.float32):
+        assert up == 0, 'tensor-core conv: conv2d() materialises the upsample first'
         wp = _packed(w, mode, 'tc')
         if stats is not None:
             call('ttg_conv2d_tc_stats', ptr(x), ptr(wp), ptr(bias), ptr(y), n, h, wd_, c_in_eff, c_out_eff, k, ptr(stats))
             return y
         # RGB layers: stage the <= 8-channel tensor as 8-channel pixels so the layer runs on the TMA kernels
-        stage8 = up == 0 and out_dtype == torch.bfloat16
+        stage8 = out_dtype == torch.bfloat16
         xin, cin_mem = (_pad8(x), 8) if (stage8 and c_in_eff < 8) else (x, c_in_eff)
         yout, cout_mem = (empty_nhwc(n, 8, h, wd_, out_dtype, x.device), 8) if (stage8 and c_out_eff < 8) else (y, c_out_eff)
         call('ttg_conv2d_tc_ex', ptr(xin), ptr(wp), ptr(bias), ptr(yout), n, h, wd_, _pad16(c_in_eff), _pad16(c_out_eff),
-             cin_mem, cout_mem, k, up, dtype_code(out_dtype), None, None, 1.0)
+             cin_mem, cout_mem, k, dtype_code(out_dtype))
         if yout is not y:
             call('ttg_unpad_channels8', ptr(yout), ptr(y), n * h * wd_, c_out_eff)
     else:
@@ -520,19 +521,20 @@ class ConvWgradFn(Function):
         cin = x.shape[1]
         gw = torch.empty((cout, cin, k, k), dtype=torch.float32, device=x.device)
         if _tc_ok(x.dtype, cin, cout) and gy.dtype == torch.bfloat16:
+            assert up == 0, 'tensor-core wgrad: conv2d() materialises the upsample first'
             ws = _ws(_lib.lib.ttg_conv2d_wgrad_tc_workspace_bytes(cin, cout, k), x.device)
-            if up == 0 and (cin < 8 or cout < 8):
+            if cin < 8 or cout < 8:
                 # RGB layers: 8-channel staging copies of the narrow operand(s); the extra rows / columns of the
                 # 8-channel weight gradient are zero and are dropped
                 xin, cin_mem = (_pad8(x), 8) if cin < 8 else (x, cin)
                 gin, cout_mem = (_pad8(gy), 8) if cout < 8 else (gy, cout)
                 gw8 = torch.empty((cout_mem, cin_mem, k, k), dtype=torch.float32, device=x.device)
                 call('ttg_conv2d_wgrad_tc_ex', ptr(xin), ptr(gin), ptr(gw8), n, h, w, _pad16(cin), _pad16(cout), cin_mem,
-                     cout_mem, k, up, ptr(ws))
+                     cout_mem, k, ptr(ws))
                 gw.copy_(gw8[:cout, :cin])
             else:
                 call('ttg_conv2d_wgrad_tc_ex', ptr(x), ptr(gy), ptr(gw), n, h, w, _pad16(cin), _pad16(cout), cin, cout, k,
-                     up, ptr(ws))
+                     ptr(ws))
         else:
             ws = _ws(_lib.lib.ttg_conv2d_wgrad_direct_workspace_bytes(n, h, w, cin, cout, k), x.device)
             call('ttg_conv2d_wgrad_direct_det', ptr(x), ptr(gy), ptr(gw), n, h, w, cin, cout, k, up,
@@ -565,12 +567,12 @@ class ConvWgradBiasFn(Function):
         ws = _ws(_lib.lib.ttg_conv2d_wgrad_tc_workspace_bytes(cin, cout, k), x.device)
         if cin < 8:           # RGB input: 8-channel staging copy, the extra columns of the gradient are dropped
             gw8 = torch.empty((cout, 8, k, k), dtype=torch.float32, device=x.device)
-            call('ttg_conv2d_wgrad_bias_tc_ex', ptr(_pad8(x)), ptr(gy), ptr(gw8), ptr(gb), n, h, w, 16, cout, 8, cout, k, 0,
+            call('ttg_conv2d_wgrad_bias_tc_ex', ptr(_pad8(x)), ptr(gy), ptr(gw8), ptr(gb), n, h, w, 16, cout, 8, cout, k,
                  ptr(ws))
             gw = gw8[:, :cin].contiguous()
         else:
             gw = torch.empty((cout, cin, k, k), dtype=torch.float32, device=x.device)
-            call('ttg_conv2d_wgrad_bias_tc_ex', ptr(x), ptr(gy), ptr(gw), ptr(gb), n, h, w, _pad16(cin), cout, cin, cout, k, 0,
+            call('ttg_conv2d_wgrad_bias_tc_ex', ptr(x), ptr(gy), ptr(gw), ptr(gb), n, h, w, _pad16(cin), cout, cin, cout, k,
                  ptr(ws))
         return gw, gb
 

@@ -87,20 +87,30 @@ class KernelProfiler:
 
     def record(self, name, args, e0, e1):
         key, nbytes, flops = '', 0, 0.0
-        if name in ('ttg_conv2d_tc', 'ttg_conv2d_direct'):
+        # the tensor-core entry points have no `up` argument (always 0); it is inserted to share the direct conv's layout
+        if name == 'ttg_conv2d_direct':
             key = _conv_key(args)
             nbytes, flops = _conv_bytes_flops(args)
-        elif name == 'ttg_conv2d_tc_ex':        # (x, wp, bias, y, N, H, W, CinP, CoutP, cin, cout, k, up, ...)
-            a = list(args[:4]) + list(args[4:7]) + [args[9], args[10], args[11], args[12]]
+        elif name in ('ttg_conv2d_tc', 'ttg_conv2d_tc_stats'):     # (x, wp, bias, y, N, H, W, Cin, Cout, k, ...)
+            a = list(args[:10]) + [0]
             key = _conv_key(a)
             nbytes, flops = _conv_bytes_flops(a)
             name = 'ttg_conv2d_tc'
-        elif name == 'ttg_conv2d_wgrad_tc_ex':  # (x, gy, gw, N, H, W, CinP, CoutP, cin, cout, k, up, ws)
-            a = list(args[:3]) + list(args[3:6]) + [args[8], args[9], args[10], args[11]]
+        elif name == 'ttg_conv2d_tc_ex':        # (x, wp, bias, y, N, H, W, CinP, CoutP, cin, cout, k, ...)
+            a = list(args[:4]) + list(args[4:7]) + [args[9], args[10], args[11], 0]
+            key = _conv_key(a)
+            nbytes, flops = _conv_bytes_flops(a)
+            name = 'ttg_conv2d_tc'
+        elif name == 'ttg_conv2d_wgrad_tc_ex':  # (x, gy, gw, N, H, W, CinP, CoutP, cin, cout, k, ws)
+            a = list(args[:3]) + list(args[3:6]) + [args[8], args[9], args[10], 0]
             key = _wgrad_key(a)
             nbytes, flops = _wgrad_bytes_flops(a)
             name = 'ttg_conv2d_wgrad_tc'
-        elif name in ('ttg_conv2d_wgrad_tc', 'ttg_conv2d_wgrad_direct', 'ttg_conv2d_wgrad_direct_det'):
+        elif name == 'ttg_conv2d_wgrad_tc':     # (x, gy, gw, N, H, W, Cin, Cout, k, ws)
+            a = list(args[:9]) + [0]
+            key = _wgrad_key(a)
+            nbytes, flops = _wgrad_bytes_flops(a)
+        elif name in ('ttg_conv2d_wgrad_direct', 'ttg_conv2d_wgrad_direct_det'):
             key = _wgrad_key(args)
             nbytes, flops = _wgrad_bytes_flops(args)
         elif name in ('ttg_bn_stats',):
@@ -113,8 +123,8 @@ class KernelProfiler:
             key = f'M{args[2]} C{args[3]}'
             nbytes = args[2] * args[3] * 2 * (2 if args[4] else 3)
             name = 'ttg_bn_act_fwd'
-        elif name in ('ttg_conv2d_wgrad_tc_acc', 'ttg_conv2d_wgrad_bias_tc_ex'):   # (x, gy, gw, gbias, N, H, W, CinP, CoutP, cin, cout, k, up, ws)
-            a = list(args[:3]) + list(args[4:7]) + [args[9], args[10], args[11], args[12]]
+        elif name in ('ttg_conv2d_wgrad_tc_acc', 'ttg_conv2d_wgrad_bias_tc_ex'):   # (x, gy, gw, gbias, N, H, W, CinP, CoutP, cin, cout, k, ...)
+            a = list(args[:3]) + list(args[4:7]) + [args[9], args[10], args[11], 0]
             key = _wgrad_key(a)
             nbytes, flops = _wgrad_bytes_flops(a)
             name = 'ttg_conv2d_wgrad_tc'
@@ -132,11 +142,6 @@ class KernelProfiler:
         elif name == 'ttg_bn_act_bwd2':
             key = f'M{args[5]} C{args[6]}'
             nbytes = args[5] * args[6] * 2 * 8          # reduce reads 3; apply reads 3 writes 2
-        elif name == 'ttg_conv2d_tc_stats':      # (x, wp, bias, y, N, H, W, Cin, Cout, k, sums): conv + statistics epilogue
-            a = list(args[:10]) + [0]
-            key = _conv_key(a)
-            nbytes, flops = _conv_bytes_flops(a)
-            name = 'ttg_conv2d_tc'
         elif name in _STREAM_MODELS:              # resampling / joins / layout / optimiser: bytes in + bytes out
             key, nbytes = _STREAM_MODELS[name](args)
         self.events.append((name, key, nbytes, flops, e0, e1))

@@ -103,31 +103,6 @@ def test_conv_static_kernels(cin, cout, hw, n):
     assert rel_l2(gxd, gx) < 1e-2 and rel_l2(gwd, gw) < 1e-2 and rel_l2(gbd, gb) < 1e-2
 
 
-@pytest.mark.parametrize('cin,cout,h,w,n', [(16, 16, 128, 128, 1), (16, 16, 10, 128, 3), (32, 32, 64, 64, 2), (32, 32, 6, 64, 5)])
-def test_conv_kx_folded_row_kernel(cin, cout, h, w, n):
-    """Layers that select conv_tc_fold_kernel (full-row tiles, horizontal taps folded into N): fprop and dgrad,
-    with a bias, image heights that are not a multiple of the 4-row tile, and against the tap-shift kernel."""
-    from tartangan_b200 import ops, _lib
-    torch.manual_seed(11)
-    x = torch.randn(n, cin, h, w).to(BF).float().requires_grad_()
-    wt = (torch.randn(cout, cin, 3, 3) / math.sqrt(cin * 9)).to(BF).float().requires_grad_()
-    b = torch.randn(cout, requires_grad=True)
-    y = F.conv2d(x, wt, b, padding=1)
-    gy = torch.randn_like(y).to(BF).float()
-    gx, = torch.autograd.grad(y, x, gy)
-    xd, wd, bd = x.detach().cuda().requires_grad_(), wt.detach().cuda(), b.detach().cuda()
-    _lib.lib.ttg_set_use_fold(1)               # the folded kernel is off by default (not faster, see conv_tc.cu)
-    try:
-        yd = ops.conv2d(ops.to_internal(xd, BF), wd, bd)
-        assert rel_l2(yd, y) < 1e-2
-        gxd, = torch.autograd.grad(yd, xd, _internal(gy))
-        assert rel_l2(gxd, gx) < 1e-2
-    finally:
-        _lib.lib.ttg_set_use_fold(0)
-    y_shift = ops.conv2d(ops.to_internal(xd, BF), wd, bd)
-    assert rel_l2(yd, y_shift) < 4e-3          # same operands, different summation order inside fp32 accumulators
-
-
 # ------------------------------------------------------------------ producer statistics
 @pytest.mark.parametrize('cin,cout,hw,n,k', [(16, 16, 32, 4, 3), (32, 64, 20, 3, 3), (128, 128, 16, 4, 3), (64, 32, 16, 2, 1)])
 def test_conv_epilogue_statistics(cin, cout, hw, n, k):

@@ -59,37 +59,3 @@ def test_tc_conv(cin, cout, k, h, w, n, up):
     assert l2 < 6e-3 and mx < 2e-2, ('dgrad', l2, mx)
     l2, mx = _rel(gwd, gw)
     assert l2 < 6e-3 and mx < 2e-2, ('wgrad', l2, mx)
-
-
-@pytest.mark.parametrize('c,co,k,h,w,n,up,rows', [
-    (32, 16, 3, 16, 16, 2, 0, 0), (16, 16, 3, 128, 128, 2, 0, 0), (16, 32, 3, 40, 24, 3, 0, 0), (64, 64, 3, 32, 32, 2, 0, 0),
-    (32, 32, 1, 64, 64, 2, 0, 0), (64, 32, 3, 12, 20, 2, 0, 0), (16, 16, 3, 64, 64, 2, 0, 1), (32, 16, 3, 128, 128, 2, 1, 1),
-    (64, 32, 3, 64, 64, 1, 1, 1), (16, 16, 1, 32, 32, 2, 1, 1), (32, 32, 3, 24, 40, 2, 0, 1)])
-def test_tc_conv_fused_prologue(c, co, k, h, w, n, up, rows):
-    """conv(lrelu(x*scale+shift)) with the BatchNorm + LeakyReLU applied inside the conv kernel (in place on the
-    TMA-delivered tile, or while the bulk-row kernel re-lays the tile out; up=1: nearest x2 upsample folded in too):
-    the padding must stay zero AFTER the activation."""
-    from tartangan_b200 import ops, _lib
-    torch.manual_seed(3 + c + h)
-    r = lambda t: t.bfloat16().float()
-    x = r(torch.randn(n, c, h >> up, w >> up))
-    wt = r(torch.randn(co, c, k, k) / math.sqrt(c * k * k))
-    scale, shift = torch.rand(c) + 0.5, torch.randn(c) * 0.3
-    a = r(F.leaky_relu(x * scale.view(1, -1, 1, 1) + shift.view(1, -1, 1, 1), 0.2))
-    if up:
-        a = F.interpolate(a, scale_factor=2, mode='nearest')
-    b = torch.randn(co)
-    y = F.conv2d(a, wt, b, padding=k // 2)
-    xd = ops.to_internal(x.cuda(), torch.bfloat16)
-    wd = wt.cuda()
-    wp = ops._packed(wd, 0, 'tc')
-    yd = ops.empty_nhwc(n, co, h, w, torch.bfloat16, 'cuda')
-    sc, sh, bd = scale.cuda(), shift.cuda(), b.cuda()
-    _lib.lib.ttg_set_use_rows(rows)
-    try:
-        _lib.call('ttg_conv2d_tc_pre', _lib.ptr(xd), _lib.ptr(wp), _lib.ptr(bd), _lib.ptr(yd), n, h, w, c, co, k, up, _lib.BF16,
-                  _lib.ptr(sc), _lib.ptr(sh), 0.2)
-    finally:
-        _lib.lib.ttg_set_use_rows(0)
-    l2, mx = _rel(yd, y)
-    assert l2 < 6e-3 and mx < 2e-2, (l2, mx)

@@ -24,16 +24,6 @@ def timeit(fn, reps=10):
 
 def main():
     kind = sys.argv[1]
-    if os.environ.get('TTG_FOLD'):
-        _lib.lib.ttg_set_use_fold(int(os.environ['TTG_FOLD']))
-    if os.environ.get('TTG_TMA_MODE'):
-        _lib.lib.ttg_set_use_tma(int(os.environ["TTG_TMA_MODE"]))
-    if os.environ.get('TTG_ROWS'):
-        _lib.lib.ttg_set_use_rows(int(os.environ['TTG_ROWS']))
-    if os.environ.get('TTG_SWZ'):
-        _lib.lib.ttg_set_use_swz(int(os.environ['TTG_SWZ']))
-    if os.environ.get('TTG_MFOLD'):
-        _lib.lib.ttg_set_wgrad_mfold(int(os.environ['TTG_MFOLD']))
     a = [int(v) for v in sys.argv[2:]]
     bf = torch.bfloat16
     if kind in ('conv', 'wgrad', 'convd'):
@@ -46,15 +36,7 @@ def main():
         if kind == 'conv':
             wp = ops._packed(wt, 0, 'tc')
             y = ops.empty_nhwc(n, cout, h, w, bf, 'cuda')
-            fn = lambda: call('ttg_conv2d_tc', ptr(x), ptr(wp), None, ptr(y), n, h, w, cin, cout, k, 0, _lib.BF16)
-            if os.environ.get('KB_PRE'):        # fused BatchNorm + LeakyReLU prologue (and KB_UP=1: fused nearest upsample)
-                up = int(os.environ.get('KB_UP', '0'))
-                xs = ops.empty_nhwc(n, cin, h >> up, w >> up, bf, 'cuda'); xs.normal_()
-                sc = torch.rand(cin, device='cuda') + 0.5; sh = torch.randn(cin, device='cuda') * 0.3
-                pre = os.environ['KB_PRE'] == '1'
-                fn = lambda: call('ttg_conv2d_tc_pre', ptr(xs), ptr(wp), None, ptr(y), n, h, w, cin, cout, k, up, _lib.BF16,
-                                  ptr(sc) if pre else None, ptr(sh) if pre else None, 0.2)
-                nbytes = n * h * w * cout * 2 + n * (h >> up) * (w >> up) * cin * 2
+            fn = lambda: call('ttg_conv2d_tc', ptr(x), ptr(wp), None, ptr(y), n, h, w, cin, cout, k, _lib.BF16)
         elif kind == 'convd':
             wp = ops._packed(wt, 0, 'direct')
             y = ops.empty_nhwc(n, cout, h, w, bf, 'cuda')
@@ -63,7 +45,7 @@ def main():
             gy = ops.empty_nhwc(n, cout, h, w, bf, 'cuda'); gy.normal_()
             gw = torch.empty(cout, cin, k, k, device='cuda')
             ws = torch.empty(_lib.lib.ttg_conv2d_wgrad_tc_workspace_bytes(cin, cout, k) // 4 + 4, device='cuda')
-            fn = lambda: call('ttg_conv2d_wgrad_tc', ptr(x), ptr(gy), ptr(gw), n, h, w, cin, cout, k, 0, ptr(ws))
+            fn = lambda: call('ttg_conv2d_wgrad_tc', ptr(x), ptr(gy), ptr(gw), n, h, w, cin, cout, k, ptr(ws))
         med, best = timeit(fn, reps)
         print(f'{kind} N{n} {h}x{w} {cin}->{cout} k{k}: median {med*1e3:.1f} us  best {best*1e3:.1f} us  '
               f'{nbytes/med/1e6:.0f} GB/s  {flops/med/1e9:.1f} TFLOP/s')
