@@ -24,8 +24,6 @@ SLOPE = 0.2
 import os as _os
 _NO_DIRECT = _os.environ.get('TTG_NO_DIRECT', '0') == '1'
 _NO_ARENA = _os.environ.get('TTG_NO_ARENA', '0') == '1'
-# TTG_SIDE_WGRAD=0: weight-gradient kernels stay on the launching stream (A/B; see side_wgrad below)
-_SIDE_WGRAD = _os.environ.get('TTG_SIDE_WGRAD', '1') == '1'
 # TTG_SKIP_STREAM=0: the skip branch of a residual block stays on the launching stream (A/B; see skip_branch below)
 _SKIP_STREAM = _os.environ.get('TTG_SKIP_STREAM', '1') == '1'
 
@@ -40,7 +38,7 @@ class _State:
     fused_attention = True         # tcgen05 attention kernels when the shape allows (else bmm / softmax / bmm)
     direct_grads = False           # inside direct_param_grads(): parameter gradients are added to p.grad by the kernels
     arena = None                   # ZeroArena of the running trainer (pre-zeroed workspaces), or None
-    wgrad_stream = None            # side stream of the in-place weight-gradient kernels (side_wgrad)
+    wgrad_stream = None            # side stream of the in-place weight-gradient kernels (_wgrad_direct)
     wgrad_pending = False          # kernels were launched on it since the last join_side_streams()
     pending_streams = set()        # other streams that carry parts of the running step (the trainer's D(fake) stream)
 
@@ -208,10 +206,6 @@ def _direct(p):
     return None
 
 
-import contextlib as _contextlib
-_null_ctx = _contextlib.nullcontext()
-
-
 def _wgrad_direct(x, gy, w, bias, up, want_b):
     """gw (and gb) of a tensor-core conv added straight into w.grad (bias.grad).  True if done."""
     cout, cin, k, _ = w.shape
@@ -225,18 +219,18 @@ def _wgrad_direct(x, gy, w, bias, up, want_b):
     # The weight gradient only feeds `.grad`: nothing later in backward depends on it, so it runs on a SIDE stream and
     # the dgrad / BatchNorm-backward chain on the launching stream does not wait for it.  The layers below 32x32 launch
     # 32-128 CTAs on 148 SMs (section 7b of DESIGN.md); their wgrad kernels now fill the SMs the chain leaves idle.
-    # All in-place weight-gradient kernels share the one side stream (no two of them ever add to a buffer
-    # concurrently); join_side_streams() orders the optimiser / all-reduce / next arena reset after them.
-    side = None
-    if _SIDE_WGRAD and x.is_cuda:
-        side = state.wgrad_stream
-        if side is None:
-            side = state.wgrad_stream = torch.cuda.Stream(device=x.device)
-        side.wait_stream(torch.cuda.current_stream())          # x, gy (and the cleared arena) are ready
-        x.record_stream(side)
-        gy.record_stream(side)
-        state.wgrad_pending = True
-    with torch.cuda.stream(side) if side is not None else _null_ctx:
+    # All in-place weight-gradient kernels share the one side stream, which is also what keeps them correct: the
+    # unpack of the partial sums and ttg_channel_sum_acc add to .grad with a plain read-modify-write, and the D(real)
+    # and D(fake) chains run on two streams.  join_side_streams() orders the optimiser / all-reduce / next arena
+    # reset after them.
+    side = state.wgrad_stream
+    if side is None:
+        side = state.wgrad_stream = torch.cuda.Stream(device=x.device)
+    side.wait_stream(torch.cuda.current_stream())              # x, gy (and the cleared arena) are ready
+    x.record_stream(side)
+    gy.record_stream(side)
+    state.wgrad_pending = True
+    with torch.cuda.stream(side):
         ws, z = _ws_zero(_lib.lib.ttg_conv2d_wgrad_tc_workspace_bytes(cin, cout, k), x.device)
         fused_bias = want_b and cout >= 16
         call('ttg_conv2d_wgrad_tc_acc', ptr(x), ptr(gy), ptr(dw), ptr(db) if fused_bias else None, n, h, wd_, _pad16(cin),
