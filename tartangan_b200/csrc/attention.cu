@@ -16,10 +16,11 @@ __global__ void maxpool2_fwd_kernel(const T* __restrict__ x, T* __restrict__ y, 
     int c = (int)(i % C); long long p = i / C;
     int ox = (int)(p % Wo); p /= Wo; int oy = (int)(p % Ho); int n = (int)(p / Ho);
     const T* s = x + (((long long)n * Ho * 2 + oy * 2) * Wi + ox * 2) * C + c;
+    // first maximum in window order; a NaN propagates and takes the index (the last NaN), like torch's max_pool2d
     float best = to_f(s[0]); int bi = 0;
-    float v = to_f(s[C]); if (v > best) { best = v; bi = 1; }
-    v = to_f(s[(long long)Wi * C]); if (v > best) { best = v; bi = 2; }
-    v = to_f(s[(long long)Wi * C + C]); if (v > best) { best = v; bi = 3; }
+    float v = to_f(s[C]); if (v > best || isnan(v)) { best = v; bi = 1; }
+    v = to_f(s[(long long)Wi * C]); if (v > best || isnan(v)) { best = v; bi = 2; }
+    v = to_f(s[(long long)Wi * C + C]); if (v > best || isnan(v)) { best = v; bi = 3; }
     y[i] = from_f<T>(best); idx[i] = (unsigned char)bi;
   }
 }
