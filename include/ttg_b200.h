@@ -154,6 +154,34 @@ int ttg_bn_act_bwd2_acc(const void* x, const void* ga, const void* u, void* g_ga
 int ttg_channel_sum_acc(const void* x, long long M, int C, float* out, int accumulate, void* workspace, int dtype,
                         void* stream);
 
+/* ---- train-mode BatchNorm + LeakyReLU with the fp64 channel sums exposed between the reduce and the apply pass, so
+ * that a caller can all-reduce them over the ranks of a data-parallel job (synchronised BatchNorm, --sync-bn).
+ * M: rows this call walks; count: pixel count the sums were taken over (world * M for equal shards; count == M is
+ * what the combined entry points above compute, bit for bit).  flags / accumulate as above.  param_scale multiplies the
+ * gamma / beta gradients (1 / world: the gradient all-reduce adds every rank's copy of the global value).
+ *   ttg_bn_sums: sums[2C] = {sum x, sum x^2}
+ *   ttg_bn_act_fwd_stats_n: ttg_bn_act_fwd_stats with statistics and running-variance correction over count
+ *   ttg_bn_act_bwd_reduce / _apply: ttg_bn_act_bwd_acc, sums[2C]; _apply with gx NULL writes the parameter gradients only
+ *   ttg_bn_act_bwd2_reduce / _apply: ttg_bn_act_bwd2_acc, sums[5C] */
+int ttg_bn_sums(const void* x, long long M, int C, double* sums, int flags, int dtype, void* stream);
+int ttg_bn_act_fwd_stats_n(const void* x, void* y, long long M, int C, long long count, const double* sums,
+                           const float* gamma, const float* beta, float eps, float momentum, float slope, float* mean,
+                           float* invstd, float* running_mean, float* running_var, long long* num_batches,
+                           long long count_mult, void* workspace, int dtype, void* stream);
+int ttg_bn_act_bwd_reduce(const void* x, const void* ga, long long M, int C, const float* mean, const float* invstd,
+                          const float* gamma, const float* beta, float slope, double* sums, int flags, int dtype,
+                          void* stream);
+int ttg_bn_act_bwd_apply(const void* x, const void* ga, void* gx, long long M, int C, long long count, const double* sums,
+                         const float* mean, const float* invstd, const float* gamma, const float* beta, float slope,
+                         float* ggamma, float* gbeta, float param_scale, int accumulate, int dtype, void* stream);
+int ttg_bn_act_bwd2_reduce(const void* x, const void* ga, const void* u, long long M, int C, const float* mean,
+                           const float* invstd, const float* gamma, const float* beta, float slope, double* sums,
+                           int flags, int dtype, void* stream);
+int ttg_bn_act_bwd2_apply(const void* x, const void* ga, const void* u, void* g_ga, void* g_x, long long M, int C,
+                          long long count, const double* sums, const float* mean, const float* invstd,
+                          const float* gamma, const float* beta, float slope, float* ggamma, float param_scale,
+                          int accumulate, int dtype, void* stream);
+
 /* ---- resampling / glue
  * pool2_sum: nn.AvgPool2d(2) with scale 0.25 (discriminator.py:67); adjoint of upsample2.
  * upsample2: F.interpolate nearest x2 (generator.py:58); adjoint of pool2_sum.

@@ -155,29 +155,48 @@ template <typename T> struct BnActFwdStatsOp {
     if (threadIdx.x == 0 && num_batches) *num_batches += 1;
   }
 };
+// {sum x, sum x^2} of x[M, C] into sums[2C] (fp64); flags bit 1: sums is already zero
+extern "C" int ttg_bn_sums(const void* x, long long M, int C, double* sums, int flags, int dtype, void* stream) {
+  TTG_REQUIRE(M > 0 && C > 0 && sums != nullptr, "bn_sums: bad arguments");
+  TTG_DISPATCH(dtype, {
+    StatsOp<T> r; r.in[0] = (const T*)x;
+    return launch_chan_reduce<T>("bn_stats", r, M, C, sums, (cudaStream_t)stream, (flags & 2) != 0);
+  });
+  return TTG_OK;
+}
+
 // train-mode BatchNorm + LeakyReLU in (at most) two launches: statistics (skipped when `sums` = {sum x, sum x^2} was
 // already produced by the conv / join kernel that wrote x) and one apply pass that also finalises the statistics.
-extern "C" int ttg_bn_act_fwd_stats(const void* x, void* y, long long M, int C, const double* sums, const float* gamma,
-                                    const float* beta, float eps, float momentum, float slope, float* mean, float* invstd,
-                                    float* running_mean, float* running_var, long long* num_batches, long long count_mult,
-                                    void* workspace, int dtype, void* stream) {
+// `count`: the pixel count the sums were taken over (synchronised BatchNorm: the sums of every rank, count = world * M);
+// the apply pass walks the M local rows.
+extern "C" int ttg_bn_act_fwd_stats_n(const void* x, void* y, long long M, int C, long long count, const double* sums,
+                                      const float* gamma, const float* beta, float eps, float momentum, float slope,
+                                      float* mean, float* invstd, float* running_mean, float* running_var,
+                                      long long* num_batches, long long count_mult, void* workspace, int dtype, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
-  TTG_REQUIRE(M > 0 && C > 0 && count_mult >= 1 && mean && invstd, "bn_act_fwd_stats: bad arguments");
-  TTG_REQUIRE(sums != nullptr || workspace != nullptr, "bn_act_fwd_stats: needs sums or a workspace to reduce them into");
+  TTG_REQUIRE(M > 0 && C > 0 && count >= M && count_mult >= 1 && mean && invstd, "bn_act_fwd_stats: bad arguments");
+  TTG_REQUIRE(sums != nullptr || (workspace != nullptr && count == M),
+              "bn_act_fwd_stats: needs sums, or a workspace to reduce the local sums into (then count == M)");
+  if (sums == nullptr) {
+    int rc = ttg_bn_sums(x, M, C, (double*)workspace, 0, dtype, stream);
+    if (rc) return rc;
+    sums = (const double*)workspace;
+  }
   TTG_DISPATCH(dtype, {
-    if (sums == nullptr) {
-      StatsOp<T> r; r.in[0] = (const T*)x;
-      int rc = launch_chan_reduce<T>("bn_stats", r, M, C, (double*)workspace, st);
-      if (rc) return rc;
-      sums = (const double*)workspace;
-    }
     BnActFwdStatsOp<T> op; op.in[0] = (const T*)x; op.out[0] = (T*)y;
     op.sums = sums; op.gamma = gamma; op.beta = beta; op.slope = slope; op.eps = eps; op.momentum = momentum;
-    op.M = M; op.invM = 1.0 / (double)M; op.count_mult = count_mult; op.C = C; op.mean = mean; op.invstd = invstd;
+    op.M = count; op.invM = 1.0 / (double)count; op.count_mult = count_mult; op.C = C; op.mean = mean; op.invstd = invstd;
     op.running_mean = running_mean; op.running_var = running_var; op.num_batches = num_batches;
     return launch_chan_map<T>("bn_act_fwd_stats", op, M * C, C, st);
   });
   return TTG_OK;
+}
+extern "C" int ttg_bn_act_fwd_stats(const void* x, void* y, long long M, int C, const double* sums, const float* gamma,
+                                    const float* beta, float eps, float momentum, float slope, float* mean, float* invstd,
+                                    float* running_mean, float* running_var, long long* num_batches, long long count_mult,
+                                    void* workspace, int dtype, void* stream) {
+  return ttg_bn_act_fwd_stats_n(x, y, M, C, M, sums, gamma, beta, eps, momentum, slope, mean, invstd, running_mean,
+                                running_var, num_batches, count_mult, workspace, dtype, stream);
 }
 
 // ---------------------------------------------------------------- backward
@@ -208,11 +227,13 @@ template <typename T> struct BnActBwdMapOp {
   const T* in[2]; T* out[1];
   const float *mean, *invstd, *gamma, *beta; float slope; const double* sums; int C; float invM;
   float *ggamma, *gbeta; int acc;                      // parameter gradients (block 0), added to the buffers when acc
+  double pscale;                                       // ... times pscale
   __device__ void finalize(int) const {
     for (int c = threadIdx.x; c < C; c += blockDim.x) {
       // (accumulating: atomic, because the D(real) and D(fake) backward chains may run on two streams at once)
-      if (gbeta) { if (acc) atomicAdd(&gbeta[c], (float)sums[c]); else gbeta[c] = (float)sums[c]; }
-      if (ggamma) { if (acc) atomicAdd(&ggamma[c], (float)sums[C + c]); else ggamma[c] = (float)sums[C + c]; }
+      const float b = (float)(sums[c] * pscale), g = (float)(sums[C + c] * pscale);
+      if (gbeta) { if (acc) atomicAdd(&gbeta[c], b); else gbeta[c] = b; }
+      if (ggamma) { if (acc) atomicAdd(&ggamma[c], g); else ggamma[c] = g; }
     }
   }
   template <int V> struct P { BnChan<V> c; float db[V], cc[V]; };
@@ -229,46 +250,64 @@ template <typename T> struct BnActBwdMapOp {
 };
 // acc != 0: the parameter gradients are ADDED to ggamma / gbeta (the caller passes views of the flat .grad buffer, so
 // autograd's AccumulateGrad add kernels disappear)
-__global__ void bn_param_grads_kernel(const double* sums, int C, float* ggamma, float* gbeta, int acc) {
+__global__ void bn_param_grads_kernel(const double* sums, int C, float* ggamma, float* gbeta, int acc, double pscale) {
   int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c < C) {
-    if (gbeta) { if (acc) atomicAdd(&gbeta[c], (float)sums[c]); else gbeta[c] = (float)sums[c]; }
-    if (ggamma) { if (acc) atomicAdd(&ggamma[c], (float)sums[C + c]); else ggamma[c] = (float)sums[C + c]; }
+    const float b = (float)(sums[c] * pscale), g = (float)(sums[C + c] * pscale);
+    if (gbeta) { if (acc) atomicAdd(&gbeta[c], b); else gbeta[c] = b; }
+    if (ggamma) { if (acc) atomicAdd(&ggamma[c], g); else ggamma[c] = g; }
   }
+}
+
+// The backward as two entry points, so that the 2C sums can be all-reduced between them (synchronised BatchNorm).
+// reduce: sums[2C] = {sum d, sum d*xhat} over the M local rows; flags bit 1: sums is already zero.
+extern "C" int ttg_bn_act_bwd_reduce(const void* x, const void* ga, long long M, int C, const float* mean,
+                                     const float* invstd, const float* gamma, const float* beta, float slope, double* sums,
+                                     int flags, int dtype, void* stream) {
+  TTG_REQUIRE(M > 0 && C > 0 && sums != nullptr, "bn_act_bwd_reduce: bad arguments");
+  TTG_DISPATCH(dtype, {
+    BnActBwdRedOp<T> r; r.in[0] = (const T*)x; r.in[1] = (const T*)ga;
+    r.mean = mean; r.invstd = invstd; r.gamma = gamma; r.beta = beta; r.slope = slope;
+    return launch_chan_reduce<T>("bn_act_bwd_reduce", r, M, C, sums, (cudaStream_t)stream, (flags & 2) != 0);
+  });
+  return TTG_OK;
+}
+// apply: gx over the M local rows from sums taken over `count` pixels; ggamma / gbeta = param_scale * sums (written, or
+// added when accumulate bit 0 is set).  gx NULL: parameter gradients only.
+extern "C" int ttg_bn_act_bwd_apply(const void* x, const void* ga, void* gx, long long M, int C, long long count,
+                                    const double* sums, const float* mean, const float* invstd, const float* gamma,
+                                    const float* beta, float slope, float* ggamma, float* gbeta, float param_scale,
+                                    int accumulate, int dtype, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  TTG_REQUIRE(M > 0 && C > 0 && count >= M && sums != nullptr, "bn_act_bwd_apply: bad arguments");
+  if (gx) {
+    TTG_DISPATCH(dtype, {
+      BnActBwdMapOp<T> m; m.in[0] = (const T*)x; m.in[1] = (const T*)ga; m.out[0] = (T*)gx;
+      m.mean = mean; m.invstd = invstd; m.gamma = gamma; m.beta = beta; m.slope = slope;
+      m.sums = sums; m.C = C; m.invM = 1.f / (float)count;
+      m.ggamma = ggamma; m.gbeta = gbeta; m.acc = accumulate & 1; m.pscale = (double)param_scale;
+      return launch_chan_map<T>("bn_act_bwd_apply", m, M * C, C, st);
+    });
+  } else if (ggamma || gbeta) {                         // (with gx the apply pass writes them)
+    bn_param_grads_kernel<<<(C + 127) / 128, 128, 0, st>>>(sums, C, ggamma, gbeta, accumulate & 1, (double)param_scale);
+    TTG_CHECK_LAUNCH("bn_param_grads");
+  }
+  return TTG_OK;
 }
 
 extern "C" int ttg_bn_act_bwd_acc(const void* x, const void* ga, void* gx, long long M, int C, const float* mean,
                                   const float* invstd, const float* gamma, const float* beta, float slope, float* ggamma,
-                                  float* gbeta, int accumulate, void* workspace, int dtype, void* stream);
+                                  float* gbeta, int accumulate, void* workspace, int dtype, void* stream) {
+  int rc = ttg_bn_act_bwd_reduce(x, ga, M, C, mean, invstd, gamma, beta, slope, (double*)workspace, accumulate & 2, dtype,
+                                 stream);
+  if (rc) return rc;
+  return ttg_bn_act_bwd_apply(x, ga, gx, M, C, M, (const double*)workspace, mean, invstd, gamma, beta, slope, ggamma,
+                              gbeta, 1.f, accumulate & 1, dtype, stream);
+}
 extern "C" int ttg_bn_act_bwd(const void* x, const void* ga, void* gx, long long M, int C, const float* mean,
                               const float* invstd, const float* gamma, const float* beta, float slope, float* ggamma,
                               float* gbeta, void* workspace, int dtype, void* stream) {
   return ttg_bn_act_bwd_acc(x, ga, gx, M, C, mean, invstd, gamma, beta, slope, ggamma, gbeta, 0, workspace, dtype, stream);
-}
-extern "C" int ttg_bn_act_bwd_acc(const void* x, const void* ga, void* gx, long long M, int C, const float* mean,
-                                  const float* invstd, const float* gamma, const float* beta, float slope, float* ggamma,
-                                  float* gbeta, int accumulate, void* workspace, int dtype, void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
-  double* ws = (double*)workspace;
-  TTG_DISPATCH(dtype, {
-    BnActBwdRedOp<T> r; r.in[0] = (const T*)x; r.in[1] = (const T*)ga;
-    r.mean = mean; r.invstd = invstd; r.gamma = gamma; r.beta = beta; r.slope = slope;
-    int rc = launch_chan_reduce<T>("bn_act_bwd_reduce", r, M, C, ws, st, (accumulate & 2) != 0);
-    if (rc) return rc;
-    if (gx) {
-      BnActBwdMapOp<T> m; m.in[0] = (const T*)x; m.in[1] = (const T*)ga; m.out[0] = (T*)gx;
-      m.mean = mean; m.invstd = invstd; m.gamma = gamma; m.beta = beta; m.slope = slope;
-      m.sums = ws; m.C = C; m.invM = 1.f / (float)M;
-      m.ggamma = ggamma; m.gbeta = gbeta; m.acc = accumulate & 1;
-      rc = launch_chan_map<T>("bn_act_bwd_apply", m, M * C, C, st);
-      if (rc) return rc;
-    }
-  });
-  if (!gx && (ggamma || gbeta)) {                       // (with gx the apply pass wrote them)
-    bn_param_grads_kernel<<<(C + 127) / 128, 128, 0, st>>>(ws, C, ggamma, gbeta, accumulate & 1);
-    TTG_CHECK_LAUNCH("bn_param_grads");
-  }
-  return TTG_OK;
 }
 
 // ---------------------------------------------------------------- backward of backward
@@ -295,14 +334,15 @@ template <typename T> struct BnActBwd2MapOp {
   static constexpr int NIN = 3, NOUT = 2;
   const T* in[3]; T* out[2];   // out: g_ga, g_x
   const float *mean, *invstd, *gamma, *beta; float slope; const double* sums; int C; float invM;
-  float* ggamma; long long M; int acc;
+  float* ggamma; long long M; int acc;                 // M: the pixel count of the sums
+  double pscale;                                       // ggamma = pscale * g_gamma
   __device__ void finalize(int) const {
     if (!ggamma) return;
     for (int c = threadIdx.x; c < C; c += blockDim.x) {
       const double iM = 1.0 / (double)M;
       const double db = sums[c] * iM, cc = sums[C + c] * iM, ub = sums[2 * C + c] * iM, e = sums[3 * C + c] * iM;
       const double cov = sums[4 * C + c] * iM - ub * db;
-      const float v = (float)((double)invstd[c] * (double)M * (cov - cc * e));
+      const float v = (float)((double)invstd[c] * (double)M * (cov - cc * e) * pscale);
       if (acc) atomicAdd(&ggamma[c], v); else ggamma[c] = v;
     }
   }
@@ -338,33 +378,48 @@ __global__ void bn_bwd2_gamma_kernel(const double* sums, const float* invstd, lo
   }
 }
 
+// The same split for the double backward: reduce -> sums[5C] over the M local rows (flags bit 1: already zero);
+// apply -> g_ga, g_x over the M local rows from sums taken over `count` pixels, ggamma = param_scale * g_gamma.
+extern "C" int ttg_bn_act_bwd2_reduce(const void* x, const void* ga, const void* u, long long M, int C, const float* mean,
+                                      const float* invstd, const float* gamma, const float* beta, float slope,
+                                      double* sums, int flags, int dtype, void* stream) {
+  TTG_REQUIRE(M > 0 && C > 0 && sums != nullptr, "bn_act_bwd2_reduce: bad arguments");
+  TTG_DISPATCH(dtype, {
+    BnActBwd2RedOp<T> r; r.in[0] = (const T*)x; r.in[1] = (const T*)ga; r.in[2] = (const T*)u;
+    r.mean = mean; r.invstd = invstd; r.gamma = gamma; r.beta = beta; r.slope = slope;
+    return launch_chan_reduce<T>("bn_act_bwd2_reduce", r, M, C, sums, (cudaStream_t)stream, (flags & 2) != 0);
+  });
+  return TTG_OK;
+}
+extern "C" int ttg_bn_act_bwd2_apply(const void* x, const void* ga, const void* u, void* g_ga, void* g_x, long long M,
+                                     int C, long long count, const double* sums, const float* mean, const float* invstd,
+                                     const float* gamma, const float* beta, float slope, float* ggamma, float param_scale,
+                                     int accumulate, int dtype, void* stream) {
+  TTG_REQUIRE(M > 0 && C > 0 && count >= M && sums != nullptr, "bn_act_bwd2_apply: bad arguments");
+  TTG_DISPATCH(dtype, {
+    BnActBwd2MapOp<T> m; m.in[0] = (const T*)x; m.in[1] = (const T*)ga; m.in[2] = (const T*)u;
+    m.out[0] = (T*)g_ga; m.out[1] = (T*)g_x;
+    m.mean = mean; m.invstd = invstd; m.gamma = gamma; m.beta = beta; m.slope = slope;
+    m.sums = sums; m.C = C; m.invM = 1.f / (float)count;
+    m.ggamma = ggamma; m.M = count; m.acc = accumulate & 1; m.pscale = (double)param_scale;
+    return launch_chan_map<T>("bn_act_bwd2_apply", m, M * C, C, (cudaStream_t)stream);
+  });
+  return TTG_OK;
+}
+
 extern "C" int ttg_bn_act_bwd2_acc(const void* x, const void* ga, const void* u, void* g_ga, void* g_x, long long M, int C,
                                    const float* mean, const float* invstd, const float* gamma, const float* beta,
-                                   float slope, float* ggamma, int accumulate, void* workspace, int dtype, void* stream);
+                                   float slope, float* ggamma, int accumulate, void* workspace, int dtype, void* stream) {
+  int rc = ttg_bn_act_bwd2_reduce(x, ga, u, M, C, mean, invstd, gamma, beta, slope, (double*)workspace, accumulate & 2,
+                                  dtype, stream);
+  if (rc) return rc;
+  return ttg_bn_act_bwd2_apply(x, ga, u, g_ga, g_x, M, C, M, (const double*)workspace, mean, invstd, gamma, beta, slope,
+                               ggamma, 1.f, accumulate & 1, dtype, stream);
+}
 extern "C" int ttg_bn_act_bwd2(const void* x, const void* ga, const void* u, void* g_ga, void* g_x, long long M, int C,
                                const float* mean, const float* invstd, const float* gamma, const float* beta,
                                float slope, float* ggamma, void* workspace, int dtype, void* stream) {
   return ttg_bn_act_bwd2_acc(x, ga, u, g_ga, g_x, M, C, mean, invstd, gamma, beta, slope, ggamma, 0, workspace, dtype, stream);
-}
-extern "C" int ttg_bn_act_bwd2_acc(const void* x, const void* ga, const void* u, void* g_ga, void* g_x, long long M, int C,
-                                   const float* mean, const float* invstd, const float* gamma, const float* beta,
-                                   float slope, float* ggamma, int accumulate, void* workspace, int dtype, void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
-  double* ws = (double*)workspace;
-  TTG_DISPATCH(dtype, {
-    BnActBwd2RedOp<T> r; r.in[0] = (const T*)x; r.in[1] = (const T*)ga; r.in[2] = (const T*)u;
-    r.mean = mean; r.invstd = invstd; r.gamma = gamma; r.beta = beta; r.slope = slope;
-    int rc = launch_chan_reduce<T>("bn_act_bwd2_reduce", r, M, C, ws, st, (accumulate & 2) != 0);
-    if (rc) return rc;
-    BnActBwd2MapOp<T> m; m.in[0] = (const T*)x; m.in[1] = (const T*)ga; m.in[2] = (const T*)u;
-    m.out[0] = (T*)g_ga; m.out[1] = (T*)g_x;
-    m.mean = mean; m.invstd = invstd; m.gamma = gamma; m.beta = beta; m.slope = slope;
-    m.sums = ws; m.C = C; m.invM = 1.f / (float)M;
-    m.ggamma = ggamma; m.M = M; m.acc = accumulate & 1;
-    rc = launch_chan_map<T>("bn_act_bwd2_apply", m, M * C, C, st);
-    if (rc) return rc;
-  });
-  return TTG_OK;
 }
 
 // ---------------------------------------------------------------- plain LeakyReLU (--norm id)

@@ -41,6 +41,7 @@ class _State:
     wgrad_stream = None            # side stream of the in-place weight-gradient kernels (_wgrad_direct)
     wgrad_pending = False          # kernels were launched on it since the last join_side_streams()
     pending_streams = set()        # other streams that carry parts of the running step (the trainer's D(fake) stream)
+    bn_group = None                # process group of synchronised BatchNorm (--sync-bn, world > 1), or None: local statistics
 
 
 state = _State()
@@ -64,6 +65,20 @@ class inputs_only_grads:
 
     def __exit__(self, *a):
         state.inputs_only = self.prev
+
+
+class local_batchnorm:
+    """Context: train-mode BatchNorm inside uses the statistics of the local batch even when synchronised BatchNorm is
+    on.  For work outside the training step (progress samples, FID): it is not part of the global batch, and a caller
+    may run it on one rank only, where a collective would wait for ranks that never issue it."""
+
+    def __enter__(self):
+        self.prev, state.bn_group = state.bn_group, None
+        return self
+
+    def __exit__(self, *a):
+        state.bn_group = self.prev
+        return False
 
 
 class ZeroArena:
@@ -648,6 +663,36 @@ class CastFn(Function):
 
 
 # --------------------------------------------------------------------------- BatchNorm + LeakyReLU
+def _bn_world(group):
+    import torch.distributed as dist
+    return dist.get_world_size(group)
+
+
+def _bn_all_reduce(sums, group):
+    """Sum the fp64 channel sums of every rank (synchronised BatchNorm), in place, ordered on the current stream."""
+    import torch.distributed as dist
+    dist.all_reduce(sums, group=group)
+
+
+def _bn_sync_ws(n, device):
+    """(fp64 [n] workspace for the sums, flag) from the arena, as _ws_zero."""
+    ws, z = _ws_zero(8 * n, device)
+    return ws.view(torch.float64)[:n], z
+
+
+def _bn_bwd_sync(x, ga, gx, mean, invstd, gamma, beta, slope, ggamma, gbeta, accumulate, group):
+    """Backward of synchronised BatchNorm + LeakyReLU: local reduce, all-reduce of the 2C sums, apply over the global
+    count.  Every rank writes 1/world of the global gamma / beta gradients; the gradient all-reduce adds them up."""
+    n, c, h, w = x.shape
+    world = _bn_world(group)
+    sums, z = _bn_sync_ws(2 * c, x.device)
+    call('ttg_bn_act_bwd_reduce', ptr(x), ptr(ga), n * h * w, c, ptr(mean), ptr(invstd), ptr(gamma), ptr(beta), slope,
+         ptr(sums), z, dtype_code(x.dtype))
+    _bn_all_reduce(sums, group)
+    call('ttg_bn_act_bwd_apply', ptr(x), ptr(ga), ptr(gx), n * h * w, c, world * n * h * w, ptr(sums), ptr(mean),
+         ptr(invstd), ptr(gamma), ptr(beta), slope, ptr(ggamma), ptr(gbeta), 1.0 / world, accumulate, dtype_code(x.dtype))
+
+
 class BnActFn(Function):
     """lrelu(batch_norm(x)) with batch statistics (train) or running statistics (eval)."""
 
@@ -661,7 +706,18 @@ class BnActFn(Function):
         mean = torch.empty(c, dtype=torch.float32, device=dev)
         invstd = torch.empty(c, dtype=torch.float32, device=dev)
         y = _empty_like(x)
-        if training:
+        group = state.bn_group if training else None
+        if group is not None:
+            # synchronised: the local sums (from the producer or reduced here) are summed over the ranks, and the
+            # statistics and running-statistics update use the global pixel count
+            if sums is None:
+                sums, z = _bn_sync_ws(2 * c, dev)
+                call('ttg_bn_sums', ptr(x), m, c, ptr(sums), z, dtype_code(x.dtype))
+            _bn_all_reduce(sums, group)
+            call('ttg_bn_act_fwd_stats_n', ptr(x), ptr(y), m, c, _bn_world(group) * m, ptr(sums), ptr(gamma), ptr(beta),
+                 eps, momentum, slope, ptr(mean), ptr(invstd), ptr(running_mean), ptr(running_var), ptr(num_batches),
+                 count_mult, None, dtype_code(x.dtype))
+        elif training:
             # statistics (already reduced by the producing conv / join kernel when `sums` is given), their
             # finalisation and the apply pass: one entry point, one or two launches
             ws = None if sums is not None else _ws(_lib.lib.ttg_bn_workspace_bytes(c), dev)
@@ -688,6 +744,9 @@ class BnActFn(Function):
             x, ga = nhwc(x), nhwc(ga)
             n, c, h, w = x.shape
             gx = _empty_like(x)
+            if state.bn_group is not None:
+                _bn_bwd_sync(x, ga, gx, mean, invstd, gamma, beta, ctx.slope, dg, db, 1, state.bn_group)
+                return gx, None, None, None, None, None, None, None, None, None, None, None
             ws, z = _ws_zero(_lib.lib.ttg_bn_workspace_bytes(c), x.device)
             call('ttg_bn_act_bwd_acc', ptr(x), ptr(ga), ptr(gx), n * h * w, c, ptr(mean), ptr(invstd), ptr(gamma),
                  ptr(beta), ctx.slope, ptr(dg), ptr(db), 1 | z, ptr(ws), dtype_code(x.dtype))
@@ -707,9 +766,12 @@ class BnActBwdFn(Function):
         gx = _empty_like(x)
         ggamma = torch.empty(c, dtype=torch.float32, device=dev)
         gbeta = torch.empty(c, dtype=torch.float32, device=dev)
-        ws = _ws(_lib.lib.ttg_bn_workspace_bytes(c), dev)
-        call('ttg_bn_act_bwd', ptr(x), ptr(ga), ptr(gx), n * h * w, c, ptr(mean), ptr(invstd), ptr(gamma), ptr(beta),
-             slope, ptr(ggamma), ptr(gbeta), ptr(ws), dtype_code(x.dtype))
+        if state.bn_group is not None:
+            _bn_bwd_sync(x, ga, gx, mean, invstd, gamma, beta, slope, ggamma, gbeta, 0, state.bn_group)
+        else:
+            ws = _ws(_lib.lib.ttg_bn_workspace_bytes(c), dev)
+            call('ttg_bn_act_bwd', ptr(x), ptr(ga), ptr(gx), n * h * w, c, ptr(mean), ptr(invstd), ptr(gamma), ptr(beta),
+                 slope, ptr(ggamma), ptr(gbeta), ptr(ws), dtype_code(x.dtype))
         ctx.save_for_backward(x, ga, gamma, beta, mean, invstd)
         ctx.slope = slope
         ctx.set_materialize_grads(False)
@@ -729,6 +791,18 @@ class BnActBwdFn(Function):
         g_ga, g_x = _empty_like(x), _empty_like(x)
         dg = None if state.inputs_only or not ctx.needs_input_grad[2] else _direct(gamma)
         g_gamma = None if (state.inputs_only or dg is not None) else torch.empty(c, dtype=torch.float32, device=dev)
+        group = state.bn_group
+        if group is not None:
+            # synchronised: g_gamma is not linear in the per-rank sums, so it too comes from the global ones
+            world = _bn_world(group)
+            sums, z = _bn_sync_ws(5 * c, dev)
+            call('ttg_bn_act_bwd2_reduce', ptr(x), ptr(ga), ptr(u), n * h * w, c, ptr(mean), ptr(invstd), ptr(gamma),
+                 ptr(beta), ctx.slope, ptr(sums), z, dtype_code(x.dtype))
+            _bn_all_reduce(sums, group)
+            call('ttg_bn_act_bwd2_apply', ptr(x), ptr(ga), ptr(u), ptr(g_ga), ptr(g_x), n * h * w, c, world * n * h * w,
+                 ptr(sums), ptr(mean), ptr(invstd), ptr(gamma), ptr(beta), ctx.slope,
+                 ptr(dg if dg is not None else g_gamma), 1.0 / world, 1 if dg is not None else 0, dtype_code(x.dtype))
+            return g_x, g_ga, g_gamma, None, None, None, None
         ws, z = _ws_zero(_lib.lib.ttg_bn_workspace_bytes(c), dev)
         call('ttg_bn_act_bwd2_acc', ptr(x), ptr(ga), ptr(u), ptr(g_ga), ptr(g_x), n * h * w, c, ptr(mean), ptr(invstd),
              ptr(gamma), ptr(beta), ctx.slope, ptr(dg if dg is not None else g_gamma), (1 if dg is not None else 0) | z,

@@ -3,7 +3,9 @@ all-reduce launched from grad-ready hooks so that the exchange overlaps the rest
 
 The reference is single-process (SURVEY.md §2.1); this is the one collective the sharded path
 needs (§8e): average D's gradients after d_loss.backward() and G's after g_loss.backward().
-Local BatchNorm statistics (= the reference run at the per-rank batch) and per-rank z/tau draws.
+Local BatchNorm statistics (= the reference run at the per-rank batch) and per-rank z/tau draws; with --sync-bn the
+BatchNorm passes all-reduce their fp64 channel sums instead (ops.state.bn_group), so the statistics are those of the
+global batch and every rank applies the same update to the running statistics.
 torch.distributed does the plumbing (NCCL over NVLink on the GPUs; gloo in the CPU tests).
 """
 import torch

@@ -165,7 +165,9 @@ class FIDEvaluator:
     def on_batch_end(self, steps, logs):
         a = self.trainer.args
         if steps and steps % a.fid_freq == 0:
-            is_mean, is_std, fid = self.metrics.get(self.trainer.sample_g, a.n_inception_imgs, num_splits=5)
+            from .. import ops
+            with ops.local_batchnorm():          # not part of the global batch: BatchNorm over these samples only
+                is_mean, is_std, fid = self.metrics.get(self.trainer.sample_g, a.n_inception_imgs, num_splits=5)
             logs['fid'].append(fid)
             logs['inception_score_mean'].append(is_mean)
             logs['inception_score_std'].append(is_std)

@@ -75,6 +75,10 @@ class GanTrainer(Trainer):
         if torch.distributed.is_available() and torch.distributed.is_initialized():
             self.world_size, self.rank = torch.distributed.get_world_size(), torch.distributed.get_rank()
             self.broadcast_parameters()
+        # --sync-bn: BatchNorm statistics over the global batch.  The BatchNorm passes then issue collectives, which
+        # every rank must issue in the same order: the step runs the single-stream schedule (see _single_stream)
+        self.sync_bn = bool(getattr(args, 'sync_bn', False)) and self.world_size > 1 and args.norm == 'bn'
+        ops.state.bn_group = torch.distributed.group.WORLD if self.sync_bn else None
 
     def init_params_selu(self, params):
         """trainers/cnn.py:96-105 / trainers/iqn.py:94-102: vectors zeroed, matrices / filters N(0, 1/fan_in).  The draws
@@ -170,7 +174,7 @@ class GanTrainer(Trainer):
         if self.args.grad_penalty:
             real = imgs.detach().requires_grad_()
         gp = None
-        if _FAKE_STREAM and self.args.grad_penalty and ops.get_precision() == 'bf16':
+        if _FAKE_STREAM and self.args.grad_penalty and not self._single_stream():
             # The fake half of the D step (forward, and through autograd its whole backward chain) runs on a second
             # stream: D(fake) forward overlaps the R1 inner backward, the fake backward chain overlaps the real one and
             # the R1 double backward.  D's layers below 32x32 launch 32-128 CTAs on 148 SMs, so two chains fill what one
@@ -211,6 +215,12 @@ class GanTrainer(Trainer):
     def d_update(self):
         self.optimizer_d.step()
 
+    def _single_stream(self):
+        """The step keeps its BatchNorm work on one stream: in fp32 mode (fixed summation order) and under synchronised
+        BatchNorm (each BatchNorm pass all-reduces its sums, so the ranks must reach them in one program order).  The
+        skip-branch and weight-gradient side streams carry no BatchNorm and stay."""
+        return ops.get_precision() != 'bf16' or getattr(self, 'sync_bn', False)
+
     def _wait_gen_sample(self, stream):
         """Graph mode with the generator-sample graph on its own stream: `stream` waits (an external event-wait node
         inside the step graph) until that graph has produced this step's sample."""
@@ -225,7 +235,7 @@ class GanTrainer(Trainer):
         staged), so it runs beside the D step; only D(fake_g) has to wait for D's update.  Order kept: it starts after
         the generator sample of the D step (G's BatchNorm running statistics: z0 pass first, then z1, like the
         reference).  Returns the sample for g_forward_backward(fake=...); None when switched off."""
-        if not _EARLY_GFWD or ops.get_precision() != 'bf16':
+        if not _EARLY_GFWD or self._single_stream():
             return None
         main = torch.cuda.current_stream()
         g2 = getattr(self, '_g_stream', None)
@@ -272,6 +282,10 @@ class GanTrainer(Trainer):
         return out
 
     def train_batch(self, imgs, as_floats=True):
+        if getattr(self, 'sync_bn', False) and len(imgs) != self.args.batch_size:
+            # the statistics divide by world * (per-rank batch): shards must be equal
+            raise ValueError(f'--sync-bn needs the same batch on every rank: got {len(imgs)} images, '
+                             f'--batch-size is {self.args.batch_size}')
         self.g.train()
         self.d.train()
         if getattr(self.args, 'cuda_graph', False) and len(imgs) == self.args.batch_size:
@@ -448,7 +462,7 @@ class GanTrainer(Trainer):
         def gen():
             with torch.no_grad():
                 out['fake'] = self.sample_g(b)
-        gen_async = _GEN_ASYNC and not blocking and ops.get_precision() == 'bf16'
+        gen_async = _GEN_ASYNC and not blocking and not self._single_stream()
         # needs no images: runs while the host batch is still in flight (and, with gen_async, beside the step graph: then
         # its intermediates must not share memory with the step graph's)
         seg(gen, own_pool=gen_async)

@@ -52,8 +52,9 @@ class ImageSampler:
     def render(self):
         """-> (progress images: 16 of target_g then 16 of g, 5x5 interpolation grid of target_g); fp32 NCHW in [-1, 1].
         Like the reference the modules stay in whatever mode the trainer left them in (train: batch statistics)."""
+        from .. import ops
         t = self.trainer
-        with torch.no_grad():
+        with torch.no_grad(), ops.local_batchnorm():     # not part of the global batch: BatchNorm over these latents only
             imgs = torch.cat([t.target_g(self.progress_samples)[:16], t.g(self.progress_samples)[:16]], dim=0)
             if not hasattr(self, '_latent_grid_samples'):
                 self._latent_grid_samples = self.sample_latent_grid(5, 5)

@@ -395,3 +395,6 @@ class Trainer:
                             'semantics) in the discriminator and / or the generator')
         p.add_argument('--attention', type=type_or_none(str), default=None,
                        help='comma-separated block indices with self-attention (overrides the config)')
+        p.add_argument('--sync-bn', action='store_true',
+                       help='data parallel: BatchNorm statistics over the global batch (all-reduced over the ranks) '
+                            'instead of each rank\'s shard; the training step then runs on one stream')
